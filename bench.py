@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- HSFM agent-steps/s of the fused crowd step on B200, next to the reference algorithm on the host CPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dtype f64|f32] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dtype f64|f32] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one SocialNavGym.step over the whole batch: swept collision / goal / reward checks, then 20 fused
 (robot.step + update_humans) sub-steps at dt = 0.0125 (social_gym/social_nav_gym.py:227-250) -- ONE kernel launch.
@@ -27,6 +27,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 DT, SUBSTEPS = 0.0125, 20
+SETTLE_STEPS = 100
 METRIC = "HSFM agent-steps/sec (envs x humans x steps)"
 WORKLOADS = {
     # name: (model, E, N, walls, consider_robot)
@@ -67,6 +68,25 @@ def build_inputs(workload, seed0):
     safety = np.zeros(states.shape[:2])
     return dict(model=model, E=E, N=N, walls=walls, robot_visible=robot_visible, states=states, goals=sc["goals"],
                 robot=sc["robot"], safety=safety)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, one out_dir/<name>.npy each -- float32 data as float32,
+    everything else (float64 data, int32 flags and indices) as float64 -- so that two builds can be compared output for output."""
+    import torch
+    host = {}
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        host[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def algorithmic_cost(inp):
@@ -313,7 +333,7 @@ def run_large_crowd(args, rank, world, local_rank):
         sc = dict(states=np.ascontiguousarray(sc["states"][:, perm]), goals=np.ascontiguousarray(sc["goals"][:, perm]))
     crowd = LargeCrowd("hsfm_farina", sc["states"][0], sc["goals"][0], dtype=tdtype, rank=rank, world=world,
                        exchange=os.environ.get("SNP_EXCHANGE", "auto"))
-    steps = min(args.steps, 50)
+    steps = args.steps
     for _ in range(args.warmup):
         crowd.step(DT, 1)
     crowd.check_peers()
@@ -332,6 +352,8 @@ def run_large_crowd(args, rank, world, local_rank):
             ev[s][1].record(stream)
         torch.cuda.synchronize()
     launches = int(lib.snp_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"dyn": crowd.eng.dyn, "goal_idx": crowd.eng.goal_idx})
     from social_navigation_pyenvs_b200.parallel import max_over_ranks
     total_ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in ev), "cuda", world)
     # the same steps with the exact far-tile culling switched off: every ordered pair is evaluated -> the all-pairs roofline
@@ -482,6 +504,8 @@ def run_laser(args, rank, world, local_rank):
             ev[s][1].record(stream)
         torch.cuda.synchronize()
     launches = int(lib.snp_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ranges": ranges, "hits": hits})
     total_ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in ev), "cuda", world)
     # end to end with host arrays through the reference-shaped call (humans [E,N,3], walls, pose [E,3] -> ranges, hits)
     humans = inp["states"][:, :N][:, :, [0, 1, 8]].copy()
@@ -573,10 +597,15 @@ def run_lookahead(args, rank, world, local_rank):
             ev[s][0].record(stream)
             nxt = eng.peek(0.25)
             ev[s][1].record(stream)
-            eng.lookahead_from(nxt, 0.25, bulk_store=bulk)
+            rot, rew = eng.lookahead_from(nxt, 0.25, bulk_store=bulk)
             ev[s][2].record(stream)
         torch.cuda.synchronize()
     launches = int(lib.snp_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        # the rotated states are 862 MB in fp64: a fixed, seeded sample of 128 envs of them
+        envs = np.sort(np.random.default_rng(0).choice(E, min(E, 128), replace=False))
+        dump_outputs(args.dump_outputs, {"next": nxt, "rewards": rew, "rotated_envs": envs,
+                                         "rotated": rot[torch.from_numpy(envs).to(rot.device)]})
     total_ms = max_over_ranks(sum(e[0].elapsed_time(e[2]) for e in ev), "cuda", world)
     look_ms = sum(e[1].elapsed_time(e[2]) for e in ev) / args.steps
     peek_ms = sum(e[0].elapsed_time(e[1]) for e in ev) / args.steps
@@ -647,7 +676,11 @@ def main():
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32"])
     ap.add_argument("--workload", default="4096x25_hsfm_ccso_walls_robot", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step as DIR/<name>.npy "
+                    "(rank 0's share when several GPUs run)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -698,17 +731,28 @@ def main():
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device="cuda")  # > 126 MB L2
     stream = torch.cuda.current_stream()
 
-    def one_step():
-        eng.step(None, DT, n_substeps=SUBSTEPS, pre_checks=True, post_checks=False, track_touch=True)
+    def one_step(e=eng):
+        e.step(None, DT, n_substeps=SUBSTEPS, pre_checks=True, post_checks=False, track_touch=True)
 
     for _ in range(args.warmup):
         one_step()
     torch.cuda.synchronize()
-    t_ramp = time.perf_counter()  # extra untimed load so the SM clock has ramped before the timed region starts
+    # extra untimed load so the SM clock has ramped before the timed region starts.  It steps a twin of the engine, so that the
+    # state the timed steps start from does not depend on how many ramp steps fit in the ramp time
+    twin = make_engine(tdtype)
+    twin.mapping = eng.mapping
+    twin.action.copy_(action_host)
+    t_ramp = time.perf_counter()
     while time.perf_counter() - t_ramp < float(os.environ.get("SNP_BENCH_RAMP_S", "0.25")):
         for _ in range(20):
-            one_step()
+            one_step(twin)
         torch.cuda.synchronize()
+    del twin
+    # A fixed number of untimed steps takes the crowd past the opening of the episode: while every human crosses the centre at
+    # once (steps ~25-55) a step costs up to 2 % more; from step ~100 on the cost per step is flat.
+    for _ in range(SETTLE_STEPS):
+        one_step()
+    torch.cuda.synchronize()
 
     # ---- timed region: K steps, each its own CUDA-event pair on the launching stream, L2 flushed between steps ----
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
@@ -726,6 +770,9 @@ def main():
         torch.cuda.synchronize()
         wall = time.perf_counter() - wall0
     launches = int(lib.snp_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"dyn": eng.dyn, "robot": eng.robot, "goal_idx": eng.goal_idx, "time_now": eng.time_now,
+                                         "flags": eng.flags, "checks": eng.checks})
     if world > 1:
         dist.barrier()
     step_ms = [a.elapsed_time(b) for a, b in ev]
