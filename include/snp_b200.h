@@ -30,7 +30,7 @@
  *   snp_robot_push_out                            <- src/robot_agent.py:35-48 RobotAgent.check_collisions (social_nav_sim.py:509)
  *   snp_reset                                     <- social_nav_gym.py:120-225 reset, social_nav_sim.py:200-431 scenario generators
  *   snp_pack_states / snp_unpack_states           <- src/agent.py:256-266 get_safe_state / set_state row layout
- *   snp_large_step                                <- same update for one very large crowd (tiled all-pairs)
+ *   snp_large_run_p2p                             <- same update for one very large crowd (tiled all-pairs)
  */
 #ifndef SNP_B200_H
 #define SNP_B200_H
@@ -41,7 +41,7 @@
 extern "C" {
 #endif
 
-#define SNP_ABI_VERSION 3
+#define SNP_ABI_VERSION 4
 
 typedef enum snp_status {
     SNP_OK = 0,
@@ -52,8 +52,7 @@ typedef enum snp_status {
 
 enum { SNP_F32 = 0, SNP_F64 = 1 };
 enum { SNP_OPT_FULL_PAIR_LOOP = 1, SNP_OPT_NO_CULLING = 2, SNP_OPT_MAP_WARP = 4, SNP_OPT_MAP_BLOCK = 8,
-       SNP_OPT_STAGED_COPIES = 16, /* snp_gym_step_host: D2H copies after the launch even for pinned result buffers */
-       SNP_OPT_LARGE_GRID = 32     /* snp_large_*: culled steps on the static (i-block, chunk) grid instead of the work list (tests / tuning) */ };
+       SNP_OPT_STAGED_COPIES = 16  /* snp_gym_step_host: D2H copies after the launch even for pinned result buffers */ };
 
 /* Field order of the structure-of-arrays buffers (each field is a contiguous run of E*N elements). */
 enum { SNP_DYN_PX = 0, SNP_DYN_PY, SNP_DYN_VX, SNP_DYN_VY, SNP_DYN_TH, SNP_DYN_BVX, SNP_DYN_BVY, SNP_DYN_OM,
@@ -237,31 +236,22 @@ int snp_pack_states(const snp_crowd *crowd, double *rows_dev, int32_t rows_per_e
  * performed in place (forces_parallel.py:229-232) to the caller's float64 rows, given the crowd's goal_idx. */
 int snp_unpack_goals(const snp_crowd *crowd, const double *goal_rows_dev, int32_t *goal_cnt_dev, void *cuda_stream);
 int snp_rotate_goal_rows(const snp_crowd *crowd, double *goal_rows_dev, void *cuda_stream);
-/* One very large crowd (the crowd's E*N agents form ONE environment): one sub-step, shared-memory tiled all-pairs.
- * `others` = [5][M] x,y,vx,vy,r+safety (SoA) of ALL M entities exerting force -- the crowd itself (gathered over ranks
- * when it is sharded by agent) plus, optionally, the robot as last entry; `self_offset` = index of this crowd's agent 0
- * in that view.  Own state is updated in place; when `next_view` is non-NULL the updated x,y,vx,vy,r+safety of the own
- * agents are also written into it (same [5][M] layout, same offset), ready to be all-gathered for the next sub-step.
- * `scratch` = device workspace of at least snp_large_scratch_bytes(n_local, M, dtype) bytes (per-chunk partial sums, tile
- * boxes, the map and lists of the (agent block, entity chunk) units in reach, the work queues' counters).  opts->reserved bit 1
- * (SNP_OPT_NO_CULLING) disables the exact far-tile culling; SNP_OPT_LARGE_GRID runs a culled step on the static grid of units
- * instead of the list worked off by persistent CTAs (same results bit for bit, slower; tests / tuning). */
-int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype);
-int snp_large_step(const snp_crowd *crowd, const snp_step_opts *opts, const void *others, int64_t M, int64_t self_offset,
-                   void *next_view, void *scratch, int64_t scratch_bytes, void *cuda_stream);
-/* Same sub-step with the all-gather FUSED into the producer kernel: `peer_next_views` is a host array of `n_peers` device
- * pointers -- the NEXT-view buffer of every rank of the node (this rank's own included), peer-mapped over NVLink (e.g. torch
- * symmetric memory) -- and the finish kernel stores each agent's new entry straight into all of them.  The caller only needs a
- * cross-rank barrier between sub-steps; no collective moves data. */
-int snp_large_step_p2p(const snp_crowd *crowd, const snp_step_opts *opts, const void *others, int64_t M, int64_t self_offset,
-                       const void *const *peer_next_views, int32_t n_peers, void *scratch, int64_t scratch_bytes, void *cuda_stream);
-/* `n_substeps` of the agent-sharded step in ONE call (the loop SocialNavGym.step runs, social_nav_gym.py:240-245, for one crowd spread
- * over `world` GPUs of a node): per sub-step two launches (tiled pairs, finish) + one single-warp barrier kernel, all enqueued on
- * `cuda_stream` without returning to the host.  Buffers, all peer-mapped (e.g. torch symmetric memory), as host arrays of `world`
- * device pointers indexed by rank: `peer_views_a` / `peer_views_b` = the two view buffers, each [5][M] entities followed by the
- * view's [ceil(M/128)][5] tile-box table (the producer writes entries AND boxes into every rank's next buffer); `peer_flags` =
+/* One very large crowd (the crowd's E*N agents form ONE environment), shared-memory tiled all-pairs: `n_substeps` sub-steps in ONE
+ * call (the loop SocialNavGym.step runs, social_nav_gym.py:240-245), all enqueued on `cuda_stream` without returning to the host.
+ * The crowd is this rank's slice of agents of a view of M entities exerting force (x,y,vx,vy,r+safety, SoA), starting at entity
+ * `self_offset`; a crowd not sharded over GPUs is the whole view (world = 1, rank = 0, self_offset = 0).  Own state is updated in
+ * place and the updated entries of the own agents are stored into the next view of every rank.  Buffers, as host arrays of `world`
+ * device pointers indexed by rank (peer-mapped over NVLink when world > 1, e.g. torch symmetric memory): `peer_views_a` /
+ * `peer_views_b` = the two view buffers, each [5][M] entities followed by the view's [ceil(M/128)][5] tile-box table; `peer_flags` =
  * uint64[world] barrier slots per rank, zero-initialised once.  `first_is_b` selects the buffer that holds the current view;
- * `epoch_base` must grow by `n_substeps` from call to call.  `error_flag` (device int32) is set if a peer never reached a barrier. */
+ * `epoch_base` must grow by `n_substeps` from call to call.  Per sub-step: the tiled pair phase, the finish kernel and, when
+ * world > 1, one single-warp barrier kernel; `error_flag` (device int32) is set if a peer never reached a barrier.  When this slice
+ * is a whole number of 128-entity tiles and the `world` slices make up the view, the producers also write the next view's tile boxes;
+ * otherwise every sub-step recomputes the boxes of the view it reads (one more launch).  An exchange of its own (e.g. an all-gather
+ * of the slices) runs between calls of one sub-step with world = 1.  `scratch` = 16-byte aligned device workspace of at least
+ * snp_large_scratch_bytes(n_local, M, dtype) bytes (per-chunk partial sums, the map and lists of the (agent block, entity chunk)
+ * units in reach, the work queues' counters).  opts->reserved bit 1 (SNP_OPT_NO_CULLING) disables the exact far-tile culling. */
+int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype);
 int snp_large_run_p2p(const snp_crowd *crowd, const snp_step_opts *opts, const void *const *peer_views_a, const void *const *peer_views_b,
                       int32_t first_is_b, int64_t M, int64_t self_offset, int32_t world, int32_t rank, const void *const *peer_flags,
                       uint64_t epoch_base, int32_t n_substeps, int32_t *error_flag, void *scratch, int64_t scratch_bytes, void *cuda_stream);

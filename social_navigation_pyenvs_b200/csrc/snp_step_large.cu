@@ -2,7 +2,8 @@
 // desired / torque / Euler epilogue as the small-crowd kernel.  One sub-step on one stream:
 //
 //   k_tile_boxes    bounding box (+ max r+safety) of every 128-entity tile of the `others` view  [5][M] = x, y, vx, vy, r+s
-//                   (first sub-step of a call only: afterwards the finish kernel writes the boxes of the tiles it produces)
+//                   (every sub-step, or -- when the producers of a call write every tile of the next view -- the first sub-step
+//                   of a call only: afterwards the finish kernel writes the boxes of the tiles it produces)
 //   pair phase      unit of work = (i-block of 128 or 256 agents, j-chunk of 128 entities): every agent accumulates the force of
 //                   the chunk's entities in ascending j from a shared-memory tile and writes ONE partial sum per chunk.  A chunk
 //                   is skipped when its box is farther from the i-block's box than the distance at which the pair law is
@@ -45,12 +46,11 @@ template <typename T> struct LargeArgs {
     KArgs<T> k;
     const T *others;
     long long M, self_offset;
-    T *next_view;
-    T *peers[8];  // next-view buffers of every rank (peer-mapped device pointers); the finish kernel stores into all of them
+    T *peers[8];  // next-view buffers of every rank (peer-mapped device pointers; one buffer: n_peers = 1); the finish kernel stores into all of them
     int n_peers;
     T *partial;   // [J][2][N_local]
-    T *boxes;     // [n_tiles][5] xmin, xmax, ymin, ymax, max(r+s)
-    T *peer_boxes[8];  // snp_large_run_p2p: the NEXT view's tile boxes on every rank; the finish kernel writes its own tiles' boxes there
+    T *boxes;     // [n_tiles][5] xmin, xmax, ymin, ymax, max(r+s) of the tiles of `others` (the view buffer's own table)
+    T *peer_boxes[8];  // the NEXT view's tile boxes on every rank, or null: the finish kernel writes its own tiles' boxes there
     unsigned char *live;  // [i-blocks][J]: 1 when the (i-block, chunk) CTA evaluated at least one tile and wrote its partial sums
     int J, n_tiles;
     int Jp;  // row stride of the `live` map: J rounded up to 16 (the finish kernel reads 16 flags per load)
@@ -274,20 +274,12 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
         }
 }
 
-// Regular grid (i-block, chunk): every ordered pair, or -- with culling -- CTAs that first decide from the tile boxes whether their
-// chunk is in reach at all, before any state is loaded or any barrier is reached.  A culled CTA leaves its partial sums unwritten
-// and says so in `live`.
+// Regular grid (i-block, chunk): every ordered pair, or -- with culling, for a slice the work list does not take -- every tile
+// tested against the box of the i-block's agents.  A CTA that culled every tile leaves its partial sums unwritten and says so in
+// `live`.
 template <typename T, int SOC, int kAgentsPerThread>
 __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
     __shared__ PairsSmem<T> sm;
-    if (la.cull_margin >= T(0) && la.self_offset % kTile == 0) {
-        T u[5];
-        iblock_box<T>(la, blockIdx.x, kAgentsPerThread, u);
-        if (!chunk_near<T>(la, u, blockIdx.y)) {  // uniform across the CTA
-            if (threadIdx.x == 0) la.live[(size_t)blockIdx.x * la.Jp + blockIdx.y] = 0;
-            return;
-        }
-    }
     bool have_tbl = false;  // the 16 kB exp table is staged only by CTAs that evaluate at least one tile (most are culled)
     pairs_chunk<T, SOC, kAgentsPerThread>(la, sm, blockIdx.x, blockIdx.y, have_tbl);
 }
@@ -487,18 +479,12 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
         a.dyn[SNP_DYN_OM * N + i] = m.om;
     }
     a.goal_idx[i] = gidx;
-    if (la.n_peers > 0) {
-        // the all-gather of the entity view fused into the producer: every rank's copy of the NEXT view receives this agent's
-        // entry through peer (NVLink) stores, so no separate collective runs between sub-steps -- only a barrier
-        const long long o = la.self_offset + i;
-        for (int p = 0; p < la.n_peers; ++p) {
-            T *v = la.peers[p];
-            v[o] = m.px; v[M + o] = m.py; v[2 * M + o] = m.vx; v[3 * M + o] = m.vy; v[4 * M + o] = m.rs;
-        }
-    } else if (la.next_view) {
-        const long long o = la.self_offset + i;
-        la.next_view[o] = m.px; la.next_view[M + o] = m.py; la.next_view[2 * M + o] = m.vx; la.next_view[3 * M + o] = m.vy;
-        la.next_view[4 * M + o] = m.rs;
+    // the all-gather of the entity view fused into the producer: every rank's copy of the NEXT view receives this agent's entry
+    // through peer (NVLink) stores, so no separate collective runs between sub-steps -- only a barrier
+    const long long o = la.self_offset + i;
+    for (int p = 0; p < la.n_peers; ++p) {
+        T *v = la.peers[p];
+        v[o] = m.px; v[M + o] = m.py; v[2 * M + o] = m.vx; v[3 * M + o] = m.vy; v[4 * M + o] = m.rs;
     }
     if (fold_boxes) {
         // k_tile_boxes folded into the producer: this block's agents ARE one tile of the next view (self_offset is a multiple of
@@ -568,18 +554,16 @@ template <typename T, int SOC, int OBS, int HEADED> int launch_large(const Large
     if (!la.boxes_ready) k_tile_boxes<T><<<(unsigned)la.n_tiles, kTile, 0, st>>>(la.others, la.M, la.boxes);
     const long long per_block = (long long)kTile * la.apt;
     dim3 grid((unsigned)((N + per_block - 1) / per_block), (unsigned)la.J);
-    if (la.use_list) {
-        if (!la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));  // first sub-step of a call; later ones: the finish kernel
+    if constexpr (SOC == 2) {  // Moussaid's pair law has no culling distance (run_large): every pair, two agents per thread
+        k_large_pairs<T, SOC, kMaxAgentsPerThread><<<grid, kTile, 0, st>>>(la);
+    } else if (la.use_list) {  // (culled: one agent per thread)
+        // the counters start empty: zeroed here on a sub-step that computes the tile boxes, else by the previous sub-step's finish kernel
+        if (!la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
         k_large_cull<T><<<grid.x, 256, 0, st>>>(la);
-        static int slots1 = 0, slots2 = 0;  // resident CTAs per SM of the two instantiations
+        static int slots = 0;  // resident CTAs per SM
         const int n_queues = device_sm_count() < kMaxQueues ? device_sm_count() : kMaxQueues;
-        if (la.apt == 1) {
-            if (!slots1) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots1, k_large_pairs_list<T, SOC, 1>, kTile, 0));
-            k_large_pairs_list<T, SOC, 1><<<(unsigned)(device_sm_count() * (slots1 > 0 ? slots1 : 1)), kTile, 0, st>>>(la, n_queues);
-        } else {
-            if (!slots2) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots2, k_large_pairs_list<T, SOC, 2>, kTile, 0));
-            k_large_pairs_list<T, SOC, 2><<<(unsigned)(device_sm_count() * (slots2 > 0 ? slots2 : 1)), kTile, 0, st>>>(la, n_queues);
-        }
+        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1>, kTile, 0));
+        k_large_pairs_list<T, SOC, 1><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
         count_launch();
     } else if (la.apt == 1) k_large_pairs<T, SOC, 1><<<grid, kTile, 0, st>>>(la);
     else k_large_pairs<T, SOC, 2><<<grid, kTile, 0, st>>>(la);
@@ -596,13 +580,31 @@ inline long long large_J(long long M) { return (M + kChunk - 1) / kChunk; }
 inline long long large_tiles(long long M) { return (M + kTile - 1) / kTile; }
 inline long long large_iblocks(long long N) { return (N + kTile - 1) / kTile; }  // sized for one agent per thread (the finer split)
 
-template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, const void *others, long long M, long long self_offset,
-                                    void *next_view, const void *const *peer_views, int n_peers, void *scratch, long long scratch_bytes,
-                                    cudaStream_t st, const void *cur_boxes = nullptr, bool boxes_ready = false, const void *const *peer_next_boxes = nullptr) {
+// The scratch of n_local agents against M entities: byte offsets of its regions (the partial sums at 0) and its size.  Every region
+// starts 16-byte aligned (the finish kernel reads the live map and the lists 16 bytes at a time).
+struct LargeScratch { long long live, counters, work, live_cnt, live_list, bytes; };
+inline LargeScratch large_scratch(long long n_local, long long M, long long elem_bytes) {
+    const long long J = large_J(M), Jp = (J + 15) & ~15LL, blocks = large_iblocks(n_local);
+    auto up16 = [](long long b) { return (b + 15) & ~15LL; };
+    LargeScratch s;
+    s.live = up16(elem_bytes * J * 2 * n_local);      // [J][2][n_local] partial sums
+    s.counters = up16(s.live + blocks * Jp);           // [blocks][Jp] live map
+    s.work = s.counters + 4 * kWorkCounters;           // counters and queues
+    s.live_cnt = up16(s.work + 4 * blocks * J);        // [blocks * J] list of the units in reach
+    s.live_list = up16(s.live_cnt + 4 * blocks);       // [blocks] live chunks per i-block
+    s.bytes = s.live_list + 4 * blocks * Jp;           // [blocks][Jp] their indices, ascending
+    return s;
+}
+
+// One sub-step: `cur` = the view buffer read ([5][M] entities + their [n_tiles][5] tile boxes), `next` = the n_peers buffers the
+// finish kernel stores the updated entries into, and their tile boxes too when `fold_boxes`.  `boxes_ready`: `cur`'s tile boxes
+// were written by the previous sub-step's producers.
+template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, const void *cur, const void *const *next, int n_peers,
+                                    long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, cudaStream_t st) {
     LargeArgs<T> la;
     la.n_peers = n_peers;
-    for (int p = 0; p < 8; ++p) la.peers[p] = (p < n_peers) ? (T *)peer_views[p] : nullptr;
-    for (int p = 0; p < 8; ++p) la.peer_boxes[p] = (peer_next_boxes && p < n_peers) ? (T *)peer_next_boxes[p] : nullptr;
+    for (int p = 0; p < 8; ++p) la.peers[p] = (p < n_peers) ? (T *)next[p] : nullptr;
+    for (int p = 0; p < 8; ++p) la.peer_boxes[p] = (fold_boxes && p < n_peers) ? (T *)next[p] + 5 * M : nullptr;
     la.boxes_ready = boxes_ready ? 1 : 0;
     KArgs<T> &a = la.k;
     a.E = 1; a.N = 0; a.G = c->G; a.EN = (long long)c->E * c->N;
@@ -612,24 +614,18 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     a.consider_robot = 0; a.symmetric = o->symmetric; a.numba = o->numba_compat; a.n_substeps = 1; a.robot_mode = 0;
     a.dt = (T)o->dt; a.dt_d = o->dt; a.action = nullptr; a.pre_checks = a.post_checks = a.track_touch = 0;
     a.time_now = nullptr; a.flags = nullptr; a.checks = nullptr; a.epw = 1; a.gpb = 1; a.mapping = 0; a.full_pair_loop = 1; a.respawn = 0; a.robot_type = 0; a.RP = a.P; a.robot_every = 0; a.robot_phase = 0; a.robot_dt = T(0);
-    la.others = (const T *)others; la.M = M; la.self_offset = self_offset; la.next_view = (T *)next_view;
+    la.others = (const T *)cur; la.M = M; la.self_offset = self_offset;
+    la.boxes = (T *)cur + 5 * M;
     la.J = (int)large_J(M); la.n_tiles = (int)large_tiles(M);
     la.Jp = (la.J + 15) & ~15;
-    const long long live_bytes = large_iblocks(a.EN) * la.Jp, list_entries = large_iblocks(a.EN) * la.J;
-    const long long need = (long long)sizeof(T) * ((long long)la.J * 2 * a.EN + (long long)la.n_tiles * 5) + live_bytes + 64 +
-                           4 * (kWorkCounters + list_entries + ((large_iblocks(a.EN) + 3) & ~3LL) + large_iblocks(a.EN) * la.Jp);
-    if (!scratch || scratch_bytes < need) { set_error("snp_large_step: scratch of %lld bytes needed, %lld given", need, scratch_bytes); return SNP_ERR_INVALID; }
-    la.partial = (T *)scratch;
-    la.boxes = la.partial + (size_t)la.J * 2 * a.EN;
-    la.live = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(la.boxes + (size_t)la.n_tiles * 5) + 15) & ~uintptr_t(15));
-    {   // counters and work list behind the live map, 16-byte aligned
-        uintptr_t p = reinterpret_cast<uintptr_t>(la.live) + (size_t)live_bytes;
-        la.work_counters = reinterpret_cast<int *>(p);
-        la.work = la.work_counters + kWorkCounters;
-        la.live_cnt = la.work + ((list_entries + 3) & ~3LL);
-        la.live_list = la.live_cnt + ((large_iblocks(a.EN) + 3) & ~3LL);
-    }
-    if (cur_boxes) la.boxes = (T *)cur_boxes;  // the view's own box table (snp_large_run_p2p)
+    const LargeScratch sc = large_scratch(a.EN, M, sizeof(T));
+    char *base = (char *)scratch;
+    la.partial = (T *)base;
+    la.live = (unsigned char *)(base + sc.live);
+    la.work_counters = (int *)(base + sc.counters);
+    la.work = (int *)(base + sc.work);
+    la.live_cnt = (int *)(base + sc.live_cnt);
+    la.live_list = (int *)(base + sc.live_list);
     // exact culling distance beyond the r+s sums: where exp(rd/B) is identically zero in the arithmetic in use
     const int soc = o->type % 3;
     const double under = sizeof(T) == 8 ? 700.0 : 88.0;
@@ -642,7 +638,7 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     // culled steps: one agent per thread (twice the units to hand out).  Round 2 kept two for fp32 on the static grid, where the
     // finer split only added CTAs to launch; on the work list one rank's slice of an 8-way split runs 0.0552 -> 0.0408 ms in fp32
     la.apt = margin >= 0.0 ? 1 : kMaxAgentsPerThread;  // fp32 pair evaluations are short: the finer split only adds launch overhead there
-    la.use_list = (margin >= 0.0 && self_offset % kTile == 0 && list_entries < (1LL << 31) && !(o->reserved & SNP_OPT_LARGE_GRID)) ? 1 : 0;
+    la.use_list = (margin >= 0.0 && self_offset % kTile == 0 && large_iblocks(a.EN) * la.J < (1LL << 31)) ? 1 : 0;
     switch (o->type) {
         case 0: return launch_large<T, 0, 0, 0>(la, st);
         case 1: return launch_large<T, 1, 1, 0>(la, st);
@@ -666,66 +662,37 @@ using namespace snp;
 extern "C" {
 
 int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype) {
-    const long long w = dtype == SNP_F64 ? 8 : 4;
-    return w * (large_J(M) * 2 * n_local + large_tiles(M) * 5) + 9 * large_iblocks(n_local) * ((large_J(M) + 15) & ~15LL) + 4 * large_iblocks(n_local) +
-           256 + 4 * kWorkCounters;
-}
-
-int snp_large_step(const snp_crowd *c, const snp_step_opts *o, const void *others, int64_t M, int64_t self_offset, void *next_view,
-                   void *scratch, int64_t scratch_bytes, void *stream) {
-    if (!c || !o || !others) { set_error("snp_large_step: null argument"); return SNP_ERR_INVALID; }
-    if (!c->dyn || !c->stat || !c->goals || !c->goal_idx || !c->goal_cnt) { set_error("snp_large_step: crowd arrays missing"); return SNP_ERR_INVALID; }
-    if (c->agent_params) { set_error("snp_large_step: per-agent parameter rows are not supported"); return SNP_ERR_UNSUPPORTED; }
-    if (c->walls_per_env) { set_error("snp_large_step: one wall set per crowd"); return SNP_ERR_INVALID; }
-    const long long N = (long long)c->E * c->N;
-    if (M < N || self_offset < 0 || self_offset + N > M + 1) { set_error("snp_large_step: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
-    if (c->dtype == SNP_F64) return run_large<double>(c, o, others, M, self_offset, next_view, nullptr, 0, scratch, scratch_bytes, (cudaStream_t)stream);
-    if (c->dtype == SNP_F32) return run_large<float>(c, o, others, M, self_offset, next_view, nullptr, 0, scratch, scratch_bytes, (cudaStream_t)stream);
-    set_error("bad dtype %d", c->dtype);
-    return SNP_ERR_INVALID;
-}
-
-int snp_large_step_p2p(const snp_crowd *c, const snp_step_opts *o, const void *others, int64_t M, int64_t self_offset,
-                       const void *const *peer_next_views, int32_t n_peers, void *scratch, int64_t scratch_bytes, void *stream) {
-    if (!c || !o || !others || !peer_next_views) { set_error("snp_large_step_p2p: null argument"); return SNP_ERR_INVALID; }
-    if (n_peers < 1 || n_peers > 8) { set_error("snp_large_step_p2p: 1..8 peers (got %d)", n_peers); return SNP_ERR_INVALID; }
-    if (!c->dyn || !c->stat || !c->goals || !c->goal_idx || !c->goal_cnt) { set_error("snp_large_step_p2p: crowd arrays missing"); return SNP_ERR_INVALID; }
-    if (c->agent_params || c->walls_per_env) { set_error("snp_large_step_p2p: uniform parameters and one wall set only"); return SNP_ERR_UNSUPPORTED; }
-    const long long N = (long long)c->E * c->N;
-    if (M < N || self_offset < 0 || self_offset + N > M + 1) { set_error("snp_large_step_p2p: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
-    if (c->dtype == SNP_F64) return run_large<double>(c, o, others, M, self_offset, nullptr, peer_next_views, n_peers, scratch, scratch_bytes, (cudaStream_t)stream);
-    if (c->dtype == SNP_F32) return run_large<float>(c, o, others, M, self_offset, nullptr, peer_next_views, n_peers, scratch, scratch_bytes, (cudaStream_t)stream);
-    set_error("bad dtype %d", c->dtype);
-    return SNP_ERR_INVALID;
+    return large_scratch(n_local, M, dtype == SNP_F64 ? 8 : 4).bytes;
 }
 
 int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *const *peer_views_a, const void *const *peer_views_b,
                       int32_t first_is_b, int64_t M, int64_t self_offset, int32_t world, int32_t rank, const void *const *peer_flags,
                       uint64_t epoch_base, int32_t n_substeps, int32_t *error_flag, void *scratch, int64_t scratch_bytes, void *stream) {
-    if (!c || !o || !peer_views_a || !peer_views_b || !peer_flags || !error_flag) { set_error("snp_large_run_p2p: null argument"); return SNP_ERR_INVALID; }
+    if (!c || !o || !peer_views_a || !peer_views_b || !peer_flags || !error_flag || !scratch) { set_error("snp_large_run_p2p: null argument"); return SNP_ERR_INVALID; }
     if (world < 1 || world > 8 || rank < 0 || rank >= world) { set_error("snp_large_run_p2p: 1..8 ranks (got world %d rank %d)", world, rank); return SNP_ERR_INVALID; }
     if (!c->dyn || !c->stat || !c->goals || !c->goal_idx || !c->goal_cnt) { set_error("snp_large_run_p2p: crowd arrays missing"); return SNP_ERR_INVALID; }
     if (c->agent_params || c->walls_per_env) { set_error("snp_large_run_p2p: uniform parameters and one wall set only"); return SNP_ERR_UNSUPPORTED; }
-    const long long N = (long long)c->E * c->N;
-    if (M < N || self_offset < 0 || self_offset + N > M) { set_error("snp_large_run_p2p: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
-    if (self_offset % kTile || N % kTile) { set_error("snp_large_run_p2p: every rank's slice must be a whole number of %d-entity tiles", kTile); return SNP_ERR_UNSUPPORTED; }
     if (c->dtype != SNP_F64 && c->dtype != SNP_F32) { set_error("bad dtype %d", c->dtype); return SNP_ERR_INVALID; }
+    const long long N = (long long)c->E * c->N;
+    if (self_offset < 0 || self_offset + N > M) { set_error("snp_large_run_p2p: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
+    const long long need = large_scratch(N, M, c->dtype == SNP_F64 ? 8 : 4).bytes;
+    if (scratch_bytes < need || reinterpret_cast<uintptr_t>(scratch) % 16) {
+        set_error("snp_large_run_p2p: 16-byte aligned scratch of %lld bytes needed, %lld given", need, (long long)scratch_bytes);
+        return SNP_ERR_INVALID;
+    }
+    // The producers write the next view's tile boxes only when together they write every tile of it: this slice is a whole number
+    // of tiles and the `world` slices make up the view.  Otherwise every sub-step recomputes the boxes of the view it reads.
+    const bool fold_boxes = self_offset % kTile == 0 && N % kTile == 0 && world * N == M;
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t w = c->dtype == SNP_F64 ? 8 : 4;
-    // a view buffer = [5][M] entity view followed by its [n_tiles][5] box table
-    auto boxes_of = [&](const void *view) { return (const void *)((const char *)view + (size_t)5 * M * w); };
     BarrierArgs b;
     for (int p = 0; p < 8; ++p) b.flags[p] = p < world ? (unsigned long long *)peer_flags[p] : nullptr;
     b.world = world; b.rank = rank; b.error = error_flag;
     int cur_is_b = first_is_b ? 1 : 0;
     for (int s = 0; s < n_substeps; ++s) {
         const void *const *cur = cur_is_b ? peer_views_b : peer_views_a, *const *nxt = cur_is_b ? peer_views_a : peer_views_b;
-        const void *nxt_boxes[8];
-        for (int p = 0; p < world; ++p) nxt_boxes[p] = boxes_of(nxt[p]);
-        int rc;
-        // sub-step 0 computes the tile boxes of the view it was handed; from then on the producer has written them
-        if (c->dtype == SNP_F64) rc = run_large<double>(c, o, cur[rank], M, self_offset, nullptr, nxt, world, scratch, scratch_bytes, st, boxes_of(cur[rank]), s > 0, nxt_boxes);
-        else rc = run_large<float>(c, o, cur[rank], M, self_offset, nullptr, nxt, world, scratch, scratch_bytes, st, boxes_of(cur[rank]), s > 0, nxt_boxes);
+        const bool boxes_ready = fold_boxes && s > 0;  // sub-step 0 computes the tile boxes of the view it was handed
+        const int rc = c->dtype == SNP_F64 ? run_large<double>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, st)
+                                           : run_large<float>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, st);
         if (rc) return rc;
         if (world > 1) {
             b.epoch = epoch_base + (unsigned long long)s + 1;

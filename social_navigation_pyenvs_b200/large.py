@@ -35,8 +35,8 @@ class LargeCrowd:
         # peer-mapped (torch symmetric memory, NVLink) pointers and only a barrier separates sub-steps; "nccl" = all-gather
         # after every sub-step.  "auto" tries p2p on multi-GPU runs and falls back to nccl.
         self.exchange, self._symm = "nccl", None
-        # a view buffer = the [5, N] entity view followed by the [N/128, 5] bounding boxes of its 128-entity tiles (written by the
-        # producer together with the entries, see snp_large_run_p2p)
+        # a view buffer = the [5, N] entity view followed by the [N/128, 5] bounding boxes of its 128-entity tiles (see
+        # snp_large_run_p2p)
         self._n_tiles = (self.n_total + 127) // 128
         vlen = 5 * self.n_total + 5 * self._n_tiles
         fused_ok = self.n_local % 128 == 0
@@ -61,21 +61,18 @@ class LargeCrowd:
                     raise
                 self._p2p_error = repr(exc)
         elif world == 1 and fused_ok and exchange != "nccl":
-            # one GPU: the same fused run (sub-step loop inside one C call, tile boxes written by the producer), no barrier
+            self.exchange = "fused"  # one GPU: the sub-step loop inside one C call, no barrier
+        if self.exchange != "p2p":  # this rank's own two view buffers
             self._vbuf = [torch.zeros((vlen,), dtype=dtype, device=self.eng.device) for _ in range(2)]
             self._flags = torch.zeros((16,), dtype=torch.int64, device=self.eng.device)
             self._peer_ptrs = [(ctypes.c_void_p * 1)(v.data_ptr()) for v in self._vbuf]
             self._peer_flags = (ctypes.c_void_p * 1)(self._flags.data_ptr())
-            self.exchange = "fused"
-        if self.exchange == "nccl":
-            self._vbuf = [torch.zeros((vlen,), dtype=dtype, device=self.eng.device) for _ in range(2)]
         self.view = [v[:5 * self.n_total].view(5, self.n_total) for v in self._vbuf]
         self._epoch = 0
         self._err = torch.zeros((1,), dtype=torch.int32, device=self.eng.device)
         nbytes = int(self.eng.lib.snp_large_scratch_bytes(self.n_local, self.n_total, L.SNP_F64 if dtype == torch.float64 else L.SNP_F32))
         self.scratch = torch.empty(nbytes, dtype=torch.uint8, device=self.eng.device)
         self.culling = True
-        self.work_list = True
         self.cur = 0
         if shard is not None:  # the frozen rest of the crowd: both view buffers start from the whole crowd's entries
             whole = CrowdEngine.from_reference_arrays(model, states[None], goals[None], consider_robot=False, all_params_equal=symmetric, dtype=dtype, device=device)
@@ -106,31 +103,19 @@ class LargeCrowd:
         c = self.eng._crowd()
         o = self.eng._opts(dt, 1)
         o.reserved = 0 if self.culling else L.SNP_OPT_NO_CULLING
-        if not self.work_list:
-            o.reserved |= L.SNP_OPT_LARGE_GRID  # culled steps on the static grid instead of the list of near (i-block, chunk) pairs
-        if self.exchange in ("p2p", "fused") and not getattr(self, "legacy_loop", False):
-            # the whole sub-step loop in ONE C call: per sub-step two launches + a single-warp cross-rank barrier kernel, nothing
-            # returns to Python in between
+        # p2p / fused: the whole sub-step loop in ONE C call, nothing returns to Python in between; nccl: one sub-step per call on
+        # this rank's own buffers, then the all-gather of the next view
+        nccl = self.exchange == "nccl"
+        world, rank, calls, k = (1, 0, n_substeps, 1) if nccl else (self.world, self.rank, 1, int(n_substeps))
+        for _ in range(calls):
             L.check(self.eng.lib.snp_large_run_p2p(ctypes.byref(c), ctypes.byref(o), self._peer_ptrs[0], self._peer_ptrs[1], self.cur, self.n_total,
-                                                   self.offset, self.world, self.rank, self._peer_flags, self._epoch, int(n_substeps),
+                                                   self.offset, world, rank, self._peer_flags, self._epoch, k,
                                                    ctypes.c_void_p(self._err.data_ptr()), ctypes.c_void_p(self.scratch.data_ptr()),
                                                    self.scratch.numel(), self._stream()))
-            self._epoch += int(n_substeps)
-            self.cur ^= int(n_substeps) & 1
-            return
-        for _ in range(n_substeps):
-            cur, nxt = self.view[self.cur], self.view[self.cur ^ 1]
-            if self.exchange == "p2p":
-                L.check(self.eng.lib.snp_large_step_p2p(ctypes.byref(c), ctypes.byref(o), ctypes.c_void_p(cur.data_ptr()), self.n_total, self.offset,
-                                                        self._peer_ptrs[self.cur ^ 1], self.world, ctypes.c_void_p(self.scratch.data_ptr()),
-                                                        self.scratch.numel(), self._stream()))
-                self._symm[self.cur ^ 1].barrier()  # every rank's stores into everybody's next view have landed
-            else:
-                L.check(self.eng.lib.snp_large_step(ctypes.byref(c), ctypes.byref(o), ctypes.c_void_p(cur.data_ptr()), self.n_total, self.offset,
-                                                    ctypes.c_void_p(nxt.data_ptr()), ctypes.c_void_p(self.scratch.data_ptr()), self.scratch.numel(),
-                                                    self._stream()))
-                self._gather(nxt)
-            self.cur ^= 1
+            self._epoch += k
+            self.cur ^= k & 1
+            if nccl:
+                self._gather(self.view[self.cur])
 
     def local_rows(self, template):
         """This rank's agents as reference rows; `template` [n_local,13] supplies the static columns."""

@@ -267,7 +267,7 @@ def spatial_order(positions, block=256):
     """Permutation that numbers the agents of ONE large crowd patch by patch: the crowd is cut into sqrt(n / block) vertical
     strips of equal head count (sorted by x) and every strip is walked in y, so that a run of consecutive agents (a 128-entity
     tile, a 256-agent block of the tiled all-pairs kernels) covers a compact patch of the plane instead of a long strip.  The
-    exact far-tile culling of snp_large_step tests bounding boxes of such runs and skips ~2x more of them.  The numbering of
+    exact far-tile culling of snp_large_run_p2p tests bounding boxes of such runs and skips ~2x more of them.  The numbering of
     the agents is the caller's (the reference keeps humans in insertion order, social_nav_sim.py:271-295, and no force depends
     on it), so this is applied to the rows BEFORE they are handed to LargeCrowd; `np.argsort(perm)` undoes it."""
     pos = np.asarray(positions, np.float64).reshape(-1, 2)

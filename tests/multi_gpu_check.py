@@ -23,24 +23,21 @@ S, G = sc["states"][0], sc["goals"][0]
 rng = np.random.RandomState(0)
 S[:, 5:7] = rng.uniform(-0.5, 0.5, (S.shape[0], 2))
 # exchange "p2p" = the whole sub-step loop in one C call (snp_large_run_p2p: producer stores entries + tile boxes into every rank's
-# next view, device-side barrier kernel); "p2p-legacy" = one snp_large_step_p2p + symmetric-memory barrier per sub-step from Python;
-# "nccl" = all-gather per sub-step.  The single-GPU crowd is run both through the fused call and the per-sub-step loop.
-for dtype, exchange in ((torch.float64, "nccl"), (torch.float32, "nccl"), (torch.float64, "p2p"), (torch.float32, "p2p"),
-                        (torch.float64, "p2p-legacy")):
-    sharded = LargeCrowd("hsfm_new_guo", S, G, dtype=dtype, rank=rank, world=world, exchange=exchange.split("-")[0])
-    assert sharded.exchange == exchange.split("-")[0]
-    sharded.legacy_loop = exchange.endswith("legacy")
+# next view, device-side barrier kernel); "nccl" = one call per sub-step, then an all-gather.  The single-GPU crowd is run both
+# through the fused call and, with "nccl" forced, one call per sub-step.
+for dtype, exchange in ((torch.float64, "nccl"), (torch.float32, "nccl"), (torch.float64, "p2p"), (torch.float32, "p2p")):
+    sharded = LargeCrowd("hsfm_new_guo", S, G, dtype=dtype, rank=rank, world=world, exchange=exchange)
+    assert sharded.exchange == exchange
     sharded.step(0.0125, n_substeps=3)
     sharded.step(0.0125, n_substeps=2)   # a second call continues from the other view buffer with a later barrier epoch
     sharded.check_peers()
     mine = sharded.local_rows(S[sharded.offset:sharded.offset + sharded.n_local])
-    for legacy in (False, True):
-        single = LargeCrowd("hsfm_new_guo", S, G, dtype=dtype, rank=0, world=1)
-        assert single.exchange == "fused"
-        single.legacy_loop = legacy
+    for single_exchange in ("fused", "nccl"):
+        single = LargeCrowd("hsfm_new_guo", S, G, dtype=dtype, rank=0, world=1, exchange={"fused": "auto", "nccl": "nccl"}[single_exchange])
+        assert single.exchange == single_exchange
         single.step(0.0125, n_substeps=5)
         ref = single.local_rows(S)[sharded.offset:sharded.offset + sharded.n_local]
-        assert np.array_equal(mine, ref), f"rank {rank}: sharded crowd differs from single-GPU crowd ({dtype}, {exchange}, legacy={legacy})"
+        assert np.array_equal(mine, ref), f"rank {rank}: sharded crowd differs from single-GPU crowd ({dtype}, {exchange}, single {single_exchange})"
 
 # ---- independent envs sharded by env: no collective on the data path ----
 states = np.concatenate([sc_env["states"], sc_env["robot"][:, None]], 1)

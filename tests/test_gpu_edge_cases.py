@@ -43,13 +43,13 @@ def test_degenerate_shapes_vs_oracle(model, N, E, robot):
 @pytest.mark.parametrize("dtype,tol", [(torch.float64, 1e-9), (torch.float32, 1e-4)])
 def test_first_crowd_of_the_tiled_kernel_vs_oracle(dtype, tol):
     """513 humans: one more than the fused kernel takes (snp_step answers SNP_ERR_UNSUPPORTED -> NotImplementedError and names
-    snp_large_step); the tiled all-pairs kernels take it, with a ragged last tile."""
+    snp_large_run_p2p); the tiled all-pairs kernels take it, with a ragged last tile."""
     from social_navigation_pyenvs_b200 import CrowdEngine
     from social_navigation_pyenvs_b200.large import LargeCrowd
     n = 513
     S, G = _random_crowd(1, n, seed=513, spread=1.1)
     if dtype == torch.float64:
-        with pytest.raises(NotImplementedError, match="snp_large_step"):
+        with pytest.raises(NotImplementedError, match="snp_large_run_p2p"):
             CrowdEngine.from_reference_arrays("hsfm_farina", S, G, all_params_equal=True).update_humans(0.0, 0.0125)
     if dtype == torch.float32:
         S = S.astype(np.float32).astype(np.float64); G = G.astype(np.float32).astype(np.float64)

@@ -1,6 +1,6 @@
 """Multi-GPU parity (-m gpu, skipped with fewer than two GPUs): tests/multi_gpu_check.py under torchrun -- the agent-sharded
-LargeCrowd (fused peer-store exchange, legacy per-sub-step loop, NCCL all-gather) must equal the single-GPU crowd BIT FOR BIT, and
-env-sharded engines the slices of one big engine."""
+LargeCrowd (fused peer-store exchange, NCCL all-gather) must equal the single-GPU crowd -- stepped in one call or one call per sub-step
+with the all-gather -- BIT FOR BIT, and env-sharded engines the slices of one big engine."""
 import os
 import subprocess
 import sys

@@ -139,7 +139,7 @@ def test_host_operator_serial_semantics_with_carried_desired_force(name):
 
 
 def test_large_crowd_tiled_kernel_vs_oracle():
-    """snp_large_step on a 1024-human crowd (type 3 and 7, walls) against the oracle's row-major pair loop, 3 sub-steps."""
+    """snp_large_run_p2p on a 1024-human crowd (type 3 and 7, walls) against the oracle's row-major pair loop, 3 sub-steps."""
     from social_navigation_pyenvs_b200 import scenarios
     from social_navigation_pyenvs_b200.large import LargeCrowd
     sc = scenarios.jittered_grid_crowd(32, pitch=1.0, jitter=0.3, seed=0)
@@ -164,9 +164,10 @@ def test_large_crowd_tiled_kernel_vs_oracle():
 @pytest.mark.parametrize("order", ["row_major", "patch"])
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
 def test_large_crowd_chunked_sums_and_exact_culling(dtype, order):
-    """5184 humans (two j-chunks, 41 tiles, a 72 m wide crowd): the chunked partial sums stay within 1e-9 of the oracle's single
+    """5184 humans (41 j-chunks and tiles, a 72 m wide crowd): the chunked partial sums stay within 1e-9 of the oracle's single
     j-ascending sum, and skipping tiles beyond the exp-underflow distance changes NOTHING (bit-identical on/off) -- with the
-    humans numbered row by row (long thin tiles) or patch by patch (scenarios.spatial_order: compact tiles, more of them culled)."""
+    humans numbered row by row (long thin tiles) or patch by patch (scenarios.spatial_order: compact tiles, more of them culled);
+    on the whole crowd (culled on the work list) and on a slice that does not start on a tile (culled on the static grid)."""
     from social_navigation_pyenvs_b200 import scenarios
     from social_navigation_pyenvs_b200.large import LargeCrowd
     sc = scenarios.jittered_grid_crowd(72, pitch=1.0, jitter=0.3, seed=3)
@@ -181,22 +182,61 @@ def test_large_crowd_chunked_sums_and_exact_culling(dtype, order):
     if dtype == torch.float32:
         S = S.astype(np.float32).astype(np.float64)
     out = {}
-    # culled on the list of near (i-block, chunk) pairs worked off by persistent CTAs (the default), culled on the static grid, all pairs
-    for cull, work_list in ((True, True), (True, False), (False, True)):
-        crowd = LargeCrowd("hsfm_farina", S[0], G[0], dtype=dtype, symmetric=True)
-        crowd.culling, crowd.work_list = cull, work_list
-        crowd.step(0.0125, n_substeps=2)
-        first = crowd.local_rows(S[0])
-        crowd.step(0.0125, n_substeps=1)  # (a second call: the list's counters were left empty by the first)
-        out[cull, work_list] = (first, crowd.local_rows(S[0]))
-    for k in (0, 1):
-        assert np.array_equal(out[True, True][k], out[False, True][k]) and np.array_equal(out[True, False][k], out[False, True][k])
-    out = {True: out[True, True][0]}
+    # the whole crowd: culled on the list of near (i-block, chunk) pairs worked off by persistent CTAs, or all pairs; a slice at
+    # offset 64: culled on the static grid, or all pairs
+    for shard in (None, (64, n - 64)):
+        for cull in (True, False):
+            crowd = LargeCrowd("hsfm_farina", S[0], G[0], dtype=dtype, symmetric=True, shard=shard)
+            crowd.culling = cull
+            rows = S[0] if shard is None else S[0, 64:]
+            crowd.step(0.0125, n_substeps=2)
+            first = crowd.local_rows(rows)
+            crowd.step(0.0125, n_substeps=1)  # (a second call: the list's counters were left empty by the first)
+            out[shard, cull] = (first, crowd.local_rows(rows))
+        for k in (0, 1):
+            assert np.array_equal(out[shard, True][k], out[shard, False][k]), (shard, k)
+    out = {True: out[None, True][0]}
     cfg = OracleConfig(oracle.type_code("hsfm_farina"), False, True, False)
     params = np.tile(oracle.default_params("hsfm_farina"), (1, n, 1))
     ref, _, _ = oracle.update_humans(cfg, S, G, None, params, np.zeros((1, n)), np.zeros((1, n, 2)), 0.0125, 2)
     tol = 1e-9 if dtype == torch.float64 else 1e-4
     assert rel_err(out[True][:, :8], ref[0, :, :8]).max() < tol
+
+
+@pytest.mark.parametrize("case", ["shard_substeps_in_one_call", "nccl_vs_fused"])
+def test_large_crowd_same_bits_however_the_substeps_are_called(case):
+    """fp32 hsfm_farina (culling reach 88 B ~ 7 m), sub-steps compared bit for bit:
+    * a shard= slice (the first 1024 humans of a 72 x 72 crowd numbered row by row: x ~ -35 m, away from the crowd's centre) stepped
+      3 sub-steps in one call == 3 calls of one: the tile boxes of the frozen rest of the crowd are recomputed every sub-step, not
+      read from a next-view table its producers only partly wrote;
+    * a 1024-human crowd with exchange="nccl" forced on one GPU (one C call per sub-step, then the all-gather) == the fused one
+      (the sub-step loop in one C call, tile boxes written by the producers), over two calls of several sub-steps each."""
+    from social_navigation_pyenvs_b200 import model_parameters, scenarios
+    from social_navigation_pyenvs_b200.large import LargeCrowd
+    side = 72 if case == "shard_substeps_in_one_call" else 32
+    sc = scenarios.jittered_grid_crowd(side, pitch=1.0, jitter=0.3, seed=4)
+    S, G = sc["states"][0], sc["goals"][0]
+    S[:, 5:7] = np.random.RandomState(2).uniform(-0.6, 0.6, (S.shape[0], 2))
+    if case == "shard_substeps_in_one_call":
+        shard, rows = (0, 1024), S[:1024]
+        reach = 88 * model_parameters("hsfm_farina")[3] + 2 * S[:, 8].max() + 0.1
+        assert S[1024:, 0].min() - S[:1024, 0].max() < reach < S[:, 0].max() - S[:1024, 0].max()  # neighbours in reach, units culled
+        assert S[:1024, 0].max() < -reach  # the zero boxes the next view's table starts with sit at the origin, out of reach
+        a = LargeCrowd("hsfm_farina", S, G, dtype=torch.float32, symmetric=True, shard=shard)
+        b = LargeCrowd("hsfm_farina", S, G, dtype=torch.float32, symmetric=True, shard=shard)
+        assert a.exchange == b.exchange == "fused"
+        a.step(0.0125, n_substeps=3)
+        for _ in range(3):
+            b.step(0.0125, n_substeps=1)
+    else:
+        rows = S
+        a = LargeCrowd("hsfm_farina", S, G, dtype=torch.float32, symmetric=True)
+        b = LargeCrowd("hsfm_farina", S, G, dtype=torch.float32, symmetric=True, exchange="nccl")
+        assert (a.exchange, b.exchange) == ("fused", "nccl")
+        for k in (3, 2):
+            a.step(0.0125, n_substeps=k)
+            b.step(0.0125, n_substeps=k)
+    assert np.array_equal(a.local_rows(rows), b.local_rows(rows))
 
 
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])

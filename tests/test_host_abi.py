@@ -29,7 +29,7 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
         assert hasattr(handle, name), f"{name} declared in include/snp_b200.h but not exported"
     assert sorted(_lib.EXPORTED_SYMBOLS) == declared, "ctypes signature table and header disagree"
     lib = _lib.lib()
-    assert lib.snp_abi_version() == 3
+    assert lib.snp_abi_version() == 4
 
 
 def test_ctypes_struct_layouts_match_the_header(tmp_path):
@@ -59,8 +59,7 @@ def test_python_constants_match_the_header_enums(tmp_path):
     """The option bits, dtype codes, field counts and flag bits the Python side uses are the header's."""
     import subprocess
     from social_navigation_pyenvs_b200 import _lib as L
-    names = ["SNP_F32", "SNP_F64", "SNP_OPT_FULL_PAIR_LOOP", "SNP_OPT_NO_CULLING", "SNP_OPT_MAP_WARP", "SNP_OPT_MAP_BLOCK", "SNP_OPT_STAGED_COPIES",
-             "SNP_OPT_LARGE_GRID"]
+    names = ["SNP_F32", "SNP_F64", "SNP_OPT_FULL_PAIR_LOOP", "SNP_OPT_NO_CULLING", "SNP_OPT_MAP_WARP", "SNP_OPT_MAP_BLOCK", "SNP_OPT_STAGED_COPIES"]
     src = tmp_path / "enums.c"
     src.write_text('#include <stdio.h>\n#include "snp_b200.h"\nint main(void) {\n' + "\n".join(f'printf("{n} %d\\n", (int){n});' for n in names) +
                    '\nprintf("DYN_FIELDS %d\\nSTAT_FIELDS %d\\nROBOT_FIELDS %d\\n", (int)SNP_DYN_FIELDS, (int)SNP_STAT_FIELDS, (int)SNP_ROBOT_FIELDS);\nreturn 0; }\n')
@@ -114,17 +113,34 @@ def test_operator_argument_validation_needs_no_gpu():
 
 
 def test_large_crowd_scratch_size_covers_every_region():
-    """snp_large_scratch_bytes is host arithmetic (no GPU): it must cover the per-chunk partial sums, the tile boxes, the live map,
-    the list of (agent block, chunk) units, the per-block ascending lists and the queue counters -- for whole and ragged sizes."""
+    """snp_large_scratch_bytes is host arithmetic (no GPU): it must cover the per-chunk partial sums, the live map, the list of
+    (agent block, chunk) units, the per-block ascending lists and the queue counters -- for whole and ragged sizes."""
     from social_navigation_pyenvs_b200 import _lib as L
     lib = L.lib()
     for n_local, M in ((8192, 65536), (65536, 65536), (5184, 5184), (1, 2), (130, 1000)):
         for dtype, w in ((L.SNP_F64, 8), (L.SNP_F32, 4)):
-            J, tiles, blocks = -(-M // 128), -(-M // 128), -(-n_local // 128)
+            J, blocks = -(-M // 128), -(-n_local // 128)
             Jp = (J + 15) // 16 * 16
-            need = w * (J * 2 * n_local + tiles * 5) + blocks * Jp + 4 * (260 + blocks * J + (blocks + 3) // 4 * 4 + blocks * Jp) + 64
+            need = w * J * 2 * n_local + blocks * Jp + 4 * (260 + blocks * J + blocks + blocks * Jp)
             got = int(lib.snp_large_scratch_bytes(n_local, M, dtype))
-            assert need <= got <= need + 4096 + 4 * blocks * Jp, (n_local, M, dtype, need, got)
+            assert need <= got <= need + 4 * 16, (n_local, M, dtype, need, got)  # (at most 15 bytes of alignment per region)
+
+
+def test_large_crowd_step_rejects_bad_slices_and_rank_counts_before_any_launch():
+    """snp_large_run_p2p validates on the host: a slice reaching past the view (offset + N = M + 1) or a world outside 1..8 is
+    SNP_ERR_INVALID before anything touches the device (the pointers are dummies)."""
+    from social_navigation_pyenvs_b200 import _lib as L
+    lib = L.lib()
+    dummy = ctypes.c_void_p(4096)
+    c = L.SnpCrowd(E=1, N=256, G=2, dtype=L.SNP_F64, dyn=dummy, stat=dummy, goals=dummy, goal_idx=dummy, goal_cnt=dummy)
+    o = L.SnpStepOpts(type=3, dt=0.0125)
+    for offset, M, world, rank in ((1, 256, 1, 0), (257, 512, 1, 0), (0, 256, 0, 0), (0, 2304, 9, 0), (0, 512, 2, 2)):
+        views = (ctypes.c_void_p * 9)(*[4096] * 9)
+        n_bytes = int(lib.snp_large_scratch_bytes(256, M, L.SNP_F64))
+        rc = lib.snp_large_run_p2p(ctypes.byref(c), ctypes.byref(o), views, views, 0, M, offset, world, rank, views, 0, 1, dummy, dummy,
+                                   n_bytes, None)
+        assert rc == -1, (offset, M, world, rank)
+        assert "snp_large_run_p2p" in lib.snp_last_error().decode()
 
 
 def test_product_package_never_imports_the_oracle():

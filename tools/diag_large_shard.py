@@ -15,9 +15,8 @@ if os.environ.get("SNP_LARGE_DEAL", "1") == "1":  # the bench's load balancing: 
 S, G = np.ascontiguousarray(sc["states"][0, perm]), np.ascontiguousarray(sc["goals"][0, perm])
 n = S.shape[0] // ways
 crowd = LargeCrowd("hsfm_farina", S, G, dtype=torch.float64, shard=(rank * n, n))
-# one sub-step per call: every call recomputes the tile boxes of the view it reads (in a real sharded run the other ranks' producers
-# write the boxes of their tiles; here the rest of the crowd is frozen and nobody would)
-crowd.work_list = os.environ.get("SNP_LARGE_GRID", "0") != "1"
+# a slice recomputes the tile boxes of the view it reads every sub-step (in a real sharded run the other ranks' producers write the
+# boxes of their tiles; here the rest of the crowd is frozen and nobody would): one launch more than a rank of a sharded run
 for _ in range(2):
     crowd.step(0.0125, 1)
 torch.cuda.synchronize()
@@ -26,4 +25,4 @@ a.record()
 for _ in range(10):
     crowd.step(0.0125, 1)
 b.record(); torch.cuda.synchronize()
-print(f"{ways}-way shard, rank {rank}: {a.elapsed_time(b) / 10:.4f} ms per sub-step ({crowd.exchange}, {'work list' if crowd.work_list else 'static grid'})")
+print(f"{ways}-way shard, rank {rank}: {a.elapsed_time(b) / 10:.4f} ms per sub-step ({crowd.exchange})")

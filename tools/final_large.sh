@@ -21,7 +21,7 @@ if [ $(stat -c %s $O/${R}_${name}.ncu-rep) -gt 8000000 ]; then rm -f $O/${R}_${n
 S=/usr/local/cuda/bin/compute-sanitizer
 : > $O/${R}_sanitizer_large.txt
 for tool in memcheck racecheck synccheck; do
-  echo "=== $tool: large crowd (cull kernel, work list, persistent pair CTAs, list-walking finish; static grid; all pairs)" >> $O/${R}_sanitizer_large.txt
+  echo "=== $tool: large crowd (cull kernel, work list, persistent pair CTAs, list-walking finish; culled static grid of an unaligned slice; all pairs)" >> $O/${R}_sanitizer_large.txt
   timeout 170 $S --tool $tool --error-exitcode 9 python -m pytest -q -m gpu -x "tests/test_gpu_sizes_large.py::test_large_crowd_chunked_sums_and_exact_culling" "tests/test_gpu_sizes_large.py::test_large_crowd_tiled_kernel_vs_oracle" 2>&1 | grep -E "ERROR SUMMARY|RACECHECK SUMMARY|passed|failed|Error|error" | tail -4 >> $O/${R}_sanitizer_large.txt
 done
 cat $O/final_gpu_tests.log $O/final_smoke.log $O/${R}_sanitizer_large.txt; wc -l $O/${R}_large_lines.jsonl
