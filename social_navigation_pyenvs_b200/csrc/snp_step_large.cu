@@ -5,15 +5,23 @@
 //                   (every sub-step, or -- when the producers of a call write every tile of the next view -- the first sub-step
 //                   of a call only: afterwards the finish kernel writes the boxes of the tiles it produces)
 //   pair phase      unit of work = (i-block of 128 or 256 agents, j-chunk of 128 entities): every agent accumulates the force of
-//                   the chunk's entities in ascending j from a shared-memory tile and writes ONE partial sum per chunk.  A chunk
-//                   is skipped when its box is farther from the i-block's box than the distance at which the pair law is
-//                   identically zero in the arithmetic in use (exp underflow: r_i+s_i+r_j+s_j + 700 B in fp64, + 88 B in fp32
-//                   with ex2.approx.ftz) -- an EXACT optimisation, the summed force is unchanged.
+//                   the chunk's entities in ascending j from a shared-memory tile and writes ONE partial sum per chunk.  A tile
+//                   is skipped when its box is farther from the i-block's box than reach = max(r+s) of the i-block + max(r+s)
+//                   of the tile + 700 B in fp64, + 88 B in fp32 (Guo: max(B, D)).  Beyond that every exponential of the pair
+//                   law is below e^-700 (fp64) / e^-88 (fp32) times its amplitude, so a skipped pair contributes at most about
+//                   A e^-700 ~ 2e-301 (fp64; the exponent clamp of exp2_scaled_times keeps even far pairs near 2^-1010) or
+//                   A e^-88 ~ 1.2e-35 and C e^-88 ~ 7e-37 (fp32: normal floats, not flushed by ex2.approx.ftz) -- NOT an
+//                   identically zero force.  Any other force on the agent absorbs terms that small, so culling on and off agree
+//                   bit for bit in practice; only an agent with no other force in reach sees them.
 //                     all pairs:  k_large_pairs on the static (i-block, chunk) grid;
 //                     culled:     k_large_cull lists the units in reach, persistent k_large_pairs_list CTAs work the list off.
 //   k_large_finish  per agent: partial sums of the live chunks added in ascending chunk order (fixed, so the result does not depend
 //                   on how the crowd is sharded over GPUs), goal switch, wall force, desired force, torque, Euler; writes the
 //                   state in place and the agent's entry (and its tile's box) of the NEXT entity view -- on every rank.
+//
+// Invariant: a chunk the finish kernel adds was written in this sub-step.  On the static grid a unit that culled every tile says
+// so in `live` and the finish kernel skips it; every unit on the work list writes its partial sums, zeros when it culled every
+// tile (k_large_cull builds the i-block's box from tile boxes, which can be larger than the box of the slice's own agents).
 //
 // Small chunks matter once culling is on and the crowd is sharded: only a few percent of the units have anything to evaluate, and
 // what one rank of an 8-way split keeps must still fill 148 SMs evenly (history: 4096-entity chunks 2.6 ms per sub-step at 65536
@@ -113,7 +121,7 @@ template <typename T> __device__ __forceinline__ void iblock_box(const LargeArgs
             u[0] = min(u[0], b[0]); u[1] = max(u[1], b[1]); u[2] = min(u[2], b[2]); u[3] = max(u[3], b[3]); u[4] = max(u[4], b[4]);
         }
 }
-// Is any tile of chunk `chunk` within reach of the box u?  (Beyond reach the pair law is identically zero.)
+// Is any tile of chunk `chunk` within reach of the box u?  (Beyond reach the pair law is below the bound in the header.)
 template <typename T> __device__ __forceinline__ bool chunk_near(const LargeArgs<T> &la, const T *u, int chunk) {
     const long long j_begin = (long long)chunk * kChunk, j_end = min(la.M, j_begin + kChunk);
     bool near = false;
@@ -265,7 +273,11 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
         }
     }
     if (threadIdx.x == 0) *live_flag = any_tile ? 1 : 0;
-    if (!any_tile) return;  // every tile was culled: the chunk contributes exactly zero and the finish kernel skips it
+    // Every tile culled: on the static grid the finish kernel reads `live` and skips the chunk, so nothing is written.  A unit on
+    // the work list is added whatever happened here, and k_large_cull listed it from the tile box of the i-block, which for the
+    // last, partly foreign tile of a slice ending inside the view is larger than the box of the agents tested above: such a unit
+    // writes its (zero) partial sums.
+    if (!any_tile && !la.use_list) return;
 #pragma unroll
     for (int q = 0; q < kAgentsPerThread; ++q)
         if (idx[q] < N) {
@@ -626,7 +638,7 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     la.work = (int *)(base + sc.work);
     la.live_cnt = (int *)(base + sc.live_cnt);
     la.live_list = (int *)(base + sc.live_list);
-    // exact culling distance beyond the r+s sums: where exp(rd/B) is identically zero in the arithmetic in use
+    // culling distance beyond the r+s sums: where exp(rd/B) has fallen below e^-700 (fp64) / e^-88 (fp32), see the header
     const int soc = o->type % 3;
     const double under = sizeof(T) == 8 ? 700.0 : 88.0;
     double margin = -1.0;

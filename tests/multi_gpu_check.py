@@ -39,6 +39,36 @@ for dtype, exchange in ((torch.float64, "nccl"), (torch.float32, "nccl"), (torch
         ref = single.local_rows(S)[sharded.offset:sharded.offset + sharded.n_local]
         assert np.array_equal(mine, ref), f"rank {rank}: sharded crowd differs from single-GPU crowd ({dtype}, {exchange}, single {single_exchange})"
 
+
+# ---- a ragged crowd sharded by agent: 5184 humans, 2592 per rank on 2 ranks and 648 on 8 -- not whole tiles, so the ranks exchange
+# over NCCL, and rank 0's slice starts on a tile and ends inside one that also holds rank 1's humans.  Scratch and tile boxes are
+# poisoned before every call, so a partial sum the sub-step did not write shows up as NaN. ----
+def poisoned_step(crowd, k):
+    crowd.scratch.fill_(0xFF)
+    for v in crowd._vbuf:
+        boxes = v[5 * crowd.n_total:].view(crowd._n_tiles, 5)
+        boxes[:, :4] = 1e30
+        boxes[:, 4] = 0.0
+    crowd.step(0.0125, n_substeps=k)
+
+
+sc = scenarios.jittered_grid_crowd(72, pitch=1.0, jitter=0.3, seed=3)
+S0, G0 = sc["states"][0], sc["goals"][0]
+S0[:, 5:7] = np.random.RandomState(1).uniform(-0.6, 0.6, (S0.shape[0], 2))
+for order in ("row", "patch"):
+    perm = scenarios.spatial_order(S0[:, 0:2]) if order == "patch" else np.arange(S0.shape[0])
+    S, G = np.ascontiguousarray(S0[perm]), np.ascontiguousarray(G0[perm])
+    for dtype in (torch.float64, torch.float32):
+        sharded = LargeCrowd("hsfm_farina", S, G, dtype=dtype, rank=rank, world=world)
+        assert sharded.exchange == "nccl" and sharded.n_local % 128 != 0
+        poisoned_step(sharded, 3)
+        poisoned_step(sharded, 2)
+        mine = sharded.local_rows(S[sharded.offset:sharded.offset + sharded.n_local])
+        single = LargeCrowd("hsfm_farina", S, G, dtype=dtype, rank=0, world=1)
+        poisoned_step(single, 5)
+        ref = single.local_rows(S)[sharded.offset:sharded.offset + sharded.n_local]
+        assert np.array_equal(mine, ref), f"rank {rank}: ragged sharded crowd differs from single-GPU crowd ({dtype}, {order} order)"
+
 # ---- independent envs sharded by env: no collective on the data path ----
 states = np.concatenate([sc_env["states"], sc_env["robot"][:, None]], 1)
 sl = parallel.env_shard(64, rank, world)

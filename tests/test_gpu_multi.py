@@ -1,6 +1,8 @@
 """Multi-GPU parity (-m gpu, skipped with fewer than two GPUs): tests/multi_gpu_check.py under torchrun -- the agent-sharded
 LargeCrowd (fused peer-store exchange, NCCL all-gather) must equal the single-GPU crowd -- stepped in one call or one call per sub-step
-with the all-gather -- BIT FOR BIT, and env-sharded engines the slices of one big engine."""
+with the all-gather -- BIT FOR BIT, and env-sharded engines the slices of one big engine.  A ragged crowd (72 x 72 = 5184 humans,
+row and patch order, fp64 and fp32) splits into slices that are not whole 128-human tiles, so its ranks exchange over NCCL and
+rank 0's slice ends inside a tile shared with rank 1; its scratch is poisoned before every call."""
 import os
 import subprocess
 import sys
