@@ -30,7 +30,8 @@
  *   snp_robot_push_out                            <- src/robot_agent.py:35-48 RobotAgent.check_collisions (social_nav_sim.py:509)
  *   snp_reset                                     <- social_nav_gym.py:120-225 reset, social_nav_sim.py:200-431 scenario generators
  *   snp_pack_states / snp_unpack_states           <- src/agent.py:256-266 get_safe_state / set_state row layout
- *   snp_large_run_p2p                             <- same update for one very large crowd (tiled all-pairs)
+ *   snp_large_run_p2p                             <- same update for one very large crowd (tiled all-pairs), with its robot
+ *   snp_large_checks                              <- the checks above for the robot of one very large crowd
  */
 #ifndef SNP_B200_H
 #define SNP_B200_H
@@ -250,11 +251,24 @@ int snp_rotate_goal_rows(const snp_crowd *crowd, double *goal_rows_dev, void *cu
  * otherwise every sub-step recomputes the boxes of the view it reads (one more launch).  An exchange of its own (e.g. an all-gather
  * of the slices) runs between calls of one sub-step with world = 1.  `scratch` = 16-byte aligned device workspace of at least
  * snp_large_scratch_bytes(n_local, M, dtype) bytes (per-chunk partial sums, the map and lists of the (agent block, entity chunk)
- * units in reach, the work queues' counters).  opts->reserved bit 1 (SNP_OPT_NO_CULLING) disables the exact far-tile culling. */
+ * units in reach, the work queues' counters).  opts->reserved bit 1 (SNP_OPT_NO_CULLING) disables the exact far-tile culling.
+ * The robot of SocialNavGym.step (crowd->robot, one env): opts->robot_mode 0 (fixed), 1 (holonomic action) or 3 (unicycle action)
+ * moves it before every sub-step as snp_step does, and opts->consider_robot adds its pair force to every human (never culled).  Every
+ * rank recomputes the robot of each sub-step from crowd->robot, so no exchange is needed; after the last sub-step crowd->robot holds
+ * the end state and opts->time_now (optional) has advanced by dt per sub-step.  The checks are snp_large_checks.  robot_mode 2,
+ * track_touch, pre_checks / post_checks, dyn_out and respawn are SNP_ERR_UNSUPPORTED, before any launch. */
 int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype);
 int snp_large_run_p2p(const snp_crowd *crowd, const snp_step_opts *opts, const void *const *peer_views_a, const void *const *peer_views_b,
                       int32_t first_is_b, int64_t M, int64_t self_offset, int32_t world, int32_t rank, const void *const *peer_flags,
                       uint64_t epoch_base, int32_t n_substeps, int32_t *error_flag, void *scratch, int64_t scratch_bytes, void *cuda_stream);
+/* The collision / goal / reward checks of SocialNavGym.step for the robot crowd->robot (one env) against the M humans of a view
+ * buffer `view` [5][M] (x, y, vx, vy, r+safety; as snp_large_run_p2p reads and writes it) with radii `radius` [M], both in the
+ * crowd's dtype.  opts->pre_checks: the swept test over one robot step of length consts[5] with opts->action (v (cos, sin)(yaw + r)
+ * for robot_mode 3), stopping at the first colliding human in index order, dmin, the goal test and the reward / info code at
+ * opts->time_now (social_nav_sim.py:949-1029).  opts->post_checks = 1: actual dmin, collision and goal (social_nav_gym.py:107-118).
+ * Writes the bits and checks fields of the checks it runs into opts->flags[0] / opts->checks[0..3] (as snp_step; the other bits and
+ * fields are left as they are).  Double arithmetic, formula-exact; one CTA, no workspace, no host synchronisation. */
+int snp_large_checks(const snp_crowd *crowd, const snp_step_opts *opts, const void *view, const void *radius, int64_t M, void *cuda_stream);
 /* Writes this crowd's [5][.] entity view (x,y,vx,vy,r+safety; v = R(yaw) bv for headed models) into `view` (field stride
  * `stride` elements, starting at element `offset`). */
 int snp_large_publish(const snp_crowd *crowd, int32_t type, void *view, int64_t stride, int64_t offset, void *cuda_stream);

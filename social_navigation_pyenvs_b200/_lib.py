@@ -82,6 +82,7 @@ _SIGNATURES = {
     "snp_unpack_goals": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_void_p, c_void_p, c_void_p]),
     "snp_rotate_goal_rows": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_void_p, c_void_p]),
     "snp_large_scratch_bytes": (c_int64, [c_int64, c_int64, c_int32]),
+    "snp_large_checks": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_void_p, c_int64, c_void_p]),
     "snp_large_publish": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_int32, c_void_p, c_int64, c_int64, c_void_p]),
     "snp_large_run_p2p": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_void_p, c_int32, c_int64, c_int64, c_int32,
                                          c_int32, c_void_p, ctypes.c_uint64, c_int32, c_void_p, c_void_p, c_int64, c_void_p]),

@@ -18,6 +18,15 @@
 //   k_large_finish  per agent: partial sums of the live chunks added in ascending chunk order (fixed, so the result does not depend
 //                   on how the crowd is sharded over GPUs), goal switch, wall force, desired force, torque, Euler; writes the
 //                   state in place and the agent's entry (and its tile's box) of the NEXT entity view -- on every rank.
+//                   With a visible robot (a separate instantiation) the robot's pair force is added after the chunk sums.
+//   k_large_robot_end  after the last sub-step of a call, one thread: the robot's end state into crowd->robot, the clock advanced.
+//
+// The robot (SocialNavGym.step, social_nav_gym.py:240-245: robot.step, then update_humans, per sub-step) is entity M of the
+// reference's ordered loop, the last one: the finish kernel adds its pair force after every chunk, never culls it, and for
+// Moussaid's symmetric path the human is agent 1 (the robot has the highest index).  Its motion does not depend on the humans
+// (robot_mode 0 fixed, 1 holonomic, 3 unicycle), so every finish thread of every rank recomputes the robot of its sub-step from the
+// call's start state in crowd->robot with k_step's expressions: the same bits everywhere, no exchange and no scratch.
+// k_large_checks is the swept / actual check of the robot against a view of the whole crowd (snp_large_checks).
 //
 // Invariant: a chunk the finish kernel adds was written in this sub-step.  On the static grid a unit that culled every tile says
 // so in `live` and the finish kernel skips it; every unit on the work list writes its partial sums, zeros when it culled every
@@ -28,7 +37,7 @@
 // humans and no gain from a second GPU; 512: 2.0 / 1.1 ms; 256 + exact culling on compact tiles + one agent per thread: 0.75 ms on
 // one GPU, 0.158 on eight; 128 + the work list + grouped evaluation: 0.59 / 0.125).  The price is J = M/128 partial sums per LIVE chunk and agent.
 // Reference: same as snp_step_small.cu (motion_model_manager.py:354-373,424-459; forces.py:63-151).
-#include "snp_kernels.cuh"
+#include "snp_gym.cuh"
 
 namespace snp {
 namespace {
@@ -71,6 +80,7 @@ template <typename T> struct LargeArgs {
     int use_list;
     int *live_cnt, *live_list;  // per i-block: how many chunks are in reach, and which, ascending ([i-blocks], [i-blocks][Jp]) -- what the
                                 // finish kernel walks instead of scanning the flags
+    int robot_steps;  // robot.step calls of this call up to and including this sub-step's (0 for a fixed robot)
 };
 constexpr int kMaxQueues = 256;                 // one queue of list entries per SM (entry k belongs to queue k mod n_queues)
 constexpr int kWorkCounters = 4 + kMaxQueues;   // ints in front of the list
@@ -371,7 +381,29 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
     }
 }
 
-template <typename T, int OBS, int HEADED>
+// The robot after `steps` robot.step calls from the state in a.robot (robot_agent.py:116-136), with k_step's expressions: rb[] gets
+// SNP_ROBOT_PX, PY, VX, VY and TH.
+template <typename T> __device__ __forceinline__ void large_robot_replay(const KArgs<T> &a, int steps, T *rb) {
+    rb[SNP_ROBOT_PX] = a.robot[SNP_ROBOT_PX]; rb[SNP_ROBOT_PY] = a.robot[SNP_ROBOT_PY];
+    rb[SNP_ROBOT_VX] = a.robot[SNP_ROBOT_VX]; rb[SNP_ROBOT_VY] = a.robot[SNP_ROBOT_VY]; rb[SNP_ROBOT_TH] = a.robot[SNP_ROBOT_TH];
+    if (steps <= 0) return;
+    const T dt = a.dt;
+    if (a.robot_mode == 1) {  // holonomic: p = p + a*dt ; v = a
+        const T ax = a.action[0], ay = a.action[1];
+        T px = rb[SNP_ROBOT_PX], py = rb[SNP_ROBOT_PY];
+        for (int s = 0; s < steps; ++s) {
+            if (sizeof(T) == 8) { px = (T)__dadd_rn((double)px, __dmul_rn((double)ax, (double)dt)); py = (T)__dadd_rn((double)py, __dmul_rn((double)ay, (double)dt)); }
+            else { px = px + ax * dt; py = py + ay * dt; }
+        }
+        rb[SNP_ROBOT_PX] = px; rb[SNP_ROBOT_PY] = py; rb[SNP_ROBOT_VX] = ax; rb[SNP_ROBOT_VY] = ay;
+    } else if (a.robot_mode == 3) {  // unicycle (v, r)
+        for (int s = 0; s < steps; ++s) robot_unicycle_step<T>(rb, (double)a.action[0], (double)a.action[1], (double)dt);
+    }
+}
+
+// RSOC: the pair law of the visible robot's force (SOC of the humans' model), or -1 for no robot -- a separate instantiation, so
+// that the common ones keep their registers.
+template <typename T, int OBS, int HEADED, int RSOC>
 __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     using R = Real<T>;
     const KArgs<T> &a = la.k;
@@ -381,7 +413,7 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     constexpr size_t kTbl = sizeof(double) * kExpN;
     Seg<T> *segs = reinterpret_cast<Seg<T> *>(smem_raw + kTbl);
     int *seg_cnt = reinterpret_cast<int *>(smem_raw + kTbl + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)));
-    if (sizeof(T) == 8 && nseg > 0) exp_table_init(exp_tbl_s);  // only the wall force evaluates exp here
+    if (sizeof(T) == 8 && (nseg > 0 || RSOC >= 0)) exp_table_init(exp_tbl_s);  // only the wall force and the robot evaluate exp here
     for (int k = threadIdx.x; k < nseg; k += blockDim.x) {
         const T *w = a.walls + (size_t)k * 4;
         segs[k] = make_seg<T>(w[0], w[1], w[2], w[3]);
@@ -472,6 +504,16 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
             for (int b = 0; b < 16; ++b)
                 if (on[b]) { fsx += vx[b]; fsy += vy[b]; }
         }
+    }
+    if constexpr (RSOC >= 0) {
+        // the robot: the last entity of the ordered loop, after every chunk; never culled (one pair per human)
+        T rb[SNP_ROBOT_FIELDS];
+        large_robot_replay<T>(a, la.robot_steps, rb);
+        const T rrs = a.robot[SNP_ROBOT_R] + a.robot[SNP_ROBOT_SAFETY];
+        T fx, fy;
+        pair_force<T, RSOC>(P, exp_tbl_s, vote_mask, m.px, m.py, m.vx, m.vy, m.rs, rb[SNP_ROBOT_PX], rb[SNP_ROBOT_PY], rb[SNP_ROBOT_VX],
+                            rb[SNP_ROBOT_VY], rrs, fx, fy);
+        fsx += fx; fsy += fy;
     }
 
     const T dg = np_norm(m.gx - m.px, m.gy - m.py);
@@ -580,7 +622,7 @@ template <typename T, int SOC, int OBS, int HEADED> int launch_large(const Large
     } else if (la.apt == 1) k_large_pairs<T, SOC, 1><<<grid, kTile, 0, st>>>(la);
     else k_large_pairs<T, SOC, 2><<<grid, kTile, 0, st>>>(la);
     const size_t smem = sizeof(double) * kExpN + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + sizeof(int) * (la.k.W + 1) + 16;
-    auto fin = k_large_finish<T, OBS, HEADED>;
+    auto fin = la.k.consider_robot ? k_large_finish<T, OBS, HEADED, SOC> : k_large_finish<T, OBS, HEADED, -1>;
     if (smem > 48 * 1024) SNP_CUDA_OK(cudaFuncSetAttribute(fin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     fin<<<(unsigned)((N + kTile - 1) / kTile), kTile, smem, st>>>(la);
     count_launch(la.boxes_ready ? 2 : 3);
@@ -610,9 +652,9 @@ inline LargeScratch large_scratch(long long n_local, long long M, long long elem
 
 // One sub-step: `cur` = the view buffer read ([5][M] entities + their [n_tiles][5] tile boxes), `next` = the n_peers buffers the
 // finish kernel stores the updated entries into, and their tile boxes too when `fold_boxes`.  `boxes_ready`: `cur`'s tile boxes
-// were written by the previous sub-step's producers.
+// were written by the previous sub-step's producers.  `sub`: index of the sub-step in the call (how far a moving robot has gone).
 template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, const void *cur, const void *const *next, int n_peers,
-                                    long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, cudaStream_t st) {
+                                    long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, int sub, cudaStream_t st) {
     LargeArgs<T> la;
     la.n_peers = n_peers;
     for (int p = 0; p < 8; ++p) la.peers[p] = (p < n_peers) ? (T *)next[p] : nullptr;
@@ -621,11 +663,12 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     KArgs<T> &a = la.k;
     a.E = 1; a.N = 0; a.G = c->G; a.EN = (long long)c->E * c->N;
     a.dyn = (T *)c->dyn; a.stat = (const T *)c->stat; a.goals = (const T *)c->goals; a.goal_idx = c->goal_idx; a.goal_cnt = c->goal_cnt;
-    a.agent_params = nullptr; a.P = make_params<T>(c->params); a.robot = nullptr;
+    a.agent_params = nullptr; a.P = make_params<T>(c->params); a.robot = (T *)c->robot;
     a.walls = (const T *)c->walls; a.W = c->W; a.S = c->W > 0 ? c->S : 0; a.walls_per_env = 0;
-    a.consider_robot = 0; a.symmetric = o->symmetric; a.numba = o->numba_compat; a.n_substeps = 1; a.robot_mode = 0;
-    a.dt = (T)o->dt; a.dt_d = o->dt; a.action = nullptr; a.pre_checks = a.post_checks = a.track_touch = 0;
+    a.consider_robot = o->consider_robot; a.symmetric = o->symmetric; a.numba = o->numba_compat; a.n_substeps = 1; a.robot_mode = o->robot_mode;
+    a.dt = (T)o->dt; a.dt_d = o->dt; a.action = (const T *)o->action; a.pre_checks = a.post_checks = a.track_touch = 0;
     a.time_now = nullptr; a.flags = nullptr; a.checks = nullptr; a.epw = 1; a.gpb = 1; a.mapping = 0; a.full_pair_loop = 1; a.respawn = 0; a.robot_type = 0; a.RP = a.P; a.robot_every = 0; a.robot_phase = 0; a.robot_dt = T(0);
+    la.robot_steps = (o->robot_mode == 1 || o->robot_mode == 3) ? sub + 1 : 0;
     la.others = (const T *)cur; la.M = M; la.self_offset = self_offset;
     la.boxes = (T *)cur + 5 * M;
     la.J = (int)large_J(M); la.n_tiles = (int)large_tiles(M);
@@ -666,6 +709,125 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     return SNP_ERR_INVALID;
 }
 
+// After the last sub-step of a call: the robot's end state (robot_mode 1 / 3; the finish kernels of the call read the start state
+// until they are done) and the clock, advanced by dt per sub-step as k_step does.  One thread.
+template <typename T> __global__ void k_large_robot_end(const KArgs<T> a, int n_substeps) {
+    if (a.robot && (a.robot_mode == 1 || a.robot_mode == 3)) {
+        T rb[SNP_ROBOT_FIELDS];
+        large_robot_replay<T>(a, n_substeps, rb);
+        a.robot[SNP_ROBOT_PX] = rb[SNP_ROBOT_PX]; a.robot[SNP_ROBOT_PY] = rb[SNP_ROBOT_PY];
+        a.robot[SNP_ROBOT_VX] = rb[SNP_ROBOT_VX]; a.robot[SNP_ROBOT_VY] = rb[SNP_ROBOT_VY]; a.robot[SNP_ROBOT_TH] = rb[SNP_ROBOT_TH];
+    }
+    if (a.time_now) {
+        double t = a.time_now[0];
+        for (int s = 0; s < n_substeps; ++s) t = __dadd_rn(t, a.dt_d);
+        a.time_now[0] = t;
+    }
+}
+
+// ---- snp_large_checks: the robot against M humans of a view (social_nav_sim.py:949-1029, social_nav_gym.py:107-118) ----
+// One CTA.  Thread t scans the contiguous run [t * per, (t + 1) * per) in index order; the runs are combined in index order (a shuffle
+// tree that only ever puts a run's summary to the LEFT of the next one's, then the same over the warps), so the result is that of
+// the reference's sequential loop: the swept test stops at the first colliding human and dmin is the minimum over the humans before
+// it, the first of equal minima kept ('<'), NaN distances never taken.
+constexpr int kCheckThreads = 1024;
+
+template <typename T> struct CheckArgs {
+    const T *robot, *action, *view, *radius;
+    long long M;
+    int mode, pre, post;
+    double consts[6];
+    const double *time_now;
+    int *flags;
+    double *checks;
+};
+
+// (dmin, hit) of a run on the left combined with the run on its right
+__device__ __forceinline__ void swept_combine(double &dmin, int &hit, double dmin_r, int hit_r) {
+    if (hit) return;
+    dmin = dmin_r < dmin ? dmin_r : dmin;
+    hit = hit_r;
+}
+
+template <typename T> __global__ void __launch_bounds__(kCheckThreads) k_large_checks(const CheckArgs<T> c) {
+    __shared__ double s_dmin[kCheckThreads / 32], s_admin[kCheckThreads / 32];
+    __shared__ int s_hit[kCheckThreads / 32];
+    const T *rbt = c.robot;
+    const T rpx = rbt[SNP_ROBOT_PX], rpy = rbt[SNP_ROBOT_PY], rr = rbt[SNP_ROBOT_R], rgx = rbt[SNP_ROBOT_GX], rgy = rbt[SNP_ROBOT_GY];
+    T ax = T(0), ay = T(0);
+    if (c.pre) {
+        ax = c.action[0]; ay = c.action[1];
+        if (c.mode == 3) {  // unicycle action (v, r): the swept test and the goal test use v (cos, sin)(yaw + r) (sim:973)
+            const double uv = (double)ax, ur = (double)ay;
+            double sn_, cs_;
+            sincos((double)rbt[SNP_ROBOT_TH] + ur, &sn_, &cs_);
+            ax = (T)__dmul_rn(uv, cs_); ay = (T)__dmul_rn(uv, sn_);
+        }
+    }
+    const long long M = c.M, per = (M + kCheckThreads - 1) / kCheckThreads;
+    const long long b = (long long)threadIdx.x * per, e = min(M, b + per);
+    const T *px = c.view, *py = c.view + M, *vx = c.view + 2 * M, *vy = c.view + 3 * M;
+    double dmin = CUDART_INF, admin = 10000.0;
+    int hit = 0;
+    if (c.pre)
+        for (long long k = b; k < e; ++k) {
+            const double cd = swept_distance((double)px[k], (double)py[k], (double)vx[k], (double)vy[k], (double)c.radius[k], (double)rpx, (double)rpy,
+                                             (double)rr, (double)ax, (double)ay, c.consts[5]);
+            if (cd < 0) { hit = 1; break; }
+            else if (cd < dmin) dmin = cd;
+        }
+    if (c.post)
+        for (long long k = b; k < e; ++k) {
+            double d = __dsub_rn(__dsub_rn(xnorm_np(__dsub_rn((double)px[k], (double)rpx), __dsub_rn((double)py[k], (double)rpy)), (double)c.radius[k]), (double)rr);
+            if (!(d < 10000.0)) d = 10000.0;
+            admin = d < admin ? d : admin;
+        }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int off = 1; off < 32; off <<= 1) {  // lane l ends up with the runs of lanes [l, l + 2 off) in order
+        const double dr = __shfl_down_sync(0xffffffffu, dmin, off), ar = __shfl_down_sync(0xffffffffu, admin, off);
+        const int hr = __shfl_down_sync(0xffffffffu, hit, off);
+        if (lane + off < 32) { swept_combine(dmin, hit, dr, hr); admin = ar < admin ? ar : admin; }
+    }
+    if (lane == 0) { s_dmin[warp] = dmin; s_admin[warp] = admin; s_hit[warp] = hit; }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    dmin = CUDART_INF; admin = 10000.0; hit = 0;
+    for (int w = 0; w < kCheckThreads / 32; ++w) { swept_combine(dmin, hit, s_dmin[w], s_hit[w]); admin = s_admin[w] < admin ? s_admin[w] : admin; }
+    int f = *c.flags;
+    if (c.pre) {
+        const double endx = __dadd_rn((double)rpx, __dmul_rn((double)ax, c.consts[5]));
+        const double endy = __dadd_rn((double)rpy, __dmul_rn((double)ay, c.consts[5]));
+        const bool goal = xnorm_np(__dsub_rn(endx, (double)rgx), __dsub_rn(endy, (double)rgy)) < (double)rr;
+        const double tnow = c.time_now ? c.time_now[0] : 0.0;
+        double reward;
+        bool term, trunc;
+        const int code = reward_and_info(hit != 0, dmin, goal, tnow, c.consts, reward, term, trunc);
+        f &= ~(SNP_FLAG_COLLISION | SNP_FLAG_REACHING_GOAL | SNP_FLAG_TERMINATED | SNP_FLAG_TRUNCATED | (7 << SNP_FLAG_INFO_SHIFT));
+        f |= (hit ? SNP_FLAG_COLLISION : 0) | (goal ? SNP_FLAG_REACHING_GOAL : 0) | (term ? SNP_FLAG_TERMINATED : 0) | (trunc ? SNP_FLAG_TRUNCATED : 0) |
+             (code << SNP_FLAG_INFO_SHIFT);
+        if (c.checks) { c.checks[0] = dmin; c.checks[1] = reward; }
+    }
+    if (c.post) {
+        const bool agoal = xnorm_np(__dsub_rn((double)rpx, (double)rgx), __dsub_rn((double)rpy, (double)rgy)) < (double)rr;
+        f &= ~(SNP_FLAG_ACTUAL_COLLISION | SNP_FLAG_ACTUAL_GOAL);
+        f |= (admin <= 0.0 ? SNP_FLAG_ACTUAL_COLLISION : 0) | (agoal ? SNP_FLAG_ACTUAL_GOAL : 0);
+        if (c.checks) c.checks[2] = admin;
+    }
+    *c.flags = f;
+}
+
+template <typename T> int launch_large_checks(const snp_crowd *cr, const snp_step_opts *o, const void *view, const void *radius, long long M, cudaStream_t st) {
+    CheckArgs<T> c;
+    c.robot = (const T *)cr->robot; c.action = (const T *)o->action; c.view = (const T *)view; c.radius = (const T *)radius; c.M = M;
+    c.mode = o->robot_mode; c.pre = o->pre_checks != 0; c.post = o->post_checks != 0;
+    for (int k = 0; k < 6; ++k) c.consts[k] = o->consts[k];
+    c.time_now = o->time_now; c.flags = o->flags; c.checks = o->checks;
+    k_large_checks<T><<<1, kCheckThreads, 0, st>>>(c);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    return SNP_OK;
+}
+
 }  // namespace
 }  // namespace snp
 
@@ -685,6 +847,15 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
     if (!c->dyn || !c->stat || !c->goals || !c->goal_idx || !c->goal_cnt) { set_error("snp_large_run_p2p: crowd arrays missing"); return SNP_ERR_INVALID; }
     if (c->agent_params || c->walls_per_env) { set_error("snp_large_run_p2p: uniform parameters and one wall set only"); return SNP_ERR_UNSUPPORTED; }
     if (c->dtype != SNP_F64 && c->dtype != SNP_F32) { set_error("bad dtype %d", c->dtype); return SNP_ERR_INVALID; }
+    // the robot of SocialNavGym.step: fixed (0), holonomic (1) or unicycle (3), visible or not; the checks are a call of their own
+    if (o->robot_mode < 0 || o->robot_mode > 3) { set_error("snp_large_run_p2p: robot_mode must be 0, 1 or 3 (got %d)", o->robot_mode); return SNP_ERR_INVALID; }
+    if (o->robot_mode == 2) { set_error("snp_large_run_p2p: robot_mode 2 (a robot moved by its own motion model) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->track_touch) { set_error("snp_large_run_p2p: track_touch is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->pre_checks || o->post_checks) { set_error("snp_large_run_p2p: run the collision / goal checks with snp_large_checks"); return SNP_ERR_UNSUPPORTED; }
+    if (o->dyn_out) { set_error("snp_large_run_p2p: dyn_out (peek) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->respawn) { set_error("snp_large_run_p2p: respawn is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if ((o->consider_robot || o->robot_mode) && !c->robot) { set_error("snp_large_run_p2p: consider_robot / robot_mode need crowd->robot"); return SNP_ERR_INVALID; }
+    if (o->robot_mode && !o->action) { set_error("snp_large_run_p2p: robot_mode %d needs opts->action", o->robot_mode); return SNP_ERR_INVALID; }
     const long long N = (long long)c->E * c->N;
     if (self_offset < 0 || self_offset + N > M) { set_error("snp_large_run_p2p: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
     const long long need = large_scratch(N, M, c->dtype == SNP_F64 ? 8 : 4).bytes;
@@ -703,8 +874,8 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
     for (int s = 0; s < n_substeps; ++s) {
         const void *const *cur = cur_is_b ? peer_views_b : peer_views_a, *const *nxt = cur_is_b ? peer_views_a : peer_views_b;
         const bool boxes_ready = fold_boxes && s > 0;  // sub-step 0 computes the tile boxes of the view it was handed
-        const int rc = c->dtype == SNP_F64 ? run_large<double>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, st)
-                                           : run_large<float>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, st);
+        const int rc = c->dtype == SNP_F64 ? run_large<double>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st)
+                                           : run_large<float>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st);
         if (rc) return rc;
         if (world > 1) {
             b.epoch = epoch_base + (unsigned long long)s + 1;
@@ -714,7 +885,35 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
         }
         cur_is_b ^= 1;
     }
+    // the robot's end state and the clock: after every finish kernel of the call has read the start state
+    if (n_substeps > 0 && ((c->robot && (o->robot_mode == 1 || o->robot_mode == 3)) || o->time_now)) {
+        if (c->dtype == SNP_F64) {
+            KArgs<double> a{}; a.robot = (double *)c->robot; a.action = (const double *)o->action; a.robot_mode = o->robot_mode;
+            a.dt = o->dt; a.dt_d = o->dt; a.time_now = o->time_now;
+            k_large_robot_end<double><<<1, 1, 0, st>>>(a, n_substeps);
+        } else {
+            KArgs<float> a{}; a.robot = (float *)c->robot; a.action = (const float *)o->action; a.robot_mode = o->robot_mode;
+            a.dt = (float)o->dt; a.dt_d = o->dt; a.time_now = o->time_now;
+            k_large_robot_end<float><<<1, 1, 0, st>>>(a, n_substeps);
+        }
+        count_launch();
+        SNP_CUDA_OK(cudaGetLastError());
+    }
     return SNP_OK;
+}
+
+int snp_large_checks(const snp_crowd *c, const snp_step_opts *o, const void *view, const void *radius, int64_t M, void *stream) {
+    if (!c || !o || !view || !radius) { set_error("snp_large_checks: null argument"); return SNP_ERR_INVALID; }
+    if (c->dtype != SNP_F64 && c->dtype != SNP_F32) { set_error("snp_large_checks: bad dtype %d", c->dtype); return SNP_ERR_INVALID; }
+    if (M < 1) { set_error("snp_large_checks: M must be >= 1 (got %lld)", (long long)M); return SNP_ERR_INVALID; }
+    if (!c->robot) { set_error("snp_large_checks: crowd->robot is required"); return SNP_ERR_INVALID; }
+    if (!o->pre_checks && !o->post_checks) { set_error("snp_large_checks: neither pre_checks nor post_checks is set"); return SNP_ERR_INVALID; }
+    if (o->post_checks != 0 && o->post_checks != 1) { set_error("snp_large_checks: post_checks 2 (imitation-learning reward) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->robot_mode != 0 && o->robot_mode != 1 && o->robot_mode != 3) { set_error("snp_large_checks: robot_mode must be 0, 1 or 3 (got %d)", o->robot_mode); return SNP_ERR_INVALID; }
+    if (o->pre_checks && !o->action) { set_error("snp_large_checks: pre_checks needs opts->action"); return SNP_ERR_INVALID; }
+    if (!o->flags) { set_error("snp_large_checks: opts->flags is required"); return SNP_ERR_INVALID; }
+    return c->dtype == SNP_F64 ? launch_large_checks<double>(c, o, view, radius, M, (cudaStream_t)stream)
+                               : launch_large_checks<float>(c, o, view, radius, M, (cudaStream_t)stream);
 }
 
 int snp_large_publish(const snp_crowd *c, int32_t type, void *view, int64_t stride, int64_t offset, void *stream) {

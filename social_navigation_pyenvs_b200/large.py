@@ -4,6 +4,16 @@ Every rank owns a contiguous slice of agents and evaluates their forces against 
 symmetric accumulation, forces.py:148, is not carried across ranks).  The only exchange per sub-step is an all-gather of the
 entity view (x, y, vx, vy, r+safety) over NCCL / NVLink; it is double buffered so the step kernel writes the next view's own
 slice while reading the current one.  Reference semantics: motion_model_manager.py:354-373 for a single env.
+
+With a robot (`robot=`), `step` is SocialNavGym.step (social_nav_gym.py:227-250) for the one env: the swept collision / goal / reward
+check, then n_substeps x (robot.step; update_humans), then optionally the actual check; `scan` is the robot's laser.  The robot is
+fixed, holonomic or unicycle (no motion model), visible to the humans or not.  Every rank keeps the robot and recomputes it
+identically, so the flags and the robot are the same on every rank.
+
+The checks read the humans from the entity view: positions, radii and the velocity the humans exert force with -- R(yaw) bv for
+headed models.  That is the stored velocity for every state the engine produces and after every reset; it can differ only for rows
+the engine did not produce, until their first step -- including rows whose velocity was computed as R(yaw) bv on the host (a host
+cos / sin can differ from the device's in the last bit).
 """
 import ctypes
 
@@ -17,10 +27,12 @@ from .parallel import all_gather_columns, agent_shard
 
 class LargeCrowd:
     def __init__(self, model, states, goals, walls=None, dtype=torch.float64, device="cuda", symmetric=True, numba_compat=False,
-                 rank=0, world=1, group=None, safety=None, exchange="auto", shard=None):
+                 rank=0, world=1, group=None, safety=None, exchange="auto", shard=None, robot=None, robot_safety=None, consider_robot=False):
         """states [N_total,13], goals [N_total,G,2] (the WHOLE crowd on every rank; each rank keeps its slice).
         shard=(offset, n_local) with world=1 steps only that slice against a frozen rest of the crowd (profiling what ONE rank of
-        a sharded run executes, on one GPU)."""
+        a sharded run executes, on one GPU).
+        robot: the robot's 13-wide reference row (robot.get_safe_state(), as CrowdEngine.set_robot_rows), robot_safety its safety
+        space (default 0); consider_robot: the humans feel its force (motion_model_manager.py:35)."""
         states = np.asarray(states, np.float64)
         goals = np.asarray(goals, np.float64)
         self.n_total = states.shape[0]
@@ -28,8 +40,17 @@ class LargeCrowd:
         self.offset, self.n_local = agent_shard(self.n_total, rank, world) if shard is None else shard
         sl = slice(self.offset, self.offset + self.n_local)
         saf = None if safety is None else np.asarray(safety, np.float64)[None, sl]
+        if consider_robot and robot is None:
+            raise ValueError("consider_robot needs a robot row")
         self.eng = CrowdEngine.from_reference_arrays(model, states[None, sl], goals[None, sl], walls=walls, safety=saf, consider_robot=False,
                                                      all_params_equal=symmetric, numba_compat=numba_compat, dtype=dtype, device=device)
+        self.has_robot = robot is not None
+        if self.has_robot:
+            self.eng.robot = torch.zeros((L.ROBOT_FIELDS, 1), dtype=dtype, device=self.eng.device)
+            self.eng.set_robot_rows(np.asarray(robot, np.float64).reshape(1, 13), safety=[0.0 if robot_safety is None else float(robot_safety)])
+            self.eng.consider_robot = bool(consider_robot)  # the robot is not a row of `states`: only the step options carry it
+            # the radii of the WHOLE crowd (the checks and the laser see every human)
+            self.radius = torch.as_tensor(states[:, 8], dtype=dtype, device=self.eng.device)
         self.type = SFMS.index(model)
         # exchange of the entity view between ranks: "p2p" = the producer kernel stores into every rank's next view through
         # peer-mapped (torch symmetric memory, NVLink) pointers and only a barrier separates sub-steps; "nccl" = all-gather
@@ -99,9 +120,28 @@ class LargeCrowd:
                                                self.offset, self._stream()))
         self._gather(v)
 
-    def step(self, dt=0.0125, n_substeps=1):
+    def step(self, dt=0.0125, n_substeps=1, action=None, kinematics="holonomic", pre_checks=False, post_checks=False):
+        """n_substeps updates of the crowd.  With a robot: SocialNavGym.step -- the swept check on the current state (pre_checks),
+        n_substeps x (robot.step(action, dt); update_humans(dt)), the actual check on the end state (post_checks); the clock
+        (eng.time_now) advances by dt per sub-step.  action (vx, vy), or (v, r) with kinematics="unicycle"; None keeps the robot
+        where it is (and the swept check sweeps a robot at rest).  Results: decode_flags(), robot_rows()."""
+        if kinematics not in ("holonomic", "unicycle"):
+            raise ValueError("kinematics must be 'holonomic' or 'unicycle'")
+        mode = 0
+        if self.has_robot:
+            if action is None:
+                self.eng.action.zero_()
+            else:
+                self.eng.action.copy_(torch.as_tensor(np.asarray(action, np.float64).reshape(2, 1), dtype=self.eng.dtype))
+                mode = 1 if kinematics == "holonomic" else 3
+            self.eng.flags.zero_()
+            self.eng.checks.zero_()
+        elif action is not None or pre_checks or post_checks:
+            raise ValueError("this crowd has no robot: build it with robot=")
+        if pre_checks:
+            self._checks(dt, mode, pre=True)
         c = self.eng._crowd()
-        o = self.eng._opts(dt, 1)
+        o = self.eng._opts(dt, 1, robot_mode=mode, advance_time=self.has_robot)
         o.reserved = 0 if self.culling else L.SNP_OPT_NO_CULLING
         # p2p / fused: the whole sub-step loop in ONE C call, nothing returns to Python in between; nccl: one sub-step per call on
         # this rank's own buffers, then the all-gather of the next view
@@ -116,6 +156,45 @@ class LargeCrowd:
             self.cur ^= k & 1
             if nccl:
                 self._gather(self.view[self.cur])
+        if post_checks:
+            self._checks(dt, mode, pre=False)
+
+    def _checks(self, dt, mode, pre):
+        o = self.eng._opts(dt, 0, robot_mode=mode, pre_checks=pre, post_checks=not pre)
+        L.check(self.eng.lib.snp_large_checks(ctypes.byref(self.eng._crowd()), ctypes.byref(o), ctypes.c_void_p(self.view[self.cur].data_ptr()),
+                                              ctypes.c_void_p(self.radius.data_ptr()), self.n_total, self._stream()))
+
+    def decode_flags(self):
+        """The checks of the last step (CrowdEngine.decode_flags for the one env: arrays of length 1)."""
+        return self.eng.decode_flags()
+
+    def robot_rows(self):
+        """The robot as a 13-wide reference row."""
+        return self.eng.robot_rows()[0][0]
+
+    def scan(self, range_, samples, max_distance, robot_radius=0.0):
+        """The robot's laser (LaserSensor.get_laser_measurements, robot_agent.py:77-82) over the whole crowd and the walls: one
+        snp_laser launch.  Returns device tensors (ranges [samples] in the crowd's dtype, hits [samples] int32: the global human
+        index, M + the wall segment's ordinal, or -1)."""
+        if not self.has_robot:
+            raise ValueError("this crowd has no robot: build it with robot=")
+        if max_distance > 10:
+            raise ValueError("Maxium distance for laser is 10 meters")  # sensors.py:13
+        e = self.eng
+        pose = e.robot[[L.ROBOT_PX, L.ROBOT_PY, L.ROBOT_TH]].contiguous()
+        ranges = torch.empty((int(samples),), dtype=e.dtype, device=e.device)
+        hits = torch.empty((int(samples),), dtype=torch.int32, device=e.device)
+        v = self.view[self.cur]
+        a = L.SnpLaserArgs()
+        a.E, a.N, a.samples = 1, self.n_total, int(samples)
+        a.dtype = L.SNP_F64 if e.dtype == torch.float64 else L.SNP_F32
+        a.px, a.py, a.radius = v[0].data_ptr(), v[1].data_ptr(), self.radius.data_ptr()
+        a.walls = None if e.walls is None else e.walls.data_ptr()
+        a.W, a.S, a.walls_per_env = e.W, e.S, 0
+        a.pose, a.range, a.max_distance, a.robot_radius = pose.data_ptr(), float(range_), float(max_distance), float(robot_radius)
+        a.ranges, a.hits = ranges.data_ptr(), hits.data_ptr()
+        L.check(e.lib.snp_laser(ctypes.byref(a), self._stream()))
+        return ranges, hits
 
     def local_rows(self, template):
         """This rank's agents as reference rows; `template` [n_local,13] supplies the static columns."""
