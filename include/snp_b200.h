@@ -269,6 +269,23 @@ int snp_large_run_p2p(const snp_crowd *crowd, const snp_step_opts *opts, const v
  * Writes the bits and checks fields of the checks it runs into opts->flags[0] / opts->checks[0..3] (as snp_step; the other bits and
  * fields are left as they are).  Double arithmetic, formula-exact; one CTA, no workspace, no host synchronisation. */
 int snp_large_checks(const snp_crowd *crowd, const snp_step_opts *opts, const void *view, const void *radius, int64_t M, void *cuda_stream);
+/* SocialNavGym.step (social_nav_gym.py:227-250) for E environments of N humans each, any N >= 1 (snp_step's limit is 512), through
+ * the tiled kernels of snp_large_run_p2p with an environment axis: tiles, chunks and agent blocks are per env, so a human only ever
+ * meets humans of its own env, and env e's result is bit for bit that of snp_large_run_p2p / snp_large_checks on env e alone.  One
+ * call, all enqueued on `cuda_stream` without host synchronisation: the entity view is published from crowd->dyn (as
+ * snp_large_publish: v = R(yaw) bv for headed models), the swept
+ * pre-checks run (opts->pre_checks), then n_substeps x (robot step; tiled update), the robot's end state and the clock
+ * (opts->time_now, optional, [E]), and the actual post-checks (opts->post_checks = 1).  Honours type, consider_robot, symmetric,
+ * numba_compat, n_substeps, robot_mode 0 / 1 / 3, action [2][E], dt, consts, flags [E], checks [E][4] and reserved bit 1
+ * (SNP_OPT_NO_CULLING); crowd->robot is [SNP_ROBOT_FIELDS][E]; walls are shared or per env (walls_per_env).  When a check runs the
+ * env's flags and checks are rewritten from zero (as snp_step); otherwise they are left as they are.  `scratch` = 16-byte aligned
+ * device workspace of at least snp_large_batch_scratch_bytes(E, N, dtype) bytes: the two view buffers, their tile boxes, the
+ * partial sums [ceil(N/128)][2][E*N], the live map and the work lists; nothing is carried from one call to the next.  Before any
+ * launch: robot_mode 2, robot_every, track_touch, post_checks 2, dyn_out, respawn and crowd->agent_params are SNP_ERR_UNSUPPORTED;
+ * bad E / N / G / dtype / type, missing arrays, a missing robot / action / flags and too small a scratch are SNP_ERR_INVALID.
+ * snp_large_batch_scratch_bytes returns -1 for bad arguments. */
+int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype);
+int snp_large_batch_step(const snp_crowd *crowd, const snp_step_opts *opts, void *scratch, int64_t scratch_bytes, void *cuda_stream);
 /* Writes this crowd's [5][.] entity view (x,y,vx,vy,r+safety; v = R(yaw) bv for headed models) into `view` (field stride
  * `stride` elements, starting at element `offset`). */
 int snp_large_publish(const snp_crowd *crowd, int32_t type, void *view, int64_t stride, int64_t offset, void *cuda_stream);

@@ -5,3 +5,4 @@ include/snp_b200.h.  Importing the package does not need a GPU; calling into it 
 """
 from .engine import CrowdEngine, SFMS, model_parameters  # noqa: F401
 from .forces_parallel import update_humans_parallel  # noqa: F401
+from .large import TiledCrowdEngine  # noqa: F401

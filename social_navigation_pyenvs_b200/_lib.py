@@ -86,7 +86,9 @@ _SIGNATURES = {
     "snp_large_publish": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_int32, c_void_p, c_int64, c_int64, c_void_p]),
     "snp_large_run_p2p": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_void_p, c_int32, c_int64, c_int64, c_int32,
                                          c_int32, c_void_p, ctypes.c_uint64, c_int32, c_void_p, c_void_p, c_int64, c_void_p]),
-    "snp_update_humans_parallel_host": (ctypes.c_int, [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
+    "snp_large_batch_scratch_bytes": (c_int64, [c_int32, c_int32, c_int32]),
+    "snp_large_batch_step": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_int64, c_void_p]),
+    "snp_update_humans_parallel_host":(ctypes.c_int, [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                                        c_void_p, c_double, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,
                                                        c_void_p, c_void_p]),
     "snp_laser_host": (ctypes.c_int, [c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_double, c_int32, c_double,

@@ -37,6 +37,8 @@
 // humans and no gain from a second GPU; 512: 2.0 / 1.1 ms; 256 + exact culling on compact tiles + one agent per thread: 0.75 ms on
 // one GPU, 0.158 on eight; 128 + the work list + grouped evaluation: 0.59 / 0.125).  The price is J = M/128 partial sums per LIVE chunk and agent.
 // Reference: same as snp_step_small.cu (motion_model_manager.py:354-373,424-459; forces.py:63-151).
+#include <type_traits>
+
 #include "snp_gym.cuh"
 
 namespace snp {
@@ -81,6 +83,11 @@ template <typename T> struct LargeArgs {
     int *live_cnt, *live_list;  // per i-block: how many chunks are in reach, and which, ascending ([i-blocks], [i-blocks][Jp]) -- what the
                                 // finish kernel walks instead of scanning the flags
     int robot_steps;  // robot.step calls of this call up to and including this sub-step's (0 for a fixed robot)
+    // A batch of k.E environments (the kBatch instantiations, snp_large_batch_step): env_n humans each, human i of env e at e * env_n + i
+    // in the view, the SoA and the partial sums.  Tiles, chunks and i-blocks are per env (clipped at the env's end), so a unit
+    // (i-block, chunk) only ever pairs humans of one env; the global tile of env e's tile t is e * env_tiles + t.
+    long long env_n;
+    int env_tiles, env_iblocks, env_fblocks;  // per env: 128-entity tiles (= chunks), i-blocks of the pair phase, finish CTAs
 };
 constexpr int kMaxQueues = 256;                 // one queue of list entries per SM (entry k belongs to queue k mod n_queues)
 constexpr int kWorkCounters = 4 + kMaxQueues;   // ints in front of the list
@@ -108,10 +115,18 @@ template <typename T> __device__ __forceinline__ void block_box(T xmin, T xmax, 
     __syncthreads();
 }
 
-template <typename T> __global__ void __launch_bounds__(kTile) k_tile_boxes(const T *others, long long M, T *boxes) {
+template <typename T, bool kBatch>
+__global__ void __launch_bounds__(kTile) k_tile_boxes(const T *others, long long M, T *boxes, long long env_n, int env_tiles) {
     __shared__ T sbox[20];
-    const long long j = (long long)blockIdx.x * kTile + threadIdx.x;
-    const bool ok = j < M;
+    long long j;
+    bool ok;
+    if constexpr (kBatch) {  // block = global tile e * env_tiles + t
+        const int e = blockIdx.x / env_tiles;
+        const long long r = (long long)(blockIdx.x - e * env_tiles) * kTile + threadIdx.x;
+        j = e * env_n + r; ok = r < env_n;
+    } else {
+        j = (long long)blockIdx.x * kTile + threadIdx.x; ok = j < M;
+    }
     const T big = Real<T>::inf();
     const T x = ok ? others[j] : T(0), y = ok ? others[M + j] : T(0), rs = ok ? others[4 * M + j] : T(0);
     T out[5];
@@ -121,22 +136,32 @@ template <typename T> __global__ void __launch_bounds__(kTile) k_tile_boxes(cons
 
 // The box of an i-block from the tile boxes alone: its agents are the entities of kAgentsPerThread consecutive tiles, whose union
 // box contains them.
-template <typename T> __device__ __forceinline__ void iblock_box(const LargeArgs<T> &la, int iblock, int apt, T *u /*[5]*/) {
-    const long long t0 = (la.self_offset + (long long)iblock * apt * kTile) / kTile;
+template <typename T, bool kBatch> __device__ __forceinline__ void iblock_box(const LargeArgs<T> &la, int iblock, int apt, T *u /*[5]*/) {
+    long long t0, t_end = la.n_tiles;
+    if constexpr (kBatch) {  // the i-block's tiles, clipped at its env's last
+        const int e = iblock / la.env_iblocks;
+        t0 = (long long)e * la.env_tiles + (long long)(iblock - e * la.env_iblocks) * apt;
+        t_end = (long long)(e + 1) * la.env_tiles;
+    } else {
+        t0 = (la.self_offset + (long long)iblock * apt * kTile) / kTile;
+    }
     const T inf = Real<T>::inf();
     u[0] = inf; u[1] = -inf; u[2] = inf; u[3] = -inf; u[4] = T(0);
     for (int q = 0; q < apt; ++q)
-        if (t0 + q < la.n_tiles) {
+        if (t0 + q < t_end) {
             const T *b = la.boxes + (size_t)(t0 + q) * 5;
             u[0] = min(u[0], b[0]); u[1] = max(u[1], b[1]); u[2] = min(u[2], b[2]); u[3] = max(u[3], b[3]); u[4] = max(u[4], b[4]);
         }
 }
-// Is any tile of chunk `chunk` within reach of the box u?  (Beyond reach the pair law is below the bound in the header.)
-template <typename T> __device__ __forceinline__ bool chunk_near(const LargeArgs<T> &la, const T *u, int chunk) {
-    const long long j_begin = (long long)chunk * kChunk, j_end = min(la.M, j_begin + kChunk);
+// Is any tile of chunk `chunk` (of env e in a batch) within reach of the box u?  (Beyond reach the pair law is below the bound in
+// the header.)
+template <typename T, bool kBatch> __device__ __forceinline__ bool chunk_near(const LargeArgs<T> &la, const T *u, int chunk, int e) {
+    long long base = 0, end = la.M, tile0 = 0;  // the env's first entity, its end and its first tile
+    if constexpr (kBatch) { base = e * la.env_n; end = base + la.env_n; tile0 = (long long)e * la.env_tiles; }
+    const long long j_begin = base + (long long)chunk * kChunk, j_end = min(end, j_begin + kChunk);
     bool near = false;
     for (long long j0 = j_begin; j0 < j_end; j0 += kTile) {
-        const T *b = la.boxes + (size_t)(j0 / kTile) * 5;
+        const T *b = la.boxes + (size_t)(tile0 + (j0 - base) / kTile) * 5;
         const T gx = max(T(0), max(u[0] - b[1], b[0] - u[1]));
         const T gy = max(T(0), max(u[2] - b[3], b[2] - u[3]));
         const T reach = u[4] + b[4] + la.cull_margin;
@@ -154,7 +179,9 @@ template <typename T> struct PairsSmem {
 };
 
 // One (i-block, chunk) unit of the pair phase: the i-block's agents against the chunk's entities, one partial sum per agent.
-template <typename T, int SOC, int kAgentsPerThread>
+// In a batch the i-block and the chunk are those of one env: agents and entities are numbered from the env's first (base), so that
+// Moussaid's jj < idx compares indices in the same numbering.
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
 __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T> &sm, int iblock, int chunk, bool &have_tbl) {
     Ent<T> *tile = reinterpret_cast<Ent<T> *>(sm.tile_raw);
     T *tile_rs = sm.tile_rs;
@@ -163,8 +190,15 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
     const KArgs<T> &a = la.k;
     const long long N = a.EN, M = la.M;
     const Params<T> &P = a.P;
-    const long long j_begin = (long long)chunk * kChunk;
-    const long long j_end = min(M, j_begin + kChunk);
+    long long base = 0, n_env = N, end = M, tile0 = 0;  // the env's first entity, its humans, its end and its first tile
+    int ib = iblock;                                     // the i-block within its env
+    if constexpr (kBatch) {
+        const int e = iblock / la.env_iblocks;
+        ib = iblock - e * la.env_iblocks;
+        base = e * la.env_n; n_env = la.env_n; end = base + la.env_n; tile0 = (long long)e * la.env_tiles;
+    }
+    const long long j_begin = base + (long long)chunk * kChunk;
+    const long long j_end = min(end, j_begin + kChunk);
     unsigned char *live_flag = la.live + (size_t)iblock * la.Jp + chunk;
     T mx[kAgentsPerThread], my[kAgentsPerThread], mvx[kAgentsPerThread], mvy[kAgentsPerThread], mrs[kAgentsPerThread];
     long long idx[kAgentsPerThread];
@@ -173,9 +207,9 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
     T bx0 = big, bx1 = -big, by0 = big, by1 = -big, brs = T(0);
 #pragma unroll
     for (int q = 0; q < kAgentsPerThread; ++q) {
-        idx[q] = ((long long)iblock * kAgentsPerThread + q) * kTile + threadIdx.x;
-        const bool live = idx[q] < N;
-        const long long o = la.self_offset + (live ? idx[q] : 0);
+        idx[q] = ((long long)ib * kAgentsPerThread + q) * kTile + threadIdx.x;
+        const bool live = idx[q] < n_env;
+        const long long o = la.self_offset + base + (live ? idx[q] : 0);
         mx[q] = la.others[o]; my[q] = la.others[M + o]; mvx[q] = la.others[2 * M + o]; mvy[q] = la.others[3 * M + o]; mrs[q] = la.others[4 * M + o];
         fsx[q] = T(0); fsy[q] = T(0);
         if (live) { bx0 = min(bx0, mx[q]); bx1 = max(bx1, mx[q]); by0 = min(by0, my[q]); by1 = max(by1, my[q]); brs = max(brs, mrs[q]); }
@@ -187,7 +221,7 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
     bool any_tile = false;
     for (long long j0 = j_begin; j0 < j_end; j0 += kTile) {
         if (la.cull_margin >= T(0)) {  // uniform across the CTA
-            const T *b = la.boxes + (size_t)(j0 / kTile) * 5;
+            const T *b = la.boxes + (size_t)(tile0 + (j0 - base) / kTile) * 5;
             const T gx = max(T(0), max(ibox[0] - b[1], b[0] - ibox[1]));
             const T gy = max(T(0), max(ibox[2] - b[3], b[2] - ibox[3]));
             const T reach = ibox[4] + b[4] + la.cull_margin;
@@ -232,7 +266,7 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
         for (int t = t_first; t < cnt; ++t) {
             const Ent<T> o = tile[t];
             const T rsj = tile_rs[t];
-            const long long jj = j0 + t - la.self_offset;  // index of the entity in this crowd's numbering
+            const long long jj = j0 + t - la.self_offset - base;  // index of the entity in this crowd's (env's) numbering
             // the self pair (jj == idx[q]) contributes exactly zero by construction (tiny_ in pair_eval)
             if constexpr (sizeof(T) == 4) {
                 // the evaluations of the thread's agents are independent and branch-free; ONE vote covers the rare contact
@@ -290,20 +324,20 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
     if (!any_tile && !la.use_list) return;
 #pragma unroll
     for (int q = 0; q < kAgentsPerThread; ++q)
-        if (idx[q] < N) {
-            la.partial[((size_t)chunk * 2 + 0) * N + idx[q]] = fsx[q];
-            la.partial[((size_t)chunk * 2 + 1) * N + idx[q]] = fsy[q];
+        if (idx[q] < n_env) {
+            la.partial[((size_t)chunk * 2 + 0) * N + base + idx[q]] = fsx[q];
+            la.partial[((size_t)chunk * 2 + 1) * N + base + idx[q]] = fsy[q];
         }
 }
 
 // Regular grid (i-block, chunk): every ordered pair, or -- with culling, for a slice the work list does not take -- every tile
 // tested against the box of the i-block's agents.  A CTA that culled every tile leaves its partial sums unwritten and says so in
 // `live`.
-template <typename T, int SOC, int kAgentsPerThread>
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
 __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
     __shared__ PairsSmem<T> sm;
     bool have_tbl = false;  // the 16 kB exp table is staged only by CTAs that evaluate at least one tile (most are culled)
-    pairs_chunk<T, SOC, kAgentsPerThread>(la, sm, blockIdx.x, blockIdx.y, have_tbl);
+    pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm, blockIdx.x, blockIdx.y, have_tbl);
 }
 
 // Culled steps of a wide crowd: of the i-blocks x J grid only a few percent of the CTAs have anything to evaluate (65536 humans on
@@ -315,16 +349,17 @@ __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
 // queue of the SM it runs on (%smid) and only when that is empty looks for another queue with entries left: every SM gets the
 // same number of entries whatever the placement of the CTAs, and every entry is taken whichever CTAs exist.  Partial sums land
 // where the grid version puts them: results are bit-identical.
-template <typename T> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
+template <typename T, bool kBatch> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
     __shared__ int warp_cnt[8];
     T u[5];
-    iblock_box<T>(la, blockIdx.x, la.apt, u);
+    iblock_box<T, kBatch>(la, blockIdx.x, la.apt, u);
+    const int env = kBatch ? (int)blockIdx.x / la.env_iblocks : 0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int *mine = la.live_list + (size_t)blockIdx.x * la.Jp;
     int listed = 0;  // chunks of this i-block listed so far (uniform)
     for (int c0 = 0; c0 < la.J; c0 += blockDim.x) {
         const int c = c0 + threadIdx.x;
-        const bool near = c < la.J && chunk_near<T>(la, u, c);
+        const bool near = c < la.J && chunk_near<T, kBatch>(la, u, c, env);
         if (c < la.J) la.live[(size_t)blockIdx.x * la.Jp + c] = near ? 1 : 0;
         const unsigned m = __ballot_sync(0xffffffffu, near);
         const int below = __popc(m & ((1u << lane) - 1u));
@@ -347,7 +382,7 @@ template <typename T> __global__ void __launch_bounds__(256) k_large_cull(const 
     if (threadIdx.x == 0) la.live_cnt[blockIdx.x] = listed;
 }
 
-template <typename T, int SOC, int kAgentsPerThread>
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
 __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> la, const int n_queues) {
     __shared__ PairsSmem<T> sm;
     bool have_tbl = false;
@@ -367,7 +402,7 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
         const int item = sm.item;
         if (item >= 0) {
             const int w = la.work[item];
-            pairs_chunk<T, SOC, kAgentsPerThread>(la, sm, w / la.J, w % la.J, have_tbl);
+            pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm, w / la.J, w % la.J, have_tbl);
             continue;
         }
         // this queue is empty (and stays so: the counters only grow): move to the nearest queue that still has entries, if any
@@ -382,14 +417,15 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
 }
 
 // The robot after `steps` robot.step calls from the state in a.robot (robot_agent.py:116-136), with k_step's expressions: rb[] gets
-// SNP_ROBOT_PX, PY, VX, VY and TH.
-template <typename T> __device__ __forceinline__ void large_robot_replay(const KArgs<T> &a, int steps, T *rb) {
-    rb[SNP_ROBOT_PX] = a.robot[SNP_ROBOT_PX]; rb[SNP_ROBOT_PY] = a.robot[SNP_ROBOT_PY];
-    rb[SNP_ROBOT_VX] = a.robot[SNP_ROBOT_VX]; rb[SNP_ROBOT_VY] = a.robot[SNP_ROBOT_VY]; rb[SNP_ROBOT_TH] = a.robot[SNP_ROBOT_TH];
+// SNP_ROBOT_PX, PY, VX, VY and TH.  In a batch env e's robot is a.robot[field * E + e] and its action a.action[e], a.action[E + e].
+template <typename T, bool kBatch> __device__ __forceinline__ void large_robot_replay(const KArgs<T> &a, int steps, T *rb, int e) {
+    const long long RE = kBatch ? a.E : 1;
+    rb[SNP_ROBOT_PX] = a.robot[SNP_ROBOT_PX * RE + e]; rb[SNP_ROBOT_PY] = a.robot[SNP_ROBOT_PY * RE + e];
+    rb[SNP_ROBOT_VX] = a.robot[SNP_ROBOT_VX * RE + e]; rb[SNP_ROBOT_VY] = a.robot[SNP_ROBOT_VY * RE + e]; rb[SNP_ROBOT_TH] = a.robot[SNP_ROBOT_TH * RE + e];
     if (steps <= 0) return;
     const T dt = a.dt;
     if (a.robot_mode == 1) {  // holonomic: p = p + a*dt ; v = a
-        const T ax = a.action[0], ay = a.action[1];
+        const T ax = a.action[e], ay = a.action[RE + e];
         T px = rb[SNP_ROBOT_PX], py = rb[SNP_ROBOT_PY];
         for (int s = 0; s < steps; ++s) {
             if (sizeof(T) == 8) { px = (T)__dadd_rn((double)px, __dmul_rn((double)ax, (double)dt)); py = (T)__dadd_rn((double)py, __dmul_rn((double)ay, (double)dt)); }
@@ -397,13 +433,14 @@ template <typename T> __device__ __forceinline__ void large_robot_replay(const K
         }
         rb[SNP_ROBOT_PX] = px; rb[SNP_ROBOT_PY] = py; rb[SNP_ROBOT_VX] = ax; rb[SNP_ROBOT_VY] = ay;
     } else if (a.robot_mode == 3) {  // unicycle (v, r)
-        for (int s = 0; s < steps; ++s) robot_unicycle_step<T>(rb, (double)a.action[0], (double)a.action[1], (double)dt);
+        for (int s = 0; s < steps; ++s) robot_unicycle_step<T>(rb, (double)a.action[e], (double)a.action[RE + e], (double)dt);
     }
 }
 
 // RSOC: the pair law of the visible robot's force (SOC of the humans' model), or -1 for no robot -- a separate instantiation, so
-// that the common ones keep their registers.
-template <typename T, int OBS, int HEADED, int RSOC>
+// that the common ones keep their registers.  kBatch: CTA b of env e is block e * env_fblocks + b and covers humans 128 b ... of env
+// e only, so that it stages its own env's walls.
+template <typename T, int OBS, int HEADED, int RSOC, bool kBatch>
 __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     using R = Real<T>;
     const KArgs<T> &a = la.k;
@@ -414,8 +451,14 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     Seg<T> *segs = reinterpret_cast<Seg<T> *>(smem_raw + kTbl);
     int *seg_cnt = reinterpret_cast<int *>(smem_raw + kTbl + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)));
     if (sizeof(T) == 8 && (nseg > 0 || RSOC >= 0)) exp_table_init(exp_tbl_s);  // only the wall force and the robot evaluate exp here
+    int env = 0;
+    const T *walls = a.walls;
+    if constexpr (kBatch) {
+        env = blockIdx.x / la.env_fblocks;
+        if (a.walls_per_env) walls += (size_t)env * nseg * 4;
+    }
     for (int k = threadIdx.x; k < nseg; k += blockDim.x) {
-        const T *w = a.walls + (size_t)k * 4;
+        const T *w = walls + (size_t)k * 4;
         segs[k] = make_seg<T>(w[0], w[1], w[2], w[3]);
     }
     __syncthreads();
@@ -426,11 +469,18 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     }
     __syncthreads();
     const long long N = a.EN, M = la.M;
-    const long long i = (long long)blockIdx.x * kTile + threadIdx.x;
+    long long i, r = 0;  // the agent; in a batch also its index in its env
+    bool gone;
+    if constexpr (kBatch) {
+        r = (long long)(blockIdx.x - env * la.env_fblocks) * kTile + threadIdx.x;
+        i = env * la.env_n + r; gone = r >= la.env_n;
+    } else {
+        i = (long long)blockIdx.x * kTile + threadIdx.x; gone = i >= N;
+    }
     if (la.use_list && blockIdx.x == 0)  // the pair phase is over: empty list and queues for the next sub-step
         for (int k = threadIdx.x; k < kWorkCounters; k += kTile) la.work_counters[k] = 0;
     const bool fold_boxes = la.peer_boxes[0] != nullptr;  // uniform; only offered when N is a whole number of tiles, so that every
-    if (i >= N) return;                                    // thread of every block reaches the box reduction at the end
+    if (gone) return;                                      // thread of every block reaches the box reduction at the end
     const unsigned vote_mask = __activemask();  // the lanes that own an agent (the tail warp is partial)
     const Params<T> &P = a.P;
     Agent<T> m;
@@ -455,13 +505,14 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     // sharding).  The flags are the same for the whole CTA and live chunks come in runs; they are read 64 at a time, and for every
     // 16 flags with a live one the loads of all live partial sums are issued together before the (ordered) additions -- a
     // flag-by-flag loop serialised one L2 round trip per live chunk.
-    const uint4 *lv = reinterpret_cast<const uint4 *>(la.live + (size_t)(i / (kTile * la.apt)) * la.Jp);
+    const long long row = kBatch ? (long long)env * la.env_iblocks + r / (kTile * la.apt) : i / (kTile * la.apt);  // the agent's i-block
+    const uint4 *lv = reinterpret_cast<const uint4 *>(la.live + (size_t)row * la.Jp);
     const int n_words = la.use_list ? 0 : la.Jp >> 4;
     if (la.use_list) {
         // the cull kernel left the i-block's live chunks as an ascending list: sixteen indices per step, the next sixteen already on
         // their way while the partial sums of the current ones are loaded
-        const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)(i / (kTile * la.apt)) * la.Jp);
-        const int cnt = la.live_cnt[i / (kTile * la.apt)];
+        const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)row * la.Jp);
+        const int cnt = la.live_cnt[row];
         int4 nxt[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) nxt[u] = ll[u];  // (a row is Jp >= 16 entries long; entries beyond cnt are ignored)
@@ -508,8 +559,9 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     if constexpr (RSOC >= 0) {
         // the robot: the last entity of the ordered loop, after every chunk; never culled (one pair per human)
         T rb[SNP_ROBOT_FIELDS];
-        large_robot_replay<T>(a, la.robot_steps, rb);
-        const T rrs = a.robot[SNP_ROBOT_R] + a.robot[SNP_ROBOT_SAFETY];
+        large_robot_replay<T, kBatch>(a, la.robot_steps, rb, env);
+        const long long RE = kBatch ? a.E : 1;
+        const T rrs = a.robot[SNP_ROBOT_R * RE + env] + a.robot[SNP_ROBOT_SAFETY * RE + env];
         T fx, fy;
         pair_force<T, RSOC>(P, exp_tbl_s, vote_mask, m.px, m.py, m.vx, m.vy, m.rs, rb[SNP_ROBOT_PX], rb[SNP_ROBOT_PY], rb[SNP_ROBOT_VX],
                             rb[SNP_ROBOT_VY], rrs, fx, fy);
@@ -601,30 +653,30 @@ template <typename T> __global__ void k_large_publish(const T *dyn, const T *sta
     view[4 * stride + o] = stat[SNP_STAT_R * N + i] + stat[SNP_STAT_SAFETY * N + i];
 }
 
-template <typename T, int SOC, int OBS, int HEADED> int launch_large(const LargeArgs<T> &la, cudaStream_t st) {
+template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_large(const LargeArgs<T> &la, cudaStream_t st) {
     const long long N = la.k.EN;
     const int nseg = la.k.W * la.k.S;
     if (sizeof(T) == 8) SNP_CUDA_OK(ensure_exp_table());
-    if (!la.boxes_ready) k_tile_boxes<T><<<(unsigned)la.n_tiles, kTile, 0, st>>>(la.others, la.M, la.boxes);
+    if (!la.boxes_ready) k_tile_boxes<T, kBatch><<<(unsigned)la.n_tiles, kTile, 0, st>>>(la.others, la.M, la.boxes, la.env_n, la.env_tiles);
     const long long per_block = (long long)kTile * la.apt;
-    dim3 grid((unsigned)((N + per_block - 1) / per_block), (unsigned)la.J);
+    dim3 grid((unsigned)(kBatch ? (long long)la.k.E * la.env_iblocks : (N + per_block - 1) / per_block), (unsigned)la.J);
     if constexpr (SOC == 2) {  // Moussaid's pair law has no culling distance (run_large): every pair, two agents per thread
-        k_large_pairs<T, SOC, kMaxAgentsPerThread><<<grid, kTile, 0, st>>>(la);
+        k_large_pairs<T, SOC, kMaxAgentsPerThread, kBatch><<<grid, kTile, 0, st>>>(la);
     } else if (la.use_list) {  // (culled: one agent per thread)
         // the counters start empty: zeroed here on a sub-step that computes the tile boxes, else by the previous sub-step's finish kernel
         if (!la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
-        k_large_cull<T><<<grid.x, 256, 0, st>>>(la);
+        k_large_cull<T, kBatch><<<grid.x, 256, 0, st>>>(la);
         static int slots = 0;  // resident CTAs per SM
         const int n_queues = device_sm_count() < kMaxQueues ? device_sm_count() : kMaxQueues;
-        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1>, kTile, 0));
-        k_large_pairs_list<T, SOC, 1><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
+        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1, kBatch>, kTile, 0));
+        k_large_pairs_list<T, SOC, 1, kBatch><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
         count_launch();
-    } else if (la.apt == 1) k_large_pairs<T, SOC, 1><<<grid, kTile, 0, st>>>(la);
-    else k_large_pairs<T, SOC, 2><<<grid, kTile, 0, st>>>(la);
+    } else if (la.apt == 1) k_large_pairs<T, SOC, 1, kBatch><<<grid, kTile, 0, st>>>(la);
+    else k_large_pairs<T, SOC, 2, kBatch><<<grid, kTile, 0, st>>>(la);
     const size_t smem = sizeof(double) * kExpN + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + sizeof(int) * (la.k.W + 1) + 16;
-    auto fin = la.k.consider_robot ? k_large_finish<T, OBS, HEADED, SOC> : k_large_finish<T, OBS, HEADED, -1>;
+    auto fin = la.k.consider_robot ? k_large_finish<T, OBS, HEADED, SOC, kBatch> : k_large_finish<T, OBS, HEADED, -1, kBatch>;
     if (smem > 48 * 1024) SNP_CUDA_OK(cudaFuncSetAttribute(fin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fin<<<(unsigned)((N + kTile - 1) / kTile), kTile, smem, st>>>(la);
+    fin<<<(unsigned)(kBatch ? (long long)la.k.E * la.env_fblocks : (N + kTile - 1) / kTile), kTile, smem, st>>>(la);
     count_launch(la.boxes_ready ? 2 : 3);
     SNP_CUDA_OK(cudaGetLastError());
     return SNP_OK;
@@ -634,12 +686,13 @@ inline long long large_J(long long M) { return (M + kChunk - 1) / kChunk; }
 inline long long large_tiles(long long M) { return (M + kTile - 1) / kTile; }
 inline long long large_iblocks(long long N) { return (N + kTile - 1) / kTile; }  // sized for one agent per thread (the finer split)
 
-// The scratch of n_local agents against M entities: byte offsets of its regions (the partial sums at 0) and its size.  Every region
-// starts 16-byte aligned (the finish kernel reads the live map and the lists 16 bytes at a time).
+inline long long up16(long long b) { return (b + 15) & ~15LL; }
+
+// The scratch of n_local agents in `blocks` i-blocks against J chunks: byte offsets of its regions (the partial sums at 0) and its
+// size.  Every region starts 16-byte aligned (the finish kernel reads the live map and the lists 16 bytes at a time).
 struct LargeScratch { long long live, counters, work, live_cnt, live_list, bytes; };
-inline LargeScratch large_scratch(long long n_local, long long M, long long elem_bytes) {
-    const long long J = large_J(M), Jp = (J + 15) & ~15LL, blocks = large_iblocks(n_local);
-    auto up16 = [](long long b) { return (b + 15) & ~15LL; };
+inline LargeScratch large_scratch_units(long long n_local, long long J, long long blocks, long long elem_bytes) {
+    const long long Jp = (J + 15) & ~15LL;
     LargeScratch s;
     s.live = up16(elem_bytes * J * 2 * n_local);      // [J][2][n_local] partial sums
     s.counters = up16(s.live + blocks * Jp);           // [blocks][Jp] live map
@@ -649,12 +702,47 @@ inline LargeScratch large_scratch(long long n_local, long long M, long long elem
     s.bytes = s.live_list + 4 * blocks * Jp;           // [blocks][Jp] their indices, ascending
     return s;
 }
+// One crowd: n_local agents against M entities.
+inline LargeScratch large_scratch(long long n_local, long long M, long long elem_bytes) {
+    return large_scratch_units(n_local, large_J(M), large_iblocks(n_local), elem_bytes);
+}
+// A batch of E envs of N humans: the regions above (chunks and i-blocks per env), then the two view buffers, each [5][E N] entities
+// and the [E ceil(N/128)][5] tile boxes.
+struct LargeBatchScratch { LargeScratch s; long long view_a, view_b, bytes; };
+inline LargeBatchScratch large_batch_scratch(long long E, long long N, long long elem_bytes) {
+    LargeBatchScratch b;
+    b.s = large_scratch_units(E * N, large_J(N), E * large_iblocks(N), elem_bytes);
+    const long long view = up16(elem_bytes * 5 * (E * N + E * large_tiles(N)));
+    b.view_a = up16(b.s.bytes);
+    b.view_b = b.view_a + view;
+    b.bytes = b.view_b + view;
+    return b;
+}
+
+template <typename T, bool kBatch> int dispatch_large(int type, const LargeArgs<T> &la, cudaStream_t st) {
+    switch (type) {
+        case 0: return launch_large<T, 0, 0, 0, kBatch>(la, st);
+        case 1: return launch_large<T, 1, 1, 0, kBatch>(la, st);
+        case 2: return launch_large<T, 2, 0, 0, kBatch>(la, st);
+        case 3: return launch_large<T, 0, 0, 1, kBatch>(la, st);
+        case 4: return launch_large<T, 1, 1, 1, kBatch>(la, st);
+        case 5: return launch_large<T, 2, 0, 1, kBatch>(la, st);
+        case 6: return launch_large<T, 0, 0, 2, kBatch>(la, st);
+        case 7: return launch_large<T, 1, 1, 2, kBatch>(la, st);
+        case 8: return launch_large<T, 2, 0, 2, kBatch>(la, st);
+    }
+    set_error("Type %d does not exist for this implementation", type);
+    return SNP_ERR_INVALID;
+}
 
 // One sub-step: `cur` = the view buffer read ([5][M] entities + their [n_tiles][5] tile boxes), `next` = the n_peers buffers the
 // finish kernel stores the updated entries into, and their tile boxes too when `fold_boxes`.  `boxes_ready`: `cur`'s tile boxes
 // were written by the previous sub-step's producers.  `sub`: index of the sub-step in the call (how far a moving robot has gone).
+// env_n > 0: the crowd is a batch of c->E envs of env_n = c->N humans (M = E N, self_offset 0, one next buffer).
 template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, const void *cur, const void *const *next, int n_peers,
-                                    long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, int sub, cudaStream_t st) {
+                                    long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, int sub, cudaStream_t st,
+                                    long long env_n = 0) {
+    const bool batch = env_n > 0;
     LargeArgs<T> la;
     la.n_peers = n_peers;
     for (int p = 0; p < 8; ++p) la.peers[p] = (p < n_peers) ? (T *)next[p] : nullptr;
@@ -665,15 +753,18 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     a.dyn = (T *)c->dyn; a.stat = (const T *)c->stat; a.goals = (const T *)c->goals; a.goal_idx = c->goal_idx; a.goal_cnt = c->goal_cnt;
     a.agent_params = nullptr; a.P = make_params<T>(c->params); a.robot = (T *)c->robot;
     a.walls = (const T *)c->walls; a.W = c->W; a.S = c->W > 0 ? c->S : 0; a.walls_per_env = 0;
+    if (batch) { a.E = c->E; a.N = c->N; a.walls_per_env = c->walls_per_env; }
     a.consider_robot = o->consider_robot; a.symmetric = o->symmetric; a.numba = o->numba_compat; a.n_substeps = 1; a.robot_mode = o->robot_mode;
     a.dt = (T)o->dt; a.dt_d = o->dt; a.action = (const T *)o->action; a.pre_checks = a.post_checks = a.track_touch = 0;
     a.time_now = nullptr; a.flags = nullptr; a.checks = nullptr; a.epw = 1; a.gpb = 1; a.mapping = 0; a.full_pair_loop = 1; a.respawn = 0; a.robot_type = 0; a.RP = a.P; a.robot_every = 0; a.robot_phase = 0; a.robot_dt = T(0);
     la.robot_steps = (o->robot_mode == 1 || o->robot_mode == 3) ? sub + 1 : 0;
     la.others = (const T *)cur; la.M = M; la.self_offset = self_offset;
     la.boxes = (T *)cur + 5 * M;
-    la.J = (int)large_J(M); la.n_tiles = (int)large_tiles(M);
+    la.env_n = env_n; la.env_tiles = (int)large_tiles(env_n);
+    la.J = (int)large_J(batch ? env_n : M); la.n_tiles = (int)(batch ? c->E * large_tiles(env_n) : large_tiles(M));
     la.Jp = (la.J + 15) & ~15;
-    const LargeScratch sc = large_scratch(a.EN, M, sizeof(T));
+    const long long blocks = batch ? c->E * large_iblocks(env_n) : large_iblocks(a.EN);  // rows of the live map
+    const LargeScratch sc = large_scratch_units(a.EN, la.J, blocks, sizeof(T));
     char *base = (char *)scratch;
     la.partial = (T *)base;
     la.live = (unsigned char *)(base + sc.live);
@@ -693,36 +784,45 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     // culled steps: one agent per thread (twice the units to hand out).  Round 2 kept two for fp32 on the static grid, where the
     // finer split only added CTAs to launch; on the work list one rank's slice of an 8-way split runs 0.0552 -> 0.0408 ms in fp32
     la.apt = margin >= 0.0 ? 1 : kMaxAgentsPerThread;  // fp32 pair evaluations are short: the finer split only adds launch overhead there
-    la.use_list = (margin >= 0.0 && self_offset % kTile == 0 && large_iblocks(a.EN) * la.J < (1LL << 31)) ? 1 : 0;
-    switch (o->type) {
-        case 0: return launch_large<T, 0, 0, 0>(la, st);
-        case 1: return launch_large<T, 1, 1, 0>(la, st);
-        case 2: return launch_large<T, 2, 0, 0>(la, st);
-        case 3: return launch_large<T, 0, 0, 1>(la, st);
-        case 4: return launch_large<T, 1, 1, 1>(la, st);
-        case 5: return launch_large<T, 2, 0, 1>(la, st);
-        case 6: return launch_large<T, 0, 0, 2>(la, st);
-        case 7: return launch_large<T, 1, 1, 2>(la, st);
-        case 8: return launch_large<T, 2, 0, 2>(la, st);
-    }
-    set_error("Type %d does not exist for this implementation", o->type);
-    return SNP_ERR_INVALID;
+    la.use_list = (margin >= 0.0 && self_offset % kTile == 0 && blocks * la.J < (1LL << 31)) ? 1 : 0;
+    const long long per_block = (long long)kTile * la.apt;
+    la.env_iblocks = (int)((env_n + per_block - 1) / per_block);
+    la.env_fblocks = (int)large_iblocks(env_n);
+    return batch ? dispatch_large<T, true>(o->type, la, st) : dispatch_large<T, false>(o->type, la, st);
 }
 
 // After the last sub-step of a call: the robot's end state (robot_mode 1 / 3; the finish kernels of the call read the start state
-// until they are done) and the clock, advanced by dt per sub-step as k_step does.  One thread.
-template <typename T> __global__ void k_large_robot_end(const KArgs<T> a, int n_substeps) {
+// until they are done) and the clock, advanced by dt per sub-step as k_step does.  One thread (per env in a batch).
+template <typename T, bool kBatch> __global__ void k_large_robot_end(const KArgs<T> a, int n_substeps) {
+    int e = 0;
+    long long RE = 1;
+    if constexpr (kBatch) {
+        e = blockIdx.x * blockDim.x + threadIdx.x; RE = a.E;
+        if (e >= a.E) return;
+    }
     if (a.robot && (a.robot_mode == 1 || a.robot_mode == 3)) {
         T rb[SNP_ROBOT_FIELDS];
-        large_robot_replay<T>(a, n_substeps, rb);
-        a.robot[SNP_ROBOT_PX] = rb[SNP_ROBOT_PX]; a.robot[SNP_ROBOT_PY] = rb[SNP_ROBOT_PY];
-        a.robot[SNP_ROBOT_VX] = rb[SNP_ROBOT_VX]; a.robot[SNP_ROBOT_VY] = rb[SNP_ROBOT_VY]; a.robot[SNP_ROBOT_TH] = rb[SNP_ROBOT_TH];
+        large_robot_replay<T, kBatch>(a, n_substeps, rb, e);
+        a.robot[SNP_ROBOT_PX * RE + e] = rb[SNP_ROBOT_PX]; a.robot[SNP_ROBOT_PY * RE + e] = rb[SNP_ROBOT_PY];
+        a.robot[SNP_ROBOT_VX * RE + e] = rb[SNP_ROBOT_VX]; a.robot[SNP_ROBOT_VY * RE + e] = rb[SNP_ROBOT_VY];
+        a.robot[SNP_ROBOT_TH * RE + e] = rb[SNP_ROBOT_TH];
     }
     if (a.time_now) {
-        double t = a.time_now[0];
+        double t = a.time_now[e];
         for (int s = 0; s < n_substeps; ++s) t = __dadd_rn(t, a.dt_d);
-        a.time_now[0] = t;
+        a.time_now[e] = t;
     }
+}
+
+template <typename T, bool kBatch> int launch_large_robot_end(const snp_crowd *c, const snp_step_opts *o, int n_substeps, cudaStream_t st) {
+    KArgs<T> a{};
+    a.E = c->E; a.robot = (T *)c->robot; a.action = (const T *)o->action; a.robot_mode = o->robot_mode;
+    a.dt = (T)o->dt; a.dt_d = o->dt; a.time_now = o->time_now;
+    if (kBatch) k_large_robot_end<T, true><<<(unsigned)((c->E + 127) / 128), 128, 0, st>>>(a, n_substeps);
+    else k_large_robot_end<T, false><<<1, 1, 0, st>>>(a, n_substeps);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    return SNP_OK;
 }
 
 // ---- snp_large_checks: the robot against M humans of a view (social_nav_sim.py:949-1029, social_nav_gym.py:107-118) ----
@@ -741,6 +841,13 @@ template <typename T> struct CheckArgs {
     int *flags;
     double *checks;
 };
+// A batch (kBatch): E envs of M humans, view [5][stride = E M], radius [E M]; clear: start from zero flags and checks.  A type of its
+// own, so that the one-crowd kernel's parameters (and registers) stay as they are.
+template <typename T> struct CheckBatchArgs : CheckArgs<T> {
+    int E, clear;
+    long long stride;
+};
+template <typename T, bool kBatch> using CheckArgsOf = std::conditional_t<kBatch, CheckBatchArgs<T>, CheckArgs<T>>;
 
 // (dmin, hit) of a run on the left combined with the run on its right
 __device__ __forceinline__ void swept_combine(double &dmin, int &hit, double dmin_r, int hit_r) {
@@ -749,36 +856,41 @@ __device__ __forceinline__ void swept_combine(double &dmin, int &hit, double dmi
     hit = hit_r;
 }
 
-template <typename T> __global__ void __launch_bounds__(kCheckThreads) k_large_checks(const CheckArgs<T> c) {
+// kBatch: one CTA per env (blockIdx.x = env).
+template <typename T, bool kBatch> __global__ void __launch_bounds__(kCheckThreads) k_large_checks(const CheckArgsOf<T, kBatch> c) {
     __shared__ double s_dmin[kCheckThreads / 32], s_admin[kCheckThreads / 32];
     __shared__ int s_hit[kCheckThreads / 32];
-    const T *rbt = c.robot;
-    const T rpx = rbt[SNP_ROBOT_PX], rpy = rbt[SNP_ROBOT_PY], rr = rbt[SNP_ROBOT_R], rgx = rbt[SNP_ROBOT_GX], rgy = rbt[SNP_ROBOT_GY];
+    int env = 0;
+    long long RE = 1, stride = c.M;
+    if constexpr (kBatch) { env = blockIdx.x; RE = c.E; stride = c.stride; }
+    const T *rbt = c.robot + env;
+    const T rpx = rbt[SNP_ROBOT_PX * RE], rpy = rbt[SNP_ROBOT_PY * RE], rr = rbt[SNP_ROBOT_R * RE], rgx = rbt[SNP_ROBOT_GX * RE], rgy = rbt[SNP_ROBOT_GY * RE];
     T ax = T(0), ay = T(0);
     if (c.pre) {
-        ax = c.action[0]; ay = c.action[1];
+        ax = c.action[env]; ay = c.action[RE + env];
         if (c.mode == 3) {  // unicycle action (v, r): the swept test and the goal test use v (cos, sin)(yaw + r) (sim:973)
             const double uv = (double)ax, ur = (double)ay;
             double sn_, cs_;
-            sincos((double)rbt[SNP_ROBOT_TH] + ur, &sn_, &cs_);
+            sincos((double)rbt[SNP_ROBOT_TH * RE] + ur, &sn_, &cs_);
             ax = (T)__dmul_rn(uv, cs_); ay = (T)__dmul_rn(uv, sn_);
         }
     }
     const long long M = c.M, per = (M + kCheckThreads - 1) / kCheckThreads;
     const long long b = (long long)threadIdx.x * per, e = min(M, b + per);
-    const T *px = c.view, *py = c.view + M, *vx = c.view + 2 * M, *vy = c.view + 3 * M;
+    const T *view = c.view + env * M, *radius = c.radius + env * M;
+    const T *px = view, *py = view + stride, *vx = view + 2 * stride, *vy = view + 3 * stride;
     double dmin = CUDART_INF, admin = 10000.0;
     int hit = 0;
     if (c.pre)
         for (long long k = b; k < e; ++k) {
-            const double cd = swept_distance((double)px[k], (double)py[k], (double)vx[k], (double)vy[k], (double)c.radius[k], (double)rpx, (double)rpy,
+            const double cd = swept_distance((double)px[k], (double)py[k], (double)vx[k], (double)vy[k], (double)radius[k], (double)rpx, (double)rpy,
                                              (double)rr, (double)ax, (double)ay, c.consts[5]);
             if (cd < 0) { hit = 1; break; }
             else if (cd < dmin) dmin = cd;
         }
     if (c.post)
         for (long long k = b; k < e; ++k) {
-            double d = __dsub_rn(__dsub_rn(xnorm_np(__dsub_rn((double)px[k], (double)rpx), __dsub_rn((double)py[k], (double)rpy)), (double)c.radius[k]), (double)rr);
+            double d = __dsub_rn(__dsub_rn(xnorm_np(__dsub_rn((double)px[k], (double)rpx), __dsub_rn((double)py[k], (double)rpy)), (double)radius[k]), (double)rr);
             if (!(d < 10000.0)) d = 10000.0;
             admin = d < admin ? d : admin;
         }
@@ -793,38 +905,79 @@ template <typename T> __global__ void __launch_bounds__(kCheckThreads) k_large_c
     if (threadIdx.x != 0) return;
     dmin = CUDART_INF; admin = 10000.0; hit = 0;
     for (int w = 0; w < kCheckThreads / 32; ++w) { swept_combine(dmin, hit, s_dmin[w], s_hit[w]); admin = s_admin[w] < admin ? s_admin[w] : admin; }
-    int f = *c.flags;
+    int *flags = c.flags + env;
+    double *checks = c.checks ? c.checks + 4 * env : nullptr;
+    int f = *flags;
+    if constexpr (kBatch) {
+        if (c.clear) {
+            f = 0;
+            if (checks) checks[0] = checks[1] = checks[2] = checks[3] = 0.0;
+        }
+    }
     if (c.pre) {
         const double endx = __dadd_rn((double)rpx, __dmul_rn((double)ax, c.consts[5]));
         const double endy = __dadd_rn((double)rpy, __dmul_rn((double)ay, c.consts[5]));
         const bool goal = xnorm_np(__dsub_rn(endx, (double)rgx), __dsub_rn(endy, (double)rgy)) < (double)rr;
-        const double tnow = c.time_now ? c.time_now[0] : 0.0;
+        const double tnow = c.time_now ? c.time_now[env] : 0.0;
         double reward;
         bool term, trunc;
         const int code = reward_and_info(hit != 0, dmin, goal, tnow, c.consts, reward, term, trunc);
         f &= ~(SNP_FLAG_COLLISION | SNP_FLAG_REACHING_GOAL | SNP_FLAG_TERMINATED | SNP_FLAG_TRUNCATED | (7 << SNP_FLAG_INFO_SHIFT));
         f |= (hit ? SNP_FLAG_COLLISION : 0) | (goal ? SNP_FLAG_REACHING_GOAL : 0) | (term ? SNP_FLAG_TERMINATED : 0) | (trunc ? SNP_FLAG_TRUNCATED : 0) |
              (code << SNP_FLAG_INFO_SHIFT);
-        if (c.checks) { c.checks[0] = dmin; c.checks[1] = reward; }
+        if (checks) { checks[0] = dmin; checks[1] = reward; }
     }
     if (c.post) {
         const bool agoal = xnorm_np(__dsub_rn((double)rpx, (double)rgx), __dsub_rn((double)rpy, (double)rgy)) < (double)rr;
         f &= ~(SNP_FLAG_ACTUAL_COLLISION | SNP_FLAG_ACTUAL_GOAL);
         f |= (admin <= 0.0 ? SNP_FLAG_ACTUAL_COLLISION : 0) | (agoal ? SNP_FLAG_ACTUAL_GOAL : 0);
-        if (c.checks) c.checks[2] = admin;
+        if (checks) checks[2] = admin;
     }
-    *c.flags = f;
+    *flags = f;
 }
 
-template <typename T> int launch_large_checks(const snp_crowd *cr, const snp_step_opts *o, const void *view, const void *radius, long long M, cudaStream_t st) {
-    CheckArgs<T> c;
+// kBatch: E = cr->E envs of M humans each, the checks selected by pre / post; `clear` zeroes each env's flags and checks first.
+template <typename T, bool kBatch> int launch_large_checks(const snp_crowd *cr, const snp_step_opts *o, const void *view, const void *radius, long long M,
+                                                           cudaStream_t st, bool pre = true, bool post = true, bool clear = false) {
+    CheckArgsOf<T, kBatch> c;
     c.robot = (const T *)cr->robot; c.action = (const T *)o->action; c.view = (const T *)view; c.radius = (const T *)radius; c.M = M;
-    c.mode = o->robot_mode; c.pre = o->pre_checks != 0; c.post = o->post_checks != 0;
+    c.mode = o->robot_mode; c.pre = pre && o->pre_checks != 0; c.post = post && o->post_checks != 0;
+    unsigned n_ctas = 1;
+    if constexpr (kBatch) { c.E = cr->E; c.clear = clear; c.stride = (long long)cr->E * M; n_ctas = (unsigned)cr->E; }
     for (int k = 0; k < 6; ++k) c.consts[k] = o->consts[k];
     c.time_now = o->time_now; c.flags = o->flags; c.checks = o->checks;
-    k_large_checks<T><<<1, kCheckThreads, 0, st>>>(c);
+    k_large_checks<T, kBatch><<<n_ctas, kCheckThreads, 0, st>>>(c);
     count_launch();
     SNP_CUDA_OK(cudaGetLastError());
+    return SNP_OK;
+}
+
+// snp_large_batch_step after validation: publish, pre-checks, n_substeps x (robot step, tiled update) between the two view buffers of
+// the scratch, the robot's end state and the clock, post-checks.
+template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scratch, cudaStream_t st) {
+    const long long E = c->E, N = c->N, EN = E * N;
+    const LargeBatchScratch sb = large_batch_scratch(E, N, sizeof(T));
+    void *views[2] = {(char *)scratch + sb.view_a, (char *)scratch + sb.view_b};
+    k_large_publish<T><<<(unsigned)((EN + 255) / 256), 256, 0, st>>>((const T *)c->dyn, (const T *)c->stat, EN, o->type >= 3, (T *)views[0], EN, 0);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    const T *radius = (const T *)c->stat + SNP_STAT_R * EN;
+    if (o->pre_checks) {
+        const int rc = launch_large_checks<T, true>(c, o, views[0], radius, N, st, true, false, true);
+        if (rc) return rc;
+    }
+    // the finish kernel writes the next view's tile boxes when its CTAs are whole tiles (LargeCrowd's rule)
+    const bool fold_boxes = N % kTile == 0;
+    for (int s = 0; s < o->n_substeps; ++s) {
+        const void *next[1] = {views[(s + 1) & 1]};
+        const int rc = run_large<T>(c, o, views[s & 1], next, 1, EN, 0, fold_boxes, fold_boxes && s > 0, scratch, s, st, N);
+        if (rc) return rc;
+    }
+    if (o->n_substeps > 0 && ((c->robot && (o->robot_mode == 1 || o->robot_mode == 3)) || o->time_now)) {
+        const int rc = launch_large_robot_end<T, true>(c, o, o->n_substeps, st);
+        if (rc) return rc;
+    }
+    if (o->post_checks) return launch_large_checks<T, true>(c, o, views[o->n_substeps & 1], radius, N, st, false, true, !o->pre_checks);
     return SNP_OK;
 }
 
@@ -886,19 +1039,8 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
         cur_is_b ^= 1;
     }
     // the robot's end state and the clock: after every finish kernel of the call has read the start state
-    if (n_substeps > 0 && ((c->robot && (o->robot_mode == 1 || o->robot_mode == 3)) || o->time_now)) {
-        if (c->dtype == SNP_F64) {
-            KArgs<double> a{}; a.robot = (double *)c->robot; a.action = (const double *)o->action; a.robot_mode = o->robot_mode;
-            a.dt = o->dt; a.dt_d = o->dt; a.time_now = o->time_now;
-            k_large_robot_end<double><<<1, 1, 0, st>>>(a, n_substeps);
-        } else {
-            KArgs<float> a{}; a.robot = (float *)c->robot; a.action = (const float *)o->action; a.robot_mode = o->robot_mode;
-            a.dt = (float)o->dt; a.dt_d = o->dt; a.time_now = o->time_now;
-            k_large_robot_end<float><<<1, 1, 0, st>>>(a, n_substeps);
-        }
-        count_launch();
-        SNP_CUDA_OK(cudaGetLastError());
-    }
+    if (n_substeps > 0 && ((c->robot && (o->robot_mode == 1 || o->robot_mode == 3)) || o->time_now))
+        return c->dtype == SNP_F64 ? launch_large_robot_end<double, false>(c, o, n_substeps, st) : launch_large_robot_end<float, false>(c, o, n_substeps, st);
     return SNP_OK;
 }
 
@@ -912,8 +1054,43 @@ int snp_large_checks(const snp_crowd *c, const snp_step_opts *o, const void *vie
     if (o->robot_mode != 0 && o->robot_mode != 1 && o->robot_mode != 3) { set_error("snp_large_checks: robot_mode must be 0, 1 or 3 (got %d)", o->robot_mode); return SNP_ERR_INVALID; }
     if (o->pre_checks && !o->action) { set_error("snp_large_checks: pre_checks needs opts->action"); return SNP_ERR_INVALID; }
     if (!o->flags) { set_error("snp_large_checks: opts->flags is required"); return SNP_ERR_INVALID; }
-    return c->dtype == SNP_F64 ? launch_large_checks<double>(c, o, view, radius, M, (cudaStream_t)stream)
-                               : launch_large_checks<float>(c, o, view, radius, M, (cudaStream_t)stream);
+    return c->dtype == SNP_F64 ? launch_large_checks<double, false>(c, o, view, radius, M, (cudaStream_t)stream)
+                               : launch_large_checks<float, false>(c, o, view, radius, M, (cudaStream_t)stream);
+}
+
+int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype) {
+    if (E < 1 || N < 1 || (dtype != SNP_F64 && dtype != SNP_F32)) { set_error("snp_large_batch_scratch_bytes: E=%d N=%d dtype=%d", E, N, dtype); return -1; }
+    return large_batch_scratch(E, N, dtype == SNP_F64 ? 8 : 4).bytes;
+}
+
+int snp_large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scratch, int64_t scratch_bytes, void *stream) {
+    if (!c || !o || !scratch) { set_error("snp_large_batch_step: null argument"); return SNP_ERR_INVALID; }
+    if (c->E < 1 || c->N < 1 || c->G < 1) { set_error("snp_large_batch_step: E, N and G must be positive (E=%d N=%d G=%d)", c->E, c->N, c->G); return SNP_ERR_INVALID; }
+    if (c->dtype != SNP_F64 && c->dtype != SNP_F32) { set_error("snp_large_batch_step: bad dtype %d", c->dtype); return SNP_ERR_INVALID; }
+    if (o->type < 0 || o->type > 8) { set_error("snp_large_batch_step: type %d does not exist for this implementation", o->type); return SNP_ERR_INVALID; }
+    if (!c->dyn || !c->stat || !c->goals || !c->goal_idx || !c->goal_cnt) { set_error("snp_large_batch_step: crowd arrays missing"); return SNP_ERR_INVALID; }
+    if (c->W < 0 || c->S < 0 || (c->W > 0 && (!c->walls || c->S == 0))) { set_error("snp_large_batch_step: walls W=%d S=%d but no segment array", c->W, c->S); return SNP_ERR_INVALID; }
+    if (o->n_substeps < 0) { set_error("snp_large_batch_step: n_substeps must be >= 0"); return SNP_ERR_INVALID; }
+    if (o->robot_mode < 0 || o->robot_mode > 3) { set_error("snp_large_batch_step: robot_mode must be 0, 1 or 3 (got %d)", o->robot_mode); return SNP_ERR_INVALID; }
+    if (large_J(c->N) > 65535) { set_error("snp_large_batch_step: at most %d humans per env", 65535 * kChunk); return SNP_ERR_INVALID; }
+    if (o->robot_mode == 2) { set_error("snp_large_batch_step: robot_mode 2 (a robot moved by its own motion model) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->robot_every) { set_error("snp_large_batch_step: robot_every is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->track_touch) { set_error("snp_large_batch_step: track_touch is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->post_checks != 0 && o->post_checks != 1) { set_error("snp_large_batch_step: post_checks 2 (imitation-learning reward) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->dyn_out) { set_error("snp_large_batch_step: dyn_out (peek) is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (o->respawn) { set_error("snp_large_batch_step: respawn is not supported"); return SNP_ERR_UNSUPPORTED; }
+    if (c->agent_params) { set_error("snp_large_batch_step: per-agent parameter rows are not supported (uniform parameters only)"); return SNP_ERR_UNSUPPORTED; }
+    if ((o->consider_robot || o->robot_mode || o->pre_checks || o->post_checks) && !c->robot) {
+        set_error("snp_large_batch_step: consider_robot, robot_mode and the checks need crowd->robot"); return SNP_ERR_INVALID;
+    }
+    if ((o->robot_mode || o->pre_checks) && !o->action) { set_error("snp_large_batch_step: robot_mode 1 / 3 and pre_checks need opts->action"); return SNP_ERR_INVALID; }
+    if ((o->pre_checks || o->post_checks) && !o->flags) { set_error("snp_large_batch_step: the checks need opts->flags"); return SNP_ERR_INVALID; }
+    const long long need = large_batch_scratch(c->E, c->N, c->dtype == SNP_F64 ? 8 : 4).bytes;
+    if (scratch_bytes < need || reinterpret_cast<uintptr_t>(scratch) % 16) {
+        set_error("snp_large_batch_step: 16-byte aligned scratch of %lld bytes needed, %lld given", need, (long long)scratch_bytes);
+        return SNP_ERR_INVALID;
+    }
+    return c->dtype == SNP_F64 ? large_batch_step<double>(c, o, scratch, (cudaStream_t)stream) : large_batch_step<float>(c, o, scratch, (cudaStream_t)stream);
 }
 
 int snp_large_publish(const snp_crowd *c, int32_t type, void *view, int64_t stride, int64_t offset, void *stream) {

@@ -199,3 +199,55 @@ class LargeCrowd:
     def local_rows(self, template):
         """This rank's agents as reference rows; `template` [n_local,13] supplies the static columns."""
         return self.eng.rows(np.asarray(template, np.float64)[None])[0]
+
+
+class TiledCrowdEngine(CrowdEngine):
+    """CrowdEngine for E environments of any number of humans each, N > 512 included: `update_humans` and `step` run
+    snp_large_batch_step (the tiled kernels of LargeCrowd with an environment axis) in one call per step.  Environment e steps
+    bit for bit as a LargeCrowd built from environment e alone.  Loading and reading are CrowdEngine's (from_reference_arrays,
+    rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env).  Per-agent parameter rows, respawn
+    and the snp_step features the tiled path does not have (peek and the lookahead through it, imitation_learning_step, sim_update,
+    step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
+    carried from one step to the next.  culling=False evaluates every pair (the same result)."""
+
+    def __init__(self, *args, **kwargs):
+        super().__init__(*args, **kwargs)
+        dt = L.SNP_F64 if self.dtype == torch.float64 else L.SNP_F32
+        self.scratch = torch.empty(int(self.lib.snp_large_batch_scratch_bytes(self.E, self.N, dt)), dtype=torch.uint8, device=self.device)
+        self.culling = True
+
+    def _run(self, o):
+        o.reserved = 0 if self.culling else L.SNP_OPT_NO_CULLING
+        L.check(self.lib.snp_large_batch_step(ctypes.byref(self._crowd()), ctypes.byref(o), ctypes.c_void_p(self.scratch.data_ptr()),
+                                              self.scratch.numel(), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+
+    def update_humans(self, t=0.0, dt=0.0125, post_update=True, n_substeps=1):
+        """MotionModelManager.update_humans (motion_model_manager.py:354) for every env: `n_substeps` Euler updates in one call."""
+        self._run(self._opts(dt, n_substeps, post_update=post_update))
+
+    def step(self, action=None, dt=0.0125, n_substeps=20, pre_checks=True, post_checks=False, kinematics="holonomic"):
+        """SocialNavGym.step for every env (social_nav_gym.py:227-250), as CrowdEngine.step: the swept check on the current state,
+        `n_substeps` x (robot.step(action, dt); update_humans(dt)), the actual check on the end state (post_checks).  `action` [E,2]
+        (vx, vy), or (v, r) with kinematics="unicycle"; None reuses self.action.  Results in self.flags / checks / time_now."""
+        if kinematics not in ("holonomic", "unicycle"):
+            raise ValueError("kinematics must be 'holonomic' or 'unicycle'")
+        if action is not None:
+            a = torch.as_tensor(action, dtype=self.dtype, device=self.device)
+            self.action.copy_(a.t() if a.shape == (self.E, 2) else a)
+        self._run(self._opts(dt, n_substeps, robot_mode=1 if kinematics == "holonomic" else 3, pre_checks=pre_checks,
+                             post_checks=post_checks, advance_time=True))
+
+    def _unsupported(self, what):
+        raise NotImplementedError(f"TiledCrowdEngine: {what} is not available on the tiled path (snp_large_batch_step)")
+
+    def peek(self, dt):
+        self._unsupported("peek (and the lookahead and observable states through it)")
+
+    def imitation_learning_step(self, dt=0.0125, n_substeps=20):
+        self._unsupported("imitation_learning_step (robot_mode 2)")
+
+    def sim_update(self, dt=0.0125, n_updates=1, robot_every=1, robot_time_step=None, phase=0):
+        self._unsupported("sim_update (robot_mode 2, track_touch)")
+
+    def step_host(self, *args, **kwargs):
+        self._unsupported("step_host")
