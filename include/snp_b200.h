@@ -53,7 +53,8 @@ typedef enum snp_status {
 
 enum { SNP_F32 = 0, SNP_F64 = 1 };
 enum { SNP_OPT_FULL_PAIR_LOOP = 1, SNP_OPT_NO_CULLING = 2, SNP_OPT_MAP_WARP = 4, SNP_OPT_MAP_BLOCK = 8,
-       SNP_OPT_STAGED_COPIES = 16  /* snp_gym_step_host: D2H copies after the launch even for pinned result buffers */ };
+       SNP_OPT_STAGED_COPIES = 16, /* snp_gym_step_host: D2H copies after the launch even for pinned result buffers */
+       SNP_OPT_UNIT_SCRATCH = 32   /* snp_large_run_p2p / snp_large_batch_step: the scratch was sized by snp_large_*scratch_bytes_units */ };
 
 /* Field order of the structure-of-arrays buffers (each field is a contiguous run of E*N elements). */
 enum { SNP_DYN_PX = 0, SNP_DYN_PY, SNP_DYN_VX, SNP_DYN_VY, SNP_DYN_TH, SNP_DYN_BVX, SNP_DYN_BVY, SNP_DYN_OM,
@@ -252,12 +253,26 @@ int snp_rotate_goal_rows(const snp_crowd *crowd, double *goal_rows_dev, void *cu
  * of the slices) runs between calls of one sub-step with world = 1.  `scratch` = 16-byte aligned device workspace of at least
  * snp_large_scratch_bytes(n_local, M, dtype) bytes (per-chunk partial sums, the map and lists of the (agent block, entity chunk)
  * units in reach, the work queues' counters).  opts->reserved bit 1 (SNP_OPT_NO_CULLING) disables the exact far-tile culling.
+ * opts->reserved bit 5 (SNP_OPT_UNIT_SCRATCH): the scratch was sized by snp_large_scratch_bytes_units(n_local, M, dtype, units); a culled
+ * step then keeps the partial sums of a unit in reach in slot k = its position on the work list, of floor(extra bytes / (2 * 128 *
+ * sizeof(T))) slots (0 or more), so memory follows the units in reach instead of n_local * M.  A unit without a slot is evaluated by
+ * the finish kernel in its place in the order: the result is bit for bit that of the default scratch whatever the slot count; it only
+ * costs time.  With the bit, before any launch, what needs the static grid is SNP_ERR_UNSUPPORTED: Moussaid types (2, 5, 8),
+ * SNP_OPT_NO_CULLING, pair-law parameters without a culling distance, a self_offset that is not a multiple of 128,
+ * ceil(n_local/128) * ceil(M/128) >= 2^31 units; and the scratch must be at least the size for 0 units.  Unit counts of the call (with
+ * the bit): int32 word 1 of the scratch = the most units listed in one sub-step, word 2 = the units the finish kernel evaluated for
+ * want of a slot; the call's first launch zeroes them, and nothing synchronises.  Without the bit the scratch and the kernels are
+ * the default ones, and words 1 and 2 hold nothing.
  * The robot of SocialNavGym.step (crowd->robot, one env): opts->robot_mode 0 (fixed), 1 (holonomic action) or 3 (unicycle action)
  * moves it before every sub-step as snp_step does, and opts->consider_robot adds its pair force to every human (never culled).  Every
  * rank recomputes the robot of each sub-step from crowd->robot, so no exchange is needed; after the last sub-step crowd->robot holds
  * the end state and opts->time_now (optional) has advanced by dt per sub-step.  The checks are snp_large_checks.  robot_mode 2,
  * track_touch, pre_checks / post_checks, dyn_out and respawn are SNP_ERR_UNSUPPORTED, before any launch. */
 int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype);
+/* The scratch of a culled step with `units` slots of partial sums (SNP_OPT_UNIT_SCRATCH); host arithmetic, -1 for bad arguments
+ * (n_local < 1, M < n_local, units < 0, bad dtype).  At units = ceil(n_local/128) * ceil(M/128) and n_local a multiple of 128 it
+ * equals snp_large_scratch_bytes. */
+int64_t snp_large_scratch_bytes_units(int64_t n_local, int64_t M, int32_t dtype, int64_t units);
 int snp_large_run_p2p(const snp_crowd *crowd, const snp_step_opts *opts, const void *const *peer_views_a, const void *const *peer_views_b,
                       int32_t first_is_b, int64_t M, int64_t self_offset, int32_t world, int32_t rank, const void *const *peer_flags,
                       uint64_t epoch_base, int32_t n_substeps, int32_t *error_flag, void *scratch, int64_t scratch_bytes, void *cuda_stream);
@@ -283,8 +298,11 @@ int snp_large_checks(const snp_crowd *crowd, const snp_step_opts *opts, const vo
  * partial sums [ceil(N/128)][2][E*N], the live map and the work lists; nothing is carried from one call to the next.  Before any
  * launch: robot_mode 2, robot_every, track_touch, post_checks 2, dyn_out, respawn and crowd->agent_params are SNP_ERR_UNSUPPORTED;
  * bad E / N / G / dtype / type, missing arrays, a missing robot / action / flags and too small a scratch are SNP_ERR_INVALID.
- * snp_large_batch_scratch_bytes returns -1 for bad arguments. */
+ * snp_large_batch_scratch_bytes returns -1 for bad arguments.  SNP_OPT_UNIT_SCRATCH and the unit counts in words 1 and 2 of the
+ * scratch are as for snp_large_run_p2p, with a scratch of snp_large_batch_scratch_bytes_units(E, N, dtype, units) bytes (units of
+ * E * ceil(N/128) * ceil(N/128); Moussaid types and SNP_OPT_NO_CULLING refused); the same bits whatever the slot count. */
 int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype);
+int64_t snp_large_batch_scratch_bytes_units(int32_t E, int32_t N, int32_t dtype, int64_t units);
 int snp_large_batch_step(const snp_crowd *crowd, const snp_step_opts *opts, void *scratch, int64_t scratch_bytes, void *cuda_stream);
 /* Writes this crowd's [5][.] entity view (x,y,vx,vy,r+safety; v = R(yaw) bv for headed models) into `view` (field stride
  * `stride` elements, starting at element `offset`). */

@@ -11,6 +11,7 @@ LIB_PATH = os.environ.get("SNP_B200_LIB", os.path.join(_HERE, "libsnp_b200.so"))
 SNP_F32, SNP_F64 = 0, 1
 # bits of snp_step_opts.reserved (include/snp_b200.h)
 SNP_OPT_FULL_PAIR_LOOP, SNP_OPT_NO_CULLING, SNP_OPT_MAP_WARP, SNP_OPT_MAP_BLOCK, SNP_OPT_STAGED_COPIES = 1, 2, 4, 8, 16
+SNP_OPT_UNIT_SCRATCH = 32
 # field order of the SoA buffers (include/snp_b200.h)
 DYN_PX, DYN_PY, DYN_VX, DYN_VY, DYN_TH, DYN_BVX, DYN_BVY, DYN_OM, DYN_DFX, DYN_DFY, DYN_FIELDS = range(11)
 STAT_R, STAT_M, STAT_VD, STAT_SAFETY, STAT_FIELDS = range(5)
@@ -82,11 +83,13 @@ _SIGNATURES = {
     "snp_unpack_goals": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_void_p, c_void_p, c_void_p]),
     "snp_rotate_goal_rows": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_void_p, c_void_p]),
     "snp_large_scratch_bytes": (c_int64, [c_int64, c_int64, c_int32]),
+    "snp_large_scratch_bytes_units": (c_int64, [c_int64, c_int64, c_int32, c_int64]),
     "snp_large_checks": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_void_p, c_int64, c_void_p]),
     "snp_large_publish": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_int32, c_void_p, c_int64, c_int64, c_void_p]),
     "snp_large_run_p2p": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_void_p, c_int32, c_int64, c_int64, c_int32,
                                          c_int32, c_void_p, ctypes.c_uint64, c_int32, c_void_p, c_void_p, c_int64, c_void_p]),
     "snp_large_batch_scratch_bytes": (c_int64, [c_int32, c_int32, c_int32]),
+    "snp_large_batch_scratch_bytes_units": (c_int64, [c_int32, c_int32, c_int32, c_int64]),
     "snp_large_batch_step": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_int64, c_void_p]),
     "snp_update_humans_parallel_host":(ctypes.c_int, [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                                        c_void_p, c_double, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,
@@ -120,6 +123,13 @@ def lib():
             fn.restype, fn.argtypes = res, args
         _lib = handle
     return _lib
+
+
+def check_size(n: int) -> int:
+    """A byte count from a *_scratch_bytes* function, or the ValueError of its -1."""
+    if n < 0:
+        raise ValueError(lib().snp_last_error().decode())
+    return n
 
 
 def check(rc: int):

@@ -88,9 +88,14 @@ template <typename T> struct LargeArgs {
     // (i-block, chunk) only ever pairs humans of one env; the global tile of env e's tile t is e * env_tiles + t.
     long long env_n;
     int env_tiles, env_iblocks, env_fblocks;  // per env: 128-entity tiles (= chunks), i-blocks of the pair phase, finish CTAs
+    // Work list: entry k writes its partial sums to slot k of the [cap][2][128] region `partial`.  An entry k >= cap has no slot: the
+    // pairs kernel skips it, the i-block's list holds -1 - chunk, and the finish kernel evaluates the chunk itself.
+    int cap;
 };
 constexpr int kMaxQueues = 256;                 // one queue of list entries per SM (entry k belongs to queue k mod n_queues)
-constexpr int kWorkCounters = 4 + kMaxQueues;   // ints in front of the list
+// The counter block (the first ints of the scratch): [0] entries listed in this sub-step, [1] most entries listed in one sub-step of
+// the call, [2] units the finish kernel evaluated in the call, [3] unused, [4 + q] entries handed out from queue q.
+constexpr int kWorkCounters = 4 + kMaxQueues;
 
 template <typename T> __device__ __forceinline__ T warp_min(T v) {
     for (int o = 16; o > 0; o >>= 1) { const T w = __shfl_xor_sync(0xffffffffu, v, o); v = w < v ? w : v; }
@@ -177,16 +182,25 @@ template <typename T> struct PairsSmem {
     T sbox[20];
     int item, steal;
 };
+// What the finish kernel stages besides its exp table to evaluate a unit the partial sums had no slot for: one tile and the box
+// reduction's scratch.
+template <typename T> struct TileSmem {
+    alignas(16) unsigned char tile_raw[sizeof(Ent<T>) * kTile];
+    T tile_rs[kTile];
+    T sbox[20];
+};
 
-// One (i-block, chunk) unit of the pair phase: the i-block's agents against the chunk's entities, one partial sum per agent.
-// In a batch the i-block and the chunk are those of one env: agents and entities are numbered from the env's first (base), so that
-// Moussaid's jj < idx compares indices in the same numbering.
-template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
-__device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T> &sm, int iblock, int chunk, bool &have_tbl) {
-    Ent<T> *tile = reinterpret_cast<Ent<T> *>(sm.tile_raw);
-    T *tile_rs = sm.tile_rs;
-    double *exp_tbl_s = sm.exp_tbl_s;
-    T *sbox = sm.sbox;
+// One (i-block, chunk) unit of the pair phase: the i-block's agents against the chunk's entities, one partial sum per agent, from
+// zero in ascending entity order.  All 128 threads of the CTA take part.  In a batch the i-block and the chunk are those of one env:
+// agents and entities are numbered from the env's first (base), so that Moussaid's jj < idx compares indices in the same numbering.
+// Where the sums go (kOut): kToGrid [J][2][N_local] by chunk and agent (the static grid); kToSlot slot `slot` of the [cap][2][128]
+// region, agent = thread (the work list, one agent per thread); kToCaller *out_x / *out_y (the finish kernel's units without a
+// slot: one agent per thread, the `live` map left alone).
+enum { kToGrid = 0, kToSlot = 1, kToCaller = 2 };
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch, int kOut = kToGrid>
+__device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, unsigned char *tile_raw, T *tile_rs, double *exp_tbl_s, T *sbox, int iblock,
+                                            int chunk, bool &have_tbl, int slot = 0, T *out_x = nullptr, T *out_y = nullptr) {
+    Ent<T> *tile = reinterpret_cast<Ent<T> *>(tile_raw);
     const KArgs<T> &a = la.k;
     const long long N = a.EN, M = la.M;
     const Params<T> &P = a.P;
@@ -316,11 +330,24 @@ __device__ __forceinline__ void pairs_chunk(const LargeArgs<T> &la, PairsSmem<T>
             }
         }
     }
+    if constexpr (kOut == kToCaller) {
+        static_assert(kAgentsPerThread == 1, "the finish kernel runs one agent per thread");
+        *out_x = fsx[0]; *out_y = fsy[0];
+        return;
+    }
     if (threadIdx.x == 0) *live_flag = any_tile ? 1 : 0;
     // Every tile culled: on the static grid the finish kernel reads `live` and skips the chunk, so nothing is written.  A unit on
     // the work list is added whatever happened here, and k_large_cull listed it from the tile box of the i-block, which for the
     // last, partly foreign tile of a slice ending inside the view is larger than the box of the agents tested above: such a unit
     // writes its (zero) partial sums.
+    if constexpr (kOut == kToSlot) {
+        static_assert(kAgentsPerThread == 1, "the work list runs one agent per thread");
+        if (idx[0] < n_env) {
+            la.partial[((size_t)slot * 2 + 0) * kTile + threadIdx.x] = fsx[0];
+            la.partial[((size_t)slot * 2 + 1) * kTile + threadIdx.x] = fsy[0];
+        }
+        return;
+    }
     if (!any_tile && !la.use_list) return;
 #pragma unroll
     for (int q = 0; q < kAgentsPerThread; ++q)
@@ -337,7 +364,7 @@ template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
 __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
     __shared__ PairsSmem<T> sm;
     bool have_tbl = false;  // the 16 kB exp table is staged only by CTAs that evaluate at least one tile (most are culled)
-    pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm, blockIdx.x, blockIdx.y, have_tbl);
+    pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, blockIdx.x, blockIdx.y, have_tbl);
 }
 
 // Culled steps of a wide crowd: of the i-blocks x J grid only a few percent of the CTAs have anything to evaluate (65536 humans on
@@ -349,7 +376,9 @@ __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
 // queue of the SM it runs on (%smid) and only when that is empty looks for another queue with entries left: every SM gets the
 // same number of entries whatever the placement of the CTAs, and every entry is taken whichever CTAs exist.  Partial sums land
 // where the grid version puts them: results are bit-identical.
-template <typename T, bool kBatch> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
+// kSlots (SNP_OPT_UNIT_SCRATCH): the i-block's list holds each unit's slot of the partial sums (its index on the work list), or
+// -1 - chunk when the index is beyond the slots; otherwise the chunk.
+template <typename T, bool kBatch, bool kSlots = false> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
     __shared__ int warp_cnt[8];
     T u[5];
     iblock_box<T, kBatch>(la, blockIdx.x, la.apt, u);
@@ -363,10 +392,12 @@ template <typename T, bool kBatch> __global__ void __launch_bounds__(256) k_larg
         if (c < la.J) la.live[(size_t)blockIdx.x * la.Jp + c] = near ? 1 : 0;
         const unsigned m = __ballot_sync(0xffffffffu, near);
         const int below = __popc(m & ((1u << lane) - 1u));
+        [[maybe_unused]] int slot = 0;
         if (m) {  // the global list of work units (any order)
             int base = 0;
             if (lane == __ffs(m) - 1) base = atomicAdd(la.work_counters, __popc(m));
             base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
+            if constexpr (kSlots) slot = base + below;
             if (near) la.work[base + below] = blockIdx.x * la.J + c;
         }
         // this i-block's own list, ascending: the order the finish kernel adds the partial sums in
@@ -375,18 +406,23 @@ template <typename T, bool kBatch> __global__ void __launch_bounds__(256) k_larg
         int before = 0, total = 0;
 #pragma unroll
         for (int w = 0; w < 8; ++w) { const int v = warp_cnt[w]; before += w < warp ? v : 0; total += v; }
-        if (near) mine[listed + before + below] = c;
+        if constexpr (kSlots) {
+            if (near) mine[listed + before + below] = slot < la.cap ? slot : -1 - c;
+        } else {
+            if (near) mine[listed + before + below] = c;
+        }
         listed += total;
         __syncthreads();
     }
     if (threadIdx.x == 0) la.live_cnt[blockIdx.x] = listed;
 }
 
-template <typename T, int SOC, int kAgentsPerThread, bool kBatch>
+// kSlots (SNP_OPT_UNIT_SCRATCH): entry k writes slot k of the partial sums, and entries beyond the slots are left to the finish kernel.
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch, bool kSlots = false>
 __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> la, const int n_queues) {
     __shared__ PairsSmem<T> sm;
     bool have_tbl = false;
-    const int n_items = la.work_counters[0];
+    const int n_items = kSlots ? min(la.work_counters[0], la.cap) : la.work_counters[0];
     int *cursor = la.work_counters + 4;
     unsigned smid;
     asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
@@ -402,7 +438,8 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
         const int item = sm.item;
         if (item >= 0) {
             const int w = la.work[item];
-            pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm, w / la.J, w % la.J, have_tbl);
+            if constexpr (kSlots) pairs_chunk<T, SOC, kAgentsPerThread, kBatch, kToSlot>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, w / la.J, w % la.J, have_tbl, item);
+            else pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, w / la.J, w % la.J, have_tbl);
             continue;
         }
         // this queue is empty (and stays so: the counters only grow): move to the nearest queue that still has entries, if any
@@ -437,10 +474,64 @@ template <typename T, bool kBatch> __device__ __forceinline__ void large_robot_r
     }
 }
 
+// The sum of the partial sums on i-block `row`'s ascending list (the order is what makes the result independent of the sharding and
+// of which units had a slot), this thread's agent = lane of the slots.  Sixteen entries per step, the next sixteen already on their
+// way while the partial sums of the current ones are loaded.  FSOC >= 0 (the CTA is the whole i-block, every thread present): an
+// entry -1 - chunk had no slot, and the chunk is evaluated here with the pairs kernel's code, in its place in the order.
+template <typename T, int FSOC, bool kBatch>
+__device__ __forceinline__ void sum_listed(const LargeArgs<T> &la, long long row, T &fsx, T &fsy, double *exp_tbl_s, TileSmem<T> *ts) {
+    const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)row * la.Jp);
+    const int cnt = la.live_cnt[row];
+    int4 nxt[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) nxt[u] = ll[u];  // (a row is Jp >= 16 entries long; entries beyond cnt are ignored)
+    for (int k = 0; k < cnt; k += 16) {
+        int4 cur[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) cur[u] = nxt[u];
+        if (k + 16 < cnt) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) nxt[u] = ll[(k >> 2) + 4 + u];
+        }
+        const int idx[16] = {cur[0].x, cur[0].y, cur[0].z, cur[0].w, cur[1].x, cur[1].y, cur[1].z, cur[1].w,
+                             cur[2].x, cur[2].y, cur[2].z, cur[2].w, cur[3].x, cur[3].y, cur[3].z, cur[3].w};
+        if constexpr (FSOC >= 0) {
+            bool miss = false;  // (uniform: the list is the CTA's)
+#pragma unroll
+            for (int b = 0; b < 16; ++b) miss |= k + b < cnt && idx[b] < 0;
+            if (miss) {  // one entry at a time
+#pragma unroll 1
+                for (int b = k; b < k + 16 && b < cnt; ++b) {
+                    const int s = la.live_list[(size_t)row * la.Jp + b];
+                    T vx, vy;
+                    if (s >= 0) {
+                        vx = la.partial[((size_t)s * 2 + 0) * kTile + threadIdx.x]; vy = la.partial[((size_t)s * 2 + 1) * kTile + threadIdx.x];
+                    } else {
+                        bool have_tbl = true;  // staged by the caller
+                        pairs_chunk<T, FSOC, 1, kBatch, kToCaller>(la, ts->tile_raw, ts->tile_rs, exp_tbl_s, ts->sbox, (int)row, -1 - s, have_tbl, 0, &vx, &vy);
+                        if (threadIdx.x == 0) atomicAdd(la.work_counters + 2, 1);
+                    }
+                    fsx += vx; fsy += vy;
+                }
+                continue;
+            }
+        }
+        T vx[16], vy[16];
+#pragma unroll
+        for (int b = 0; b < 16; ++b)
+            if (k + b < cnt) { vx[b] = la.partial[((size_t)idx[b] * 2 + 0) * kTile + threadIdx.x]; vy[b] = la.partial[((size_t)idx[b] * 2 + 1) * kTile + threadIdx.x]; }
+#pragma unroll
+        for (int b = 0; b < 16; ++b)
+            if (k + b < cnt) { fsx += vx[b]; fsy += vy[b]; }
+    }
+}
+
 // RSOC: the pair law of the visible robot's force (SOC of the humans' model), or -1 for no robot -- a separate instantiation, so
 // that the common ones keep their registers.  kBatch: CTA b of env e is block e * env_fblocks + b and covers humans 128 b ... of env
-// e only, so that it stages its own env's walls.
-template <typename T, int OBS, int HEADED, int RSOC, bool kBatch>
+// e only, so that it stages its own env's walls.  FSOC >= 0 (steps with SNP_OPT_UNIT_SCRATCH, another instantiation): the list holds
+// slots of the [cap][2][128] partial sums, and -1 - chunk for a unit without one, which this kernel evaluates with the pair law FSOC
+// (sum_listed; a tile staged in TileSmem after the segment counts, and the exp table).
+template <typename T, int OBS, int HEADED, int RSOC, bool kBatch, int FSOC = -1>
 __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     using R = Real<T>;
     const KArgs<T> &a = la.k;
@@ -450,7 +541,7 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     constexpr size_t kTbl = sizeof(double) * kExpN;
     Seg<T> *segs = reinterpret_cast<Seg<T> *>(smem_raw + kTbl);
     int *seg_cnt = reinterpret_cast<int *>(smem_raw + kTbl + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)));
-    if (sizeof(T) == 8 && (nseg > 0 || RSOC >= 0)) exp_table_init(exp_tbl_s);  // only the wall force and the robot evaluate exp here
+    if (sizeof(T) == 8 && (nseg > 0 || RSOC >= 0 || FSOC >= 0)) exp_table_init(exp_tbl_s);  // only the wall force, the robot and units without a slot evaluate exp here
     int env = 0;
     const T *walls = a.walls;
     if constexpr (kBatch) {
@@ -477,8 +568,19 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     } else {
         i = (long long)blockIdx.x * kTile + threadIdx.x; gone = i >= N;
     }
-    if (la.use_list && blockIdx.x == 0)  // the pair phase is over: empty list and queues for the next sub-step
-        for (int k = threadIdx.x; k < kWorkCounters; k += kTile) la.work_counters[k] = 0;
+    if constexpr (FSOC < 0) {
+        if (la.use_list && blockIdx.x == 0)  // the pair phase is over: empty list and queues for the next sub-step
+            for (int k = threadIdx.x; k < kWorkCounters; k += kTile) la.work_counters[k] = 0;
+    } else if (blockIdx.x == 0) {  // the same, but the call's unit counts (words 1-3) stay; word 1 keeps the most units listed
+        if (threadIdx.x == 0) la.work_counters[1] = max(la.work_counters[1], la.work_counters[0]);
+        for (int k = threadIdx.x; k < kWorkCounters; k += kTile)
+            if (k == 0 || k >= 4) la.work_counters[k] = 0;
+    }
+    [[maybe_unused]] T listed_x = T(0), listed_y = T(0);
+    if constexpr (FSOC >= 0) {  // before any thread leaves: the units without a slot are evaluated by the whole CTA (= the i-block)
+        const size_t seg_end = kTbl + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + ((sizeof(int) * (size_t)(a.W + 1) + 15) & ~size_t(15));
+        sum_listed<T, FSOC, kBatch>(la, blockIdx.x, listed_x, listed_y, exp_tbl_s, reinterpret_cast<TileSmem<T> *>(smem_raw + seg_end));
+    }
     const bool fold_boxes = la.peer_boxes[0] != nullptr;  // uniform; only offered when N is a whole number of tiles, so that every
     if (gone) return;                                      // thread of every block reaches the box reduction at the end
     const unsigned vote_mask = __activemask();  // the lanes that own an agent (the tail warp is partial)
@@ -501,6 +603,7 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     const int gcnt = a.goal_cnt[i];
     m.gx = a.goals[((size_t)gidx * 2 + 0) * N + i]; m.gy = a.goals[((size_t)gidx * 2 + 1) * N + i];
     T fsx = T(0), fsy = T(0);
+    if constexpr (FSOC >= 0) { fsx = listed_x; fsy = listed_y; }
     // Sum of the live chunks' partial sums in ascending chunk order (the order is what makes the result independent of the
     // sharding).  The flags are the same for the whole CTA and live chunks come in runs; they are read 64 at a time, and for every
     // 16 flags with a live one the loads of all live partial sums are issued together before the (ordered) additions -- a
@@ -508,7 +611,7 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     const long long row = kBatch ? (long long)env * la.env_iblocks + r / (kTile * la.apt) : i / (kTile * la.apt);  // the agent's i-block
     const uint4 *lv = reinterpret_cast<const uint4 *>(la.live + (size_t)row * la.Jp);
     const int n_words = la.use_list ? 0 : la.Jp >> 4;
-    if (la.use_list) {
+    if (FSOC < 0 && la.use_list) {
         // the cull kernel left the i-block's live chunks as an ascending list: sixteen indices per step, the next sixteen already on
         // their way while the partial sums of the current ones are loaded
         const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)row * la.Jp);
@@ -653,7 +756,9 @@ template <typename T> __global__ void k_large_publish(const T *dyn, const T *sta
     view[4 * stride + o] = stat[SNP_STAT_R * N + i] + stat[SNP_STAT_SAFETY * N + i];
 }
 
-template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_large(const LargeArgs<T> &la, cudaStream_t st) {
+// unit_slots (SNP_OPT_UNIT_SCRATCH, never Moussaid): the culled step through the slot instantiations of the cull, pairs and finish
+// kernels; `first`: the call's first sub-step.
+template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_large(const LargeArgs<T> &la, bool unit_slots, bool first, cudaStream_t st) {
     const long long N = la.k.EN;
     const int nseg = la.k.W * la.k.S;
     if (sizeof(T) == 8) SNP_CUDA_OK(ensure_exp_table());
@@ -662,6 +767,16 @@ template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_larg
     dim3 grid((unsigned)(kBatch ? (long long)la.k.E * la.env_iblocks : (N + per_block - 1) / per_block), (unsigned)la.J);
     if constexpr (SOC == 2) {  // Moussaid's pair law has no culling distance (run_large): every pair, two agents per thread
         k_large_pairs<T, SOC, kMaxAgentsPerThread, kBatch><<<grid, kTile, 0, st>>>(la);
+    } else if (la.use_list && unit_slots) {  // (culled, partial sums in slots)
+        // the counters start empty: zeroed here on the call's first sub-step (the call's unit counts too), else by the previous
+        // sub-step's finish kernel
+        if (first) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
+        k_large_cull<T, kBatch, true><<<grid.x, 256, 0, st>>>(la);
+        static int slots = 0;  // resident CTAs per SM
+        const int n_queues = device_sm_count() < kMaxQueues ? device_sm_count() : kMaxQueues;
+        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1, kBatch, true>, kTile, 0));
+        k_large_pairs_list<T, SOC, 1, kBatch, true><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
+        count_launch();
     } else if (la.use_list) {  // (culled: one agent per thread)
         // the counters start empty: zeroed here on a sub-step that computes the tile boxes, else by the previous sub-step's finish kernel
         if (!la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
@@ -673,8 +788,17 @@ template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_larg
         count_launch();
     } else if (la.apt == 1) k_large_pairs<T, SOC, 1, kBatch><<<grid, kTile, 0, st>>>(la);
     else k_large_pairs<T, SOC, 2, kBatch><<<grid, kTile, 0, st>>>(la);
-    const size_t smem = sizeof(double) * kExpN + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + sizeof(int) * (la.k.W + 1) + 16;
+    size_t smem = sizeof(double) * kExpN + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + sizeof(int) * (la.k.W + 1) + 16;
     auto fin = la.k.consider_robot ? k_large_finish<T, OBS, HEADED, SOC, kBatch> : k_large_finish<T, OBS, HEADED, -1, kBatch>;
+    if constexpr (SOC != 2) {
+        // partial sums in slots: the finish instantiation that reads them and evaluates the units without one (a tile staged after
+        // the segment counts)
+        if (la.use_list && unit_slots) {
+            fin = la.k.consider_robot ? k_large_finish<T, OBS, HEADED, SOC, kBatch, SOC> : k_large_finish<T, OBS, HEADED, -1, kBatch, SOC>;
+            smem = sizeof(double) * kExpN + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + ((sizeof(int) * (size_t)(la.k.W + 1) + 15) & ~size_t(15)) +
+                   sizeof(TileSmem<T>);
+        }
+    }
     if (smem > 48 * 1024) SNP_CUDA_OK(cudaFuncSetAttribute(fin, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     fin<<<(unsigned)(kBatch ? (long long)la.k.E * la.env_fblocks : (N + kTile - 1) / kTile), kTile, smem, st>>>(la);
     count_launch(la.boxes_ready ? 2 : 3);
@@ -688,48 +812,64 @@ inline long long large_iblocks(long long N) { return (N + kTile - 1) / kTile; } 
 
 inline long long up16(long long b) { return (b + 15) & ~15LL; }
 
-// The scratch of n_local agents in `blocks` i-blocks against J chunks: byte offsets of its regions (the partial sums at 0) and its
-// size.  Every region starts 16-byte aligned (the finish kernel reads the live map and the lists 16 bytes at a time).
-struct LargeScratch { long long live, counters, work, live_cnt, live_list, bytes; };
-inline LargeScratch large_scratch_units(long long n_local, long long J, long long blocks, long long elem_bytes) {
+// The scratch of `blocks` i-blocks against J chunks with `partial_bytes` of partial sums: byte offsets of its regions (the counters
+// at 0) and its size.  Every region starts 16-byte aligned (the finish kernel reads the live map and the lists 16 bytes at a time).
+// The partial sums are [J][2][n_local] on the static grid (the default size) or, on the work list, [cap][2][128] slots; a multiple
+// of 16 bytes more of them moves every later region by exactly that much.
+struct LargeScratch { long long partial, live, work, live_cnt, live_list, bytes; };
+inline LargeScratch large_scratch_regions(long long partial_bytes, long long J, long long blocks) {
     const long long Jp = (J + 15) & ~15LL;
     LargeScratch s;
-    s.live = up16(elem_bytes * J * 2 * n_local);      // [J][2][n_local] partial sums
-    s.counters = up16(s.live + blocks * Jp);           // [blocks][Jp] live map
-    s.work = s.counters + 4 * kWorkCounters;           // counters and queues
-    s.live_cnt = up16(s.work + 4 * blocks * J);        // [blocks * J] list of the units in reach
-    s.live_list = up16(s.live_cnt + 4 * blocks);       // [blocks] live chunks per i-block
-    s.bytes = s.live_list + 4 * blocks * Jp;           // [blocks][Jp] their indices, ascending
+    s.partial = up16(4 * kWorkCounters);               // counters and queues (kWorkCounters ints), then the partial sums
+    s.live = up16(s.partial + partial_bytes);          // [blocks][Jp] live map
+    s.work = up16(s.live + blocks * Jp);               // [blocks * J] list of the units in reach
+    s.live_cnt = up16(s.work + 4 * blocks * J);        // [blocks] live chunks per i-block
+    s.live_list = up16(s.live_cnt + 4 * blocks);       // [blocks][Jp] their slots (or -1 - chunk), ascending by chunk
+    s.bytes = s.live_list + 4 * blocks * Jp;
     return s;
 }
-// One crowd: n_local agents against M entities.
-inline LargeScratch large_scratch(long long n_local, long long M, long long elem_bytes) {
-    return large_scratch_units(n_local, large_J(M), large_iblocks(n_local), elem_bytes);
+inline long long unit_bytes(long long elem_bytes) { return 2 * kTile * elem_bytes; }  // one slot: [2][128]
+// One crowd: n_local agents against M entities; units < 0: the default size, [J][2][n_local] partial sums.
+inline LargeScratch large_scratch(long long n_local, long long M, long long elem_bytes, long long units = -1) {
+    const long long J = large_J(M);
+    return large_scratch_regions(units < 0 ? elem_bytes * J * 2 * n_local : units * unit_bytes(elem_bytes), J, large_iblocks(n_local));
 }
 // A batch of E envs of N humans: the regions above (chunks and i-blocks per env), then the two view buffers, each [5][E N] entities
 // and the [E ceil(N/128)][5] tile boxes.
 struct LargeBatchScratch { LargeScratch s; long long view_a, view_b, bytes; };
-inline LargeBatchScratch large_batch_scratch(long long E, long long N, long long elem_bytes) {
+inline LargeBatchScratch large_batch_scratch(long long E, long long N, long long elem_bytes, long long units = -1) {
     LargeBatchScratch b;
-    b.s = large_scratch_units(E * N, large_J(N), E * large_iblocks(N), elem_bytes);
+    const long long J = large_J(N);
+    b.s = large_scratch_regions(units < 0 ? elem_bytes * J * 2 * E * N : units * unit_bytes(elem_bytes), J, E * large_iblocks(N));
     const long long view = up16(elem_bytes * 5 * (E * N + E * large_tiles(N)));
     b.view_a = up16(b.s.bytes);
     b.view_b = b.view_a + view;
     b.bytes = b.view_b + view;
     return b;
 }
+// The slots a scratch of `scratch_bytes` holds (SNP_OPT_UNIT_SCRATCH): what is left after the regions of a scratch with none.
+inline long long units_in(long long scratch_bytes, long long bytes_for_none, long long elem_bytes) {
+    return scratch_bytes < bytes_for_none ? -1 : (scratch_bytes - bytes_for_none) / unit_bytes(elem_bytes);
+}
+// Does a step take the work list (culled, one agent per thread) and hence the slot layout?  Otherwise the static grid.
+inline bool large_uses_list(const snp_crowd *c, const snp_step_opts *o, long long self_offset, long long blocks, long long J) {
+    const int soc = o->type % 3;
+    const bool culled = !(o->reserved & SNP_OPT_NO_CULLING) &&
+                        ((soc == 0 && c->params[3] > 0) || (soc == 1 && c->params[3] > 0 && c->params[7] > 0));
+    return culled && self_offset % kTile == 0 && blocks * J < (1LL << 31);
+}
 
-template <typename T, bool kBatch> int dispatch_large(int type, const LargeArgs<T> &la, cudaStream_t st) {
+template <typename T, bool kBatch> int dispatch_large(int type, const LargeArgs<T> &la, bool unit_slots, bool first, cudaStream_t st) {
     switch (type) {
-        case 0: return launch_large<T, 0, 0, 0, kBatch>(la, st);
-        case 1: return launch_large<T, 1, 1, 0, kBatch>(la, st);
-        case 2: return launch_large<T, 2, 0, 0, kBatch>(la, st);
-        case 3: return launch_large<T, 0, 0, 1, kBatch>(la, st);
-        case 4: return launch_large<T, 1, 1, 1, kBatch>(la, st);
-        case 5: return launch_large<T, 2, 0, 1, kBatch>(la, st);
-        case 6: return launch_large<T, 0, 0, 2, kBatch>(la, st);
-        case 7: return launch_large<T, 1, 1, 2, kBatch>(la, st);
-        case 8: return launch_large<T, 2, 0, 2, kBatch>(la, st);
+        case 0: return launch_large<T, 0, 0, 0, kBatch>(la, unit_slots, first, st);
+        case 1: return launch_large<T, 1, 1, 0, kBatch>(la, unit_slots, first, st);
+        case 2: return launch_large<T, 2, 0, 0, kBatch>(la, unit_slots, first, st);
+        case 3: return launch_large<T, 0, 0, 1, kBatch>(la, unit_slots, first, st);
+        case 4: return launch_large<T, 1, 1, 1, kBatch>(la, unit_slots, first, st);
+        case 5: return launch_large<T, 2, 0, 1, kBatch>(la, unit_slots, first, st);
+        case 6: return launch_large<T, 0, 0, 2, kBatch>(la, unit_slots, first, st);
+        case 7: return launch_large<T, 1, 1, 2, kBatch>(la, unit_slots, first, st);
+        case 8: return launch_large<T, 2, 0, 2, kBatch>(la, unit_slots, first, st);
     }
     set_error("Type %d does not exist for this implementation", type);
     return SNP_ERR_INVALID;
@@ -738,10 +878,11 @@ template <typename T, bool kBatch> int dispatch_large(int type, const LargeArgs<
 // One sub-step: `cur` = the view buffer read ([5][M] entities + their [n_tiles][5] tile boxes), `next` = the n_peers buffers the
 // finish kernel stores the updated entries into, and their tile boxes too when `fold_boxes`.  `boxes_ready`: `cur`'s tile boxes
 // were written by the previous sub-step's producers.  `sub`: index of the sub-step in the call (how far a moving robot has gone).
-// env_n > 0: the crowd is a batch of c->E envs of env_n = c->N humans (M = E N, self_offset 0, one next buffer).
+// units: the slots of the partial sums (SNP_OPT_UNIT_SCRATCH), or -1 for the default size.  env_n > 0: the crowd is a batch of c->E
+// envs of env_n = c->N humans (M = E N, self_offset 0, one next buffer).
 template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, const void *cur, const void *const *next, int n_peers,
                                     long long M, long long self_offset, bool fold_boxes, bool boxes_ready, void *scratch, int sub, cudaStream_t st,
-                                    long long env_n = 0) {
+                                    long long units, long long env_n = 0) {
     const bool batch = env_n > 0;
     LargeArgs<T> la;
     la.n_peers = n_peers;
@@ -764,11 +905,12 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     la.J = (int)large_J(batch ? env_n : M); la.n_tiles = (int)(batch ? c->E * large_tiles(env_n) : large_tiles(M));
     la.Jp = (la.J + 15) & ~15;
     const long long blocks = batch ? c->E * large_iblocks(env_n) : large_iblocks(a.EN);  // rows of the live map
-    const LargeScratch sc = large_scratch_units(a.EN, la.J, blocks, sizeof(T));
+    const long long partial_bytes = units < 0 ? (long long)sizeof(T) * la.J * 2 * a.EN : units * unit_bytes(sizeof(T));
+    const LargeScratch sc = large_scratch_regions(partial_bytes, la.J, blocks);
     char *base = (char *)scratch;
-    la.partial = (T *)base;
+    la.partial = (T *)(base + sc.partial);
     la.live = (unsigned char *)(base + sc.live);
-    la.work_counters = (int *)(base + sc.counters);
+    la.work_counters = (int *)base;
     la.work = (int *)(base + sc.work);
     la.live_cnt = (int *)(base + sc.live_cnt);
     la.live_list = (int *)(base + sc.live_list);
@@ -784,11 +926,14 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     // culled steps: one agent per thread (twice the units to hand out).  Round 2 kept two for fp32 on the static grid, where the
     // finer split only added CTAs to launch; on the work list one rank's slice of an 8-way split runs 0.0552 -> 0.0408 ms in fp32
     la.apt = margin >= 0.0 ? 1 : kMaxAgentsPerThread;  // fp32 pair evaluations are short: the finer split only adds launch overhead there
-    la.use_list = (margin >= 0.0 && self_offset % kTile == 0 && blocks * la.J < (1LL << 31)) ? 1 : 0;
+    la.use_list = large_uses_list(c, o, self_offset, blocks, la.J) ? 1 : 0;
+    // SNP_OPT_UNIT_SCRATCH: the slots the partial sums hold, at most one per unit (the default size keeps [J][2][N_local])
+    const long long cap = partial_bytes / unit_bytes(sizeof(T));
+    la.cap = la.use_list && units >= 0 ? (int)(cap < blocks * la.J ? cap : blocks * la.J) : 0;
     const long long per_block = (long long)kTile * la.apt;
     la.env_iblocks = (int)((env_n + per_block - 1) / per_block);
     la.env_fblocks = (int)large_iblocks(env_n);
-    return batch ? dispatch_large<T, true>(o->type, la, st) : dispatch_large<T, false>(o->type, la, st);
+    return batch ? dispatch_large<T, true>(o->type, la, units >= 0, sub == 0, st) : dispatch_large<T, false>(o->type, la, units >= 0, sub == 0, st);
 }
 
 // After the last sub-step of a call: the robot's end state (robot_mode 1 / 3; the finish kernels of the call read the start state
@@ -954,9 +1099,9 @@ template <typename T, bool kBatch> int launch_large_checks(const snp_crowd *cr, 
 
 // snp_large_batch_step after validation: publish, pre-checks, n_substeps x (robot step, tiled update) between the two view buffers of
 // the scratch, the robot's end state and the clock, post-checks.
-template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scratch, cudaStream_t st) {
+template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scratch, long long units, cudaStream_t st) {
     const long long E = c->E, N = c->N, EN = E * N;
-    const LargeBatchScratch sb = large_batch_scratch(E, N, sizeof(T));
+    const LargeBatchScratch sb = large_batch_scratch(E, N, sizeof(T), units);
     void *views[2] = {(char *)scratch + sb.view_a, (char *)scratch + sb.view_b};
     k_large_publish<T><<<(unsigned)((EN + 255) / 256), 256, 0, st>>>((const T *)c->dyn, (const T *)c->stat, EN, o->type >= 3, (T *)views[0], EN, 0);
     count_launch();
@@ -970,7 +1115,7 @@ template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_op
     const bool fold_boxes = N % kTile == 0;
     for (int s = 0; s < o->n_substeps; ++s) {
         const void *next[1] = {views[(s + 1) & 1]};
-        const int rc = run_large<T>(c, o, views[s & 1], next, 1, EN, 0, fold_boxes, fold_boxes && s > 0, scratch, s, st, N);
+        const int rc = run_large<T>(c, o, views[s & 1], next, 1, EN, 0, fold_boxes, fold_boxes && s > 0, scratch, s, st, units, N);
         if (rc) return rc;
     }
     if (o->n_substeps > 0 && ((c->robot && (o->robot_mode == 1 || o->robot_mode == 3)) || o->time_now)) {
@@ -992,6 +1137,24 @@ int64_t snp_large_scratch_bytes(int64_t n_local, int64_t M, int32_t dtype) {
     return large_scratch(n_local, M, dtype == SNP_F64 ? 8 : 4).bytes;
 }
 
+int64_t snp_large_scratch_bytes_units(int64_t n_local, int64_t M, int32_t dtype, int64_t units) {
+    if (n_local < 1 || M < n_local || units < 0 || (dtype != SNP_F64 && dtype != SNP_F32)) {
+        set_error("snp_large_scratch_bytes_units: n_local=%lld M=%lld dtype=%d units=%lld", (long long)n_local, (long long)M, dtype, (long long)units);
+        return -1;
+    }
+    return large_scratch(n_local, M, dtype == SNP_F64 ? 8 : 4, units).bytes;
+}
+
+// SNP_OPT_UNIT_SCRATCH: the refusals of a step whose partial sums are slots of the work list (`what` names the entry point), or SNP_OK.
+static int unit_scratch_refusals(const char *what, const snp_crowd *c, const snp_step_opts *o, long long self_offset, long long blocks, long long J) {
+    if (o->type % 3 == 2) { set_error("%s: SNP_OPT_UNIT_SCRATCH: Moussaid's pair law (type %d) is never culled and needs the default scratch", what, o->type); return SNP_ERR_UNSUPPORTED; }
+    if (o->reserved & SNP_OPT_NO_CULLING) { set_error("%s: SNP_OPT_UNIT_SCRATCH with SNP_OPT_NO_CULLING: every unit is evaluated, use the default scratch", what); return SNP_ERR_UNSUPPORTED; }
+    if (self_offset % kTile) { set_error("%s: SNP_OPT_UNIT_SCRATCH needs a slice starting on a 128-entity tile (self_offset %lld)", what, self_offset); return SNP_ERR_UNSUPPORTED; }
+    if (blocks * J >= (1LL << 31)) { set_error("%s: SNP_OPT_UNIT_SCRATCH: %lld units exceed the int32 unit index", what, blocks * J); return SNP_ERR_UNSUPPORTED; }
+    if (!large_uses_list(c, o, self_offset, blocks, J)) { set_error("%s: SNP_OPT_UNIT_SCRATCH: these pair-law parameters have no culling distance", what); return SNP_ERR_UNSUPPORTED; }
+    return SNP_OK;
+}
+
 int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *const *peer_views_a, const void *const *peer_views_b,
                       int32_t first_is_b, int64_t M, int64_t self_offset, int32_t world, int32_t rank, const void *const *peer_flags,
                       uint64_t epoch_base, int32_t n_substeps, int32_t *error_flag, void *scratch, int64_t scratch_bytes, void *stream) {
@@ -1011,7 +1174,14 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
     if (o->robot_mode && !o->action) { set_error("snp_large_run_p2p: robot_mode %d needs opts->action", o->robot_mode); return SNP_ERR_INVALID; }
     const long long N = (long long)c->E * c->N;
     if (self_offset < 0 || self_offset + N > M) { set_error("snp_large_run_p2p: M=%lld offset=%lld N=%lld", (long long)M, (long long)self_offset, N); return SNP_ERR_INVALID; }
-    const long long need = large_scratch(N, M, c->dtype == SNP_F64 ? 8 : 4).bytes;
+    const int w = c->dtype == SNP_F64 ? 8 : 4;
+    const bool unit_scratch = (o->reserved & SNP_OPT_UNIT_SCRATCH) != 0;
+    if (unit_scratch) {
+        const int rc = unit_scratch_refusals("snp_large_run_p2p", c, o, self_offset, large_iblocks(N), large_J(M));
+        if (rc) return rc;
+    }
+    const long long need = large_scratch(N, M, w, unit_scratch ? 0 : -1).bytes;  // with the bit: the size for no slot at all
+    const long long units = unit_scratch ? units_in(scratch_bytes, need, w) : -1;
     if (scratch_bytes < need || reinterpret_cast<uintptr_t>(scratch) % 16) {
         set_error("snp_large_run_p2p: 16-byte aligned scratch of %lld bytes needed, %lld given", need, (long long)scratch_bytes);
         return SNP_ERR_INVALID;
@@ -1027,8 +1197,8 @@ int snp_large_run_p2p(const snp_crowd *c, const snp_step_opts *o, const void *co
     for (int s = 0; s < n_substeps; ++s) {
         const void *const *cur = cur_is_b ? peer_views_b : peer_views_a, *const *nxt = cur_is_b ? peer_views_a : peer_views_b;
         const bool boxes_ready = fold_boxes && s > 0;  // sub-step 0 computes the tile boxes of the view it was handed
-        const int rc = c->dtype == SNP_F64 ? run_large<double>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st)
-                                           : run_large<float>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st);
+        const int rc = c->dtype == SNP_F64 ? run_large<double>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st, units)
+                                           : run_large<float>(c, o, cur[rank], nxt, world, M, self_offset, fold_boxes, boxes_ready, scratch, s, st, units);
         if (rc) return rc;
         if (world > 1) {
             b.epoch = epoch_base + (unsigned long long)s + 1;
@@ -1063,6 +1233,14 @@ int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype) {
     return large_batch_scratch(E, N, dtype == SNP_F64 ? 8 : 4).bytes;
 }
 
+int64_t snp_large_batch_scratch_bytes_units(int32_t E, int32_t N, int32_t dtype, int64_t units) {
+    if (E < 1 || N < 1 || units < 0 || (dtype != SNP_F64 && dtype != SNP_F32)) {
+        set_error("snp_large_batch_scratch_bytes_units: E=%d N=%d dtype=%d units=%lld", E, N, dtype, (long long)units);
+        return -1;
+    }
+    return large_batch_scratch(E, N, dtype == SNP_F64 ? 8 : 4, units).bytes;
+}
+
 int snp_large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scratch, int64_t scratch_bytes, void *stream) {
     if (!c || !o || !scratch) { set_error("snp_large_batch_step: null argument"); return SNP_ERR_INVALID; }
     if (c->E < 1 || c->N < 1 || c->G < 1) { set_error("snp_large_batch_step: E, N and G must be positive (E=%d N=%d G=%d)", c->E, c->N, c->G); return SNP_ERR_INVALID; }
@@ -1085,12 +1263,20 @@ int snp_large_batch_step(const snp_crowd *c, const snp_step_opts *o, void *scrat
     }
     if ((o->robot_mode || o->pre_checks) && !o->action) { set_error("snp_large_batch_step: robot_mode 1 / 3 and pre_checks need opts->action"); return SNP_ERR_INVALID; }
     if ((o->pre_checks || o->post_checks) && !o->flags) { set_error("snp_large_batch_step: the checks need opts->flags"); return SNP_ERR_INVALID; }
-    const long long need = large_batch_scratch(c->E, c->N, c->dtype == SNP_F64 ? 8 : 4).bytes;
+    const int w = c->dtype == SNP_F64 ? 8 : 4;
+    const bool unit_scratch = (o->reserved & SNP_OPT_UNIT_SCRATCH) != 0;
+    if (unit_scratch) {
+        const int rc = unit_scratch_refusals("snp_large_batch_step", c, o, 0, (long long)c->E * large_iblocks(c->N), large_J(c->N));
+        if (rc) return rc;
+    }
+    const long long need = large_batch_scratch(c->E, c->N, w, unit_scratch ? 0 : -1).bytes;  // with the bit: the size for no slot at all
     if (scratch_bytes < need || reinterpret_cast<uintptr_t>(scratch) % 16) {
         set_error("snp_large_batch_step: 16-byte aligned scratch of %lld bytes needed, %lld given", need, (long long)scratch_bytes);
         return SNP_ERR_INVALID;
     }
-    return c->dtype == SNP_F64 ? large_batch_step<double>(c, o, scratch, (cudaStream_t)stream) : large_batch_step<float>(c, o, scratch, (cudaStream_t)stream);
+    const long long units = unit_scratch ? units_in(scratch_bytes, need, w) : -1;
+    return c->dtype == SNP_F64 ? large_batch_step<double>(c, o, scratch, units, (cudaStream_t)stream)
+                               : large_batch_step<float>(c, o, scratch, units, (cudaStream_t)stream);
 }
 
 int snp_large_publish(const snp_crowd *c, int32_t type, void *view, int64_t stride, int64_t offset, void *stream) {

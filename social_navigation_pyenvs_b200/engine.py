@@ -99,10 +99,11 @@ class CrowdEngine:
     @classmethod
     def from_reference_arrays(cls, model, states, goals, walls=None, params=None, safety=None, consider_robot=False,
                               all_params_equal=True, numba_compat=False, dtype=torch.float64, device="cuda", robot=None,
-                              full_pair_loop=False):
+                              full_pair_loop=False, **engine_kw):
         """states [E,rows,13] float64 rows (agent.py:256; rows = N + consider_robot), goals [E,N,G,2] NaN padded,
         walls [W,S,2,2] or [E,W,S,2,2] NaN padded, params [20] / [E,N,20], safety [E,rows], robot [E,13] (when the robot is
-        not a row of `states` but checks are wanted)."""
+        not a row of `states` but checks are wanted).  Further keywords go to the constructor (e.g. TiledCrowdEngine's
+        unit_capacity)."""
         states = np.ascontiguousarray(states, np.float64)
         goals = np.ascontiguousarray(goals, np.float64)
         E, rows, _ = states.shape
@@ -122,7 +123,7 @@ class CrowdEngine:
                     p_rows = params.reshape(E, N, 20)
         eng = cls(model, E, N, G, dtype=dtype, device=device, consider_robot=consider_robot, symmetric=all_params_equal,
                   numba_compat=numba_compat, params=p_uniform, walls=walls, has_robot=consider_robot or robot is not None,
-                  full_pair_loop=full_pair_loop)
+                  full_pair_loop=full_pair_loop, **engine_kw)
         if p_rows is not None:
             eng.agent_params = torch.as_tensor(np.ascontiguousarray(p_rows.transpose(2, 0, 1)), dtype=dtype, device=eng.device)
         eng.load_rows(states, safety)

@@ -24,15 +24,84 @@ from . import _lib as L
 from .engine import CrowdEngine, SFMS
 from .parallel import all_gather_columns, agent_shard
 
+# unit_capacity="auto" starts with this many partial-sum slots per 128-agent block (DESIGN 4.3: what the bench crowd lists)
+AUTO_UNITS_PER_BLOCK = 32
 
-class LargeCrowd:
+
+class _UnitSlots:
+    """The scratch of the tiled path, with the partial sums of a culled step sized for `unit_capacity` (agent block, entity chunk)
+    units in reach (SNP_OPT_UNIT_SCRATCH) instead of one per chunk and agent.  None: the default size.  An int: that many slots.
+    "auto": min(all units, AUTO_UNITS_PER_BLOCK per agent block) to start with; after a call that listed more units than that, the
+    next call gets ceil(1.25 x the most listed) -- which costs one device synchronisation per call to read the count.  Units without
+    a slot are evaluated by the finish kernel: the results are the same bits whatever the capacity, only slower."""
+
+    def _setup_units(self, unit_capacity, blocks, J, size_of, device):
+        self._units_all, self._size_of, self._units_device = blocks * J, size_of, device
+        self._auto = isinstance(unit_capacity, str)
+        if unit_capacity is None:
+            cap = None
+        elif self._auto:
+            if unit_capacity != "auto":
+                raise ValueError(f"unit_capacity must be None, an int >= 0 or 'auto' (got {unit_capacity!r})")
+            cap = min(self._units_all, AUTO_UNITS_PER_BLOCK * blocks)
+        else:
+            cap = int(unit_capacity)
+            if cap < 0 or cap != unit_capacity or isinstance(unit_capacity, bool):
+                raise ValueError(f"unit_capacity must be None, an int >= 0 or 'auto' (got {unit_capacity!r})")
+        self._stats = torch.zeros((2,), dtype=torch.int32, device=device)  # the last call's (most units listed, units without a slot)
+        self._stats_valid, self._last_capacity = False, cap
+        self._alloc_units(cap)
+
+    def _alloc_units(self, cap):
+        self.unit_capacity = cap
+        self.scratch = None  # release the old scratch before the new one is allocated
+        self.scratch = torch.empty(int(self._size_of(cap)), dtype=torch.uint8, device=self._units_device)
+
+    def _unit_bits(self):
+        return 0 if self.unit_capacity is None else L.SNP_OPT_UNIT_SCRATCH
+
+    def _collect_units(self, first):
+        """After a C call with a capacity: its unit counts (int32 words 1 and 2 of the scratch) into the step's, on the stream."""
+        if self.unit_capacity is None:  # the default size keeps no counts
+            return
+        w = self.scratch[:12].view(torch.int32)[1:3]
+        if first:
+            self._stats.copy_(w)
+        else:
+            torch.maximum(self._stats[0:1], w[0:1], out=self._stats[0:1])
+            self._stats[1:2] += w[1:2]
+
+    def _end_units(self):
+        """After a step: the counts exist when it had a capacity (a step with one that does not take the work list is refused
+        before any launch).  "auto" grows for the next step."""
+        listed = self.unit_capacity is not None
+        self._stats_valid, self._last_capacity = listed, self.unit_capacity
+        if self._auto and listed:
+            most = int(self._stats[0].item())  # the synchronisation "auto" costs
+            if most > self.unit_capacity:
+                self._alloc_units(min(self._units_all, -(-5 * most // 4)))
+
+    def unit_stats(self):
+        """The last step's {capacity, max_listed, fallback_units}: the partial-sum slots it had (None: the default size), the most
+        (agent block, entity chunk) units listed in one of its sub-steps and the units the finish kernel evaluated for want of a slot.
+        The counts are kept only with a capacity: None at the default size."""
+        most, fallback = (int(v) for v in self._stats.tolist()) if self._stats_valid else (None, None)
+        return {"capacity": self._last_capacity, "max_listed": most, "fallback_units": fallback}
+
+
+class LargeCrowd(_UnitSlots):
     def __init__(self, model, states, goals, walls=None, dtype=torch.float64, device="cuda", symmetric=True, numba_compat=False,
-                 rank=0, world=1, group=None, safety=None, exchange="auto", shard=None, robot=None, robot_safety=None, consider_robot=False):
+                 rank=0, world=1, group=None, safety=None, exchange="auto", shard=None, robot=None, robot_safety=None, consider_robot=False,
+                 unit_capacity=None):
         """states [N_total,13], goals [N_total,G,2] (the WHOLE crowd on every rank; each rank keeps its slice).
         shard=(offset, n_local) with world=1 steps only that slice against a frozen rest of the crowd (profiling what ONE rank of
         a sharded run executes, on one GPU).
         robot: the robot's 13-wide reference row (robot.get_safe_state(), as CrowdEngine.set_robot_rows), robot_safety its safety
-        space (default 0); consider_robot: the humans feel its force (motion_model_manager.py:35)."""
+        space (default 0); consider_robot: the humans feel its force (motion_model_manager.py:35).
+        unit_capacity: None, an int or "auto" -- the partial-sum slots of the scratch (_UnitSlots; unit_stats()).  The default size
+        holds n_local * n_total / 16 bytes of partial sums in fp64; a capacity near what a step lists lets crowds of millions of
+        humans fit on one GPU.  With a capacity, Moussaid models, culling = False and a slice that does not start on a 128-human
+        tile raise NotImplementedError at the step."""
         states = np.asarray(states, np.float64)
         goals = np.asarray(goals, np.float64)
         self.n_total = states.shape[0]
@@ -91,8 +160,10 @@ class LargeCrowd:
         self.view = [v[:5 * self.n_total].view(5, self.n_total) for v in self._vbuf]
         self._epoch = 0
         self._err = torch.zeros((1,), dtype=torch.int32, device=self.eng.device)
-        nbytes = int(self.eng.lib.snp_large_scratch_bytes(self.n_local, self.n_total, L.SNP_F64 if dtype == torch.float64 else L.SNP_F32))
-        self.scratch = torch.empty(nbytes, dtype=torch.uint8, device=self.eng.device)
+        dt, lib = (L.SNP_F64 if dtype == torch.float64 else L.SNP_F32), self.eng.lib
+        size_of = lambda units: (lib.snp_large_scratch_bytes(self.n_local, self.n_total, dt) if units is None else
+                                 L.check_size(lib.snp_large_scratch_bytes_units(self.n_local, self.n_total, dt, units)))
+        self._setup_units(unit_capacity, -(-self.n_local // 128), -(-self.n_total // 128), size_of, self.eng.device)
         self.culling = True
         self.cur = 0
         if shard is not None:  # the frozen rest of the crowd: both view buffers start from the whole crowd's entries
@@ -142,20 +213,23 @@ class LargeCrowd:
             self._checks(dt, mode, pre=True)
         c = self.eng._crowd()
         o = self.eng._opts(dt, 1, robot_mode=mode, advance_time=self.has_robot)
-        o.reserved = 0 if self.culling else L.SNP_OPT_NO_CULLING
+        o.reserved = (0 if self.culling else L.SNP_OPT_NO_CULLING) | self._unit_bits()
         # p2p / fused: the whole sub-step loop in ONE C call, nothing returns to Python in between; nccl: one sub-step per call on
         # this rank's own buffers, then the all-gather of the next view
         nccl = self.exchange == "nccl"
         world, rank, calls, k = (1, 0, n_substeps, 1) if nccl else (self.world, self.rank, 1, int(n_substeps))
-        for _ in range(calls):
+        for call in range(calls):
             L.check(self.eng.lib.snp_large_run_p2p(ctypes.byref(c), ctypes.byref(o), self._peer_ptrs[0], self._peer_ptrs[1], self.cur, self.n_total,
                                                    self.offset, world, rank, self._peer_flags, self._epoch, k,
                                                    ctypes.c_void_p(self._err.data_ptr()), ctypes.c_void_p(self.scratch.data_ptr()),
                                                    self.scratch.numel(), self._stream()))
+            self._collect_units(first=call == 0)
             self._epoch += k
             self.cur ^= k & 1
             if nccl:
                 self._gather(self.view[self.cur])
+        if n_substeps > 0:
+            self._end_units()
         if post_checks:
             self._checks(dt, mode, pre=False)
 
@@ -201,25 +275,31 @@ class LargeCrowd:
         return self.eng.rows(np.asarray(template, np.float64)[None])[0]
 
 
-class TiledCrowdEngine(CrowdEngine):
+class TiledCrowdEngine(_UnitSlots, CrowdEngine):
     """CrowdEngine for E environments of any number of humans each, N > 512 included: `update_humans` and `step` run
     snp_large_batch_step (the tiled kernels of LargeCrowd with an environment axis) in one call per step.  Environment e steps
     bit for bit as a LargeCrowd built from environment e alone.  Loading and reading are CrowdEngine's (from_reference_arrays,
     rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env).  Per-agent parameter rows, respawn
     and the snp_step features the tiled path does not have (peek and the lookahead through it, imitation_learning_step, sim_update,
     step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
-    carried from one step to the next.  culling=False evaluates every pair (the same result)."""
+    carried from one step to the next.  culling=False evaluates every pair (the same result).  unit_capacity (a constructor and
+    from_reference_arrays keyword): None, an int or "auto", as for LargeCrowd (_UnitSlots; unit_stats())."""
 
-    def __init__(self, *args, **kwargs):
+    def __init__(self, *args, unit_capacity=None, **kwargs):
         super().__init__(*args, **kwargs)
-        dt = L.SNP_F64 if self.dtype == torch.float64 else L.SNP_F32
-        self.scratch = torch.empty(int(self.lib.snp_large_batch_scratch_bytes(self.E, self.N, dt)), dtype=torch.uint8, device=self.device)
+        dt, lib, E, N = (L.SNP_F64 if self.dtype == torch.float64 else L.SNP_F32), self.lib, self.E, self.N
+        size_of = lambda units: (lib.snp_large_batch_scratch_bytes(E, N, dt) if units is None else
+                                 L.check_size(lib.snp_large_batch_scratch_bytes_units(E, N, dt, units)))
+        self._setup_units(unit_capacity, E * -(-N // 128), -(-N // 128), size_of, self.device)
         self.culling = True
 
     def _run(self, o):
-        o.reserved = 0 if self.culling else L.SNP_OPT_NO_CULLING
+        o.reserved = (0 if self.culling else L.SNP_OPT_NO_CULLING) | self._unit_bits()
         L.check(self.lib.snp_large_batch_step(ctypes.byref(self._crowd()), ctypes.byref(o), ctypes.c_void_p(self.scratch.data_ptr()),
                                               self.scratch.numel(), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+        if o.n_substeps > 0:
+            self._collect_units(first=True)
+            self._end_units()
 
     def update_humans(self, t=0.0, dt=0.0125, post_update=True, n_substeps=1):
         """MotionModelManager.update_humans (motion_model_manager.py:354) for every env: `n_substeps` Euler updates in one call."""
