@@ -37,8 +37,6 @@
 // humans and no gain from a second GPU; 512: 2.0 / 1.1 ms; 256 + exact culling on compact tiles + one agent per thread: 0.75 ms on
 // one GPU, 0.158 on eight; 128 + the work list + grouped evaluation: 0.59 / 0.125).  The price is J = M/128 partial sums per LIVE chunk and agent.
 // Reference: same as snp_step_small.cu (motion_model_manager.py:354-373,424-459; forces.py:63-151).
-#include <type_traits>
-
 #include "snp_gym.cuh"
 
 namespace snp {
@@ -378,7 +376,7 @@ __global__ void __launch_bounds__(kTile) k_large_pairs(const LargeArgs<T> la) {
 // where the grid version puts them: results are bit-identical.
 // kSlots (SNP_OPT_UNIT_SCRATCH): the i-block's list holds each unit's slot of the partial sums (its index on the work list), or
 // -1 - chunk when the index is beyond the slots; otherwise the chunk.
-template <typename T, bool kBatch, bool kSlots = false> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
+template <typename T, bool kBatch, bool kSlots> __global__ void __launch_bounds__(256) k_large_cull(const LargeArgs<T> la) {
     __shared__ int warp_cnt[8];
     T u[5];
     iblock_box<T, kBatch>(la, blockIdx.x, la.apt, u);
@@ -418,7 +416,7 @@ template <typename T, bool kBatch, bool kSlots = false> __global__ void __launch
 }
 
 // kSlots (SNP_OPT_UNIT_SCRATCH): entry k writes slot k of the partial sums, and entries beyond the slots are left to the finish kernel.
-template <typename T, int SOC, int kAgentsPerThread, bool kBatch, bool kSlots = false>
+template <typename T, int SOC, int kAgentsPerThread, bool kBatch, bool kSlots>
 __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> la, const int n_queues) {
     __shared__ PairsSmem<T> sm;
     bool have_tbl = false;
@@ -438,8 +436,7 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
         const int item = sm.item;
         if (item >= 0) {
             const int w = la.work[item];
-            if constexpr (kSlots) pairs_chunk<T, SOC, kAgentsPerThread, kBatch, kToSlot>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, w / la.J, w % la.J, have_tbl, item);
-            else pairs_chunk<T, SOC, kAgentsPerThread, kBatch>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, w / la.J, w % la.J, have_tbl);
+            pairs_chunk<T, SOC, kAgentsPerThread, kBatch, kSlots ? kToSlot : kToGrid>(la, sm.tile_raw, sm.tile_rs, sm.exp_tbl_s, sm.sbox, w / la.J, w % la.J, have_tbl, item);
             continue;
         }
         // this queue is empty (and stays so: the counters only grow): move to the nearest queue that still has entries, if any
@@ -475,11 +472,12 @@ template <typename T, bool kBatch> __device__ __forceinline__ void large_robot_r
 }
 
 // The sum of the partial sums on i-block `row`'s ascending list (the order is what makes the result independent of the sharding and
-// of which units had a slot), this thread's agent = lane of the slots.  Sixteen entries per step, the next sixteen already on their
-// way while the partial sums of the current ones are loaded.  FSOC >= 0 (the CTA is the whole i-block, every thread present): an
-// entry -1 - chunk had no slot, and the chunk is evaluated here with the pairs kernel's code, in its place in the order.
+// of which units had a slot), added to fsx, fsy.  Sixteen entries per step, the next sixteen already on their way while the partial
+// sums of the current ones are loaded.  FSOC < 0: the entries are chunks of the [J][2][N_local] sums, agent i.  FSOC >= 0 (the CTA
+// is the whole i-block, every thread present): the entries are slots of the [cap][2][128] sums, agent = lane; an entry -1 - chunk
+// had no slot, and the chunk is evaluated here with the pairs kernel's code, in its place in the order.
 template <typename T, int FSOC, bool kBatch>
-__device__ __forceinline__ void sum_listed(const LargeArgs<T> &la, long long row, T &fsx, T &fsy, double *exp_tbl_s, TileSmem<T> *ts) {
+__device__ __forceinline__ void sum_listed(const LargeArgs<T> &la, long long row, long long n, long long lane, T &fsx, T &fsy, double *exp_tbl_s, TileSmem<T> *ts) {
     const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)row * la.Jp);
     const int cnt = la.live_cnt[row];
     int4 nxt[4];
@@ -505,7 +503,7 @@ __device__ __forceinline__ void sum_listed(const LargeArgs<T> &la, long long row
                     const int s = la.live_list[(size_t)row * la.Jp + b];
                     T vx, vy;
                     if (s >= 0) {
-                        vx = la.partial[((size_t)s * 2 + 0) * kTile + threadIdx.x]; vy = la.partial[((size_t)s * 2 + 1) * kTile + threadIdx.x];
+                        vx = la.partial[((size_t)s * 2 + 0) * n + lane]; vy = la.partial[((size_t)s * 2 + 1) * n + lane];
                     } else {
                         bool have_tbl = true;  // staged by the caller
                         pairs_chunk<T, FSOC, 1, kBatch, kToCaller>(la, ts->tile_raw, ts->tile_rs, exp_tbl_s, ts->sbox, (int)row, -1 - s, have_tbl, 0, &vx, &vy);
@@ -519,7 +517,7 @@ __device__ __forceinline__ void sum_listed(const LargeArgs<T> &la, long long row
         T vx[16], vy[16];
 #pragma unroll
         for (int b = 0; b < 16; ++b)
-            if (k + b < cnt) { vx[b] = la.partial[((size_t)idx[b] * 2 + 0) * kTile + threadIdx.x]; vy[b] = la.partial[((size_t)idx[b] * 2 + 1) * kTile + threadIdx.x]; }
+            if (k + b < cnt) { vx[b] = la.partial[((size_t)idx[b] * 2 + 0) * n + lane]; vy[b] = la.partial[((size_t)idx[b] * 2 + 1) * n + lane]; }
 #pragma unroll
         for (int b = 0; b < 16; ++b)
             if (k + b < cnt) { fsx += vx[b]; fsy += vy[b]; }
@@ -579,7 +577,7 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     [[maybe_unused]] T listed_x = T(0), listed_y = T(0);
     if constexpr (FSOC >= 0) {  // before any thread leaves: the units without a slot are evaluated by the whole CTA (= the i-block)
         const size_t seg_end = kTbl + ((sizeof(Seg<T>) * (size_t)nseg + 15) & ~size_t(15)) + ((sizeof(int) * (size_t)(a.W + 1) + 15) & ~size_t(15));
-        sum_listed<T, FSOC, kBatch>(la, blockIdx.x, listed_x, listed_y, exp_tbl_s, reinterpret_cast<TileSmem<T> *>(smem_raw + seg_end));
+        sum_listed<T, FSOC, kBatch>(la, blockIdx.x, kTile, threadIdx.x, listed_x, listed_y, exp_tbl_s, reinterpret_cast<TileSmem<T> *>(smem_raw + seg_end));
     }
     const bool fold_boxes = la.peer_boxes[0] != nullptr;  // uniform; only offered when N is a whole number of tiles, so that every
     if (gone) return;                                      // thread of every block reaches the box reduction at the end
@@ -605,39 +603,14 @@ __global__ void __launch_bounds__(kTile) k_large_finish(const LargeArgs<T> la) {
     T fsx = T(0), fsy = T(0);
     if constexpr (FSOC >= 0) { fsx = listed_x; fsy = listed_y; }
     // Sum of the live chunks' partial sums in ascending chunk order (the order is what makes the result independent of the
-    // sharding).  The flags are the same for the whole CTA and live chunks come in runs; they are read 64 at a time, and for every
-    // 16 flags with a live one the loads of all live partial sums are issued together before the (ordered) additions -- a
-    // flag-by-flag loop serialised one L2 round trip per live chunk.
+    // sharding).  On the work list the cull kernel left them as the i-block's ascending list.  On the static grid the flags are the
+    // same for the whole CTA and live chunks come in runs; they are read 64 at a time, and for every 16 flags with a live one the
+    // loads of all live partial sums are issued together before the (ordered) additions -- a flag-by-flag loop serialised one L2
+    // round trip per live chunk.
     const long long row = kBatch ? (long long)env * la.env_iblocks + r / (kTile * la.apt) : i / (kTile * la.apt);  // the agent's i-block
     const uint4 *lv = reinterpret_cast<const uint4 *>(la.live + (size_t)row * la.Jp);
     const int n_words = la.use_list ? 0 : la.Jp >> 4;
-    if (FSOC < 0 && la.use_list) {
-        // the cull kernel left the i-block's live chunks as an ascending list: sixteen indices per step, the next sixteen already on
-        // their way while the partial sums of the current ones are loaded
-        const int4 *ll = reinterpret_cast<const int4 *>(la.live_list + (size_t)row * la.Jp);
-        const int cnt = la.live_cnt[row];
-        int4 nxt[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) nxt[u] = ll[u];  // (a row is Jp >= 16 entries long; entries beyond cnt are ignored)
-        for (int k = 0; k < cnt; k += 16) {
-            int4 cur[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) cur[u] = nxt[u];
-            if (k + 16 < cnt) {
-#pragma unroll
-                for (int u = 0; u < 4; ++u) nxt[u] = ll[(k >> 2) + 4 + u];
-            }
-            const int idx[16] = {cur[0].x, cur[0].y, cur[0].z, cur[0].w, cur[1].x, cur[1].y, cur[1].z, cur[1].w,
-                                 cur[2].x, cur[2].y, cur[2].z, cur[2].w, cur[3].x, cur[3].y, cur[3].z, cur[3].w};
-            T vx[16], vy[16];
-#pragma unroll
-            for (int b = 0; b < 16; ++b)
-                if (k + b < cnt) { vx[b] = la.partial[((size_t)idx[b] * 2 + 0) * N + i]; vy[b] = la.partial[((size_t)idx[b] * 2 + 1) * N + i]; }
-#pragma unroll
-            for (int b = 0; b < 16; ++b)
-                if (k + b < cnt) { fsx += vx[b]; fsy += vy[b]; }
-        }
-    }
+    if (FSOC < 0 && la.use_list) sum_listed<T, FSOC, kBatch>(la, row, N, i, fsx, fsy, exp_tbl_s, nullptr);
     for (int w0 = 0; w0 < n_words; w0 += 4) {
         uint4 f[4];
 #pragma unroll
@@ -767,24 +740,18 @@ template <typename T, int SOC, int OBS, int HEADED, bool kBatch> int launch_larg
     dim3 grid((unsigned)(kBatch ? (long long)la.k.E * la.env_iblocks : (N + per_block - 1) / per_block), (unsigned)la.J);
     if constexpr (SOC == 2) {  // Moussaid's pair law has no culling distance (run_large): every pair, two agents per thread
         k_large_pairs<T, SOC, kMaxAgentsPerThread, kBatch><<<grid, kTile, 0, st>>>(la);
-    } else if (la.use_list && unit_slots) {  // (culled, partial sums in slots)
-        // the counters start empty: zeroed here on the call's first sub-step (the call's unit counts too), else by the previous
-        // sub-step's finish kernel
-        if (first) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
-        k_large_cull<T, kBatch, true><<<grid.x, 256, 0, st>>>(la);
-        static int slots = 0;  // resident CTAs per SM
-        const int n_queues = device_sm_count() < kMaxQueues ? device_sm_count() : kMaxQueues;
-        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1, kBatch, true>, kTile, 0));
-        k_large_pairs_list<T, SOC, 1, kBatch, true><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
-        count_launch();
     } else if (la.use_list) {  // (culled: one agent per thread)
-        // the counters start empty: zeroed here on a sub-step that computes the tile boxes, else by the previous sub-step's finish kernel
-        if (!la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
-        k_large_cull<T, kBatch><<<grid.x, 256, 0, st>>>(la);
-        static int slots = 0;  // resident CTAs per SM
+        // the counters start empty: zeroed here, else by the previous sub-step's finish kernel.  With slots on the call's first
+        // sub-step (the call's unit counts too), without on a sub-step that computes the tile boxes.
+        if (unit_slots ? first : !la.boxes_ready) SNP_CUDA_OK(cudaMemsetAsync(la.work_counters, 0, kWorkCounters * sizeof(int), st));
+        const auto cull = unit_slots ? k_large_cull<T, kBatch, true> : k_large_cull<T, kBatch, false>;
+        const auto pairs = unit_slots ? k_large_pairs_list<T, SOC, 1, kBatch, true> : k_large_pairs_list<T, SOC, 1, kBatch, false>;
+        cull<<<grid.x, 256, 0, st>>>(la);
+        static int slots[2] = {0, 0};  // resident CTAs per SM of each pairs kernel
+        int &sl = slots[unit_slots ? 1 : 0];
         const int n_queues = device_sm_count() < kMaxQueues ? device_sm_count() : kMaxQueues;
-        if (!slots) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slots, k_large_pairs_list<T, SOC, 1, kBatch>, kTile, 0));
-        k_large_pairs_list<T, SOC, 1, kBatch><<<(unsigned)(device_sm_count() * (slots > 0 ? slots : 1)), kTile, 0, st>>>(la, n_queues);
+        if (!sl) SNP_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sl, pairs, kTile, 0));
+        pairs<<<(unsigned)(device_sm_count() * (sl > 0 ? sl : 1)), kTile, 0, st>>>(la, n_queues);
         count_launch();
     } else if (la.apt == 1) k_large_pairs<T, SOC, 1, kBatch><<<grid, kTile, 0, st>>>(la);
     else k_large_pairs<T, SOC, 2, kBatch><<<grid, kTile, 0, st>>>(la);
@@ -977,22 +944,16 @@ template <typename T, bool kBatch> int launch_large_robot_end(const snp_crowd *c
 // it, the first of equal minima kept ('<'), NaN distances never taken.
 constexpr int kCheckThreads = 1024;
 
+// E envs of M humans (one crowd: E = 1), view [5][stride = E M], radius [E M]; clear: start from zero flags and checks.
 template <typename T> struct CheckArgs {
     const T *robot, *action, *view, *radius;
-    long long M;
-    int mode, pre, post;
+    long long M, stride;
+    int E, mode, pre, post, clear;
     double consts[6];
     const double *time_now;
     int *flags;
     double *checks;
 };
-// A batch (kBatch): E envs of M humans, view [5][stride = E M], radius [E M]; clear: start from zero flags and checks.  A type of its
-// own, so that the one-crowd kernel's parameters (and registers) stay as they are.
-template <typename T> struct CheckBatchArgs : CheckArgs<T> {
-    int E, clear;
-    long long stride;
-};
-template <typename T, bool kBatch> using CheckArgsOf = std::conditional_t<kBatch, CheckBatchArgs<T>, CheckArgs<T>>;
 
 // (dmin, hit) of a run on the left combined with the run on its right
 __device__ __forceinline__ void swept_combine(double &dmin, int &hit, double dmin_r, int hit_r) {
@@ -1001,13 +962,12 @@ __device__ __forceinline__ void swept_combine(double &dmin, int &hit, double dmi
     hit = hit_r;
 }
 
-// kBatch: one CTA per env (blockIdx.x = env).
-template <typename T, bool kBatch> __global__ void __launch_bounds__(kCheckThreads) k_large_checks(const CheckArgsOf<T, kBatch> c) {
+// One CTA per env (blockIdx.x = env).
+template <typename T> __global__ void __launch_bounds__(kCheckThreads) k_large_checks(const CheckArgs<T> c) {
     __shared__ double s_dmin[kCheckThreads / 32], s_admin[kCheckThreads / 32];
     __shared__ int s_hit[kCheckThreads / 32];
-    int env = 0;
-    long long RE = 1, stride = c.M;
-    if constexpr (kBatch) { env = blockIdx.x; RE = c.E; stride = c.stride; }
+    const int env = blockIdx.x;
+    const long long RE = c.E, stride = c.stride;
     const T *rbt = c.robot + env;
     const T rpx = rbt[SNP_ROBOT_PX * RE], rpy = rbt[SNP_ROBOT_PY * RE], rr = rbt[SNP_ROBOT_R * RE], rgx = rbt[SNP_ROBOT_GX * RE], rgy = rbt[SNP_ROBOT_GY * RE];
     T ax = T(0), ay = T(0);
@@ -1053,11 +1013,9 @@ template <typename T, bool kBatch> __global__ void __launch_bounds__(kCheckThrea
     int *flags = c.flags + env;
     double *checks = c.checks ? c.checks + 4 * env : nullptr;
     int f = *flags;
-    if constexpr (kBatch) {
-        if (c.clear) {
-            f = 0;
-            if (checks) checks[0] = checks[1] = checks[2] = checks[3] = 0.0;
-        }
+    if (c.clear) {
+        f = 0;
+        if (checks) checks[0] = checks[1] = checks[2] = checks[3] = 0.0;
     }
     if (c.pre) {
         const double endx = __dadd_rn((double)rpx, __dmul_rn((double)ax, c.consts[5]));
@@ -1081,17 +1039,16 @@ template <typename T, bool kBatch> __global__ void __launch_bounds__(kCheckThrea
     *flags = f;
 }
 
-// kBatch: E = cr->E envs of M humans each, the checks selected by pre / post; `clear` zeroes each env's flags and checks first.
-template <typename T, bool kBatch> int launch_large_checks(const snp_crowd *cr, const snp_step_opts *o, const void *view, const void *radius, long long M,
-                                                           cudaStream_t st, bool pre = true, bool post = true, bool clear = false) {
-    CheckArgsOf<T, kBatch> c;
-    c.robot = (const T *)cr->robot; c.action = (const T *)o->action; c.view = (const T *)view; c.radius = (const T *)radius; c.M = M;
+// E envs of M humans each, the checks selected by pre / post; `clear` zeroes each env's flags and checks first.
+template <typename T> int launch_large_checks(const snp_crowd *cr, const snp_step_opts *o, const void *view, const void *radius, int E, long long M,
+                                              cudaStream_t st, bool pre = true, bool post = true, bool clear = false) {
+    CheckArgs<T> c;
+    c.robot = (const T *)cr->robot; c.action = (const T *)o->action; c.view = (const T *)view; c.radius = (const T *)radius;
+    c.M = M; c.stride = (long long)E * M; c.E = E; c.clear = clear;
     c.mode = o->robot_mode; c.pre = pre && o->pre_checks != 0; c.post = post && o->post_checks != 0;
-    unsigned n_ctas = 1;
-    if constexpr (kBatch) { c.E = cr->E; c.clear = clear; c.stride = (long long)cr->E * M; n_ctas = (unsigned)cr->E; }
     for (int k = 0; k < 6; ++k) c.consts[k] = o->consts[k];
     c.time_now = o->time_now; c.flags = o->flags; c.checks = o->checks;
-    k_large_checks<T, kBatch><<<n_ctas, kCheckThreads, 0, st>>>(c);
+    k_large_checks<T><<<(unsigned)E, kCheckThreads, 0, st>>>(c);
     count_launch();
     SNP_CUDA_OK(cudaGetLastError());
     return SNP_OK;
@@ -1108,7 +1065,7 @@ template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_op
     SNP_CUDA_OK(cudaGetLastError());
     const T *radius = (const T *)c->stat + SNP_STAT_R * EN;
     if (o->pre_checks) {
-        const int rc = launch_large_checks<T, true>(c, o, views[0], radius, N, st, true, false, true);
+        const int rc = launch_large_checks<T>(c, o, views[0], radius, c->E, N, st, true, false, true);
         if (rc) return rc;
     }
     // the finish kernel writes the next view's tile boxes when its CTAs are whole tiles (LargeCrowd's rule)
@@ -1122,7 +1079,7 @@ template <typename T> int large_batch_step(const snp_crowd *c, const snp_step_op
         const int rc = launch_large_robot_end<T, true>(c, o, o->n_substeps, st);
         if (rc) return rc;
     }
-    if (o->post_checks) return launch_large_checks<T, true>(c, o, views[o->n_substeps & 1], radius, N, st, false, true, !o->pre_checks);
+    if (o->post_checks) return launch_large_checks<T>(c, o, views[o->n_substeps & 1], radius, c->E, N, st, false, true, !o->pre_checks);
     return SNP_OK;
 }
 
@@ -1224,8 +1181,8 @@ int snp_large_checks(const snp_crowd *c, const snp_step_opts *o, const void *vie
     if (o->robot_mode != 0 && o->robot_mode != 1 && o->robot_mode != 3) { set_error("snp_large_checks: robot_mode must be 0, 1 or 3 (got %d)", o->robot_mode); return SNP_ERR_INVALID; }
     if (o->pre_checks && !o->action) { set_error("snp_large_checks: pre_checks needs opts->action"); return SNP_ERR_INVALID; }
     if (!o->flags) { set_error("snp_large_checks: opts->flags is required"); return SNP_ERR_INVALID; }
-    return c->dtype == SNP_F64 ? launch_large_checks<double, false>(c, o, view, radius, M, (cudaStream_t)stream)
-                               : launch_large_checks<float, false>(c, o, view, radius, M, (cudaStream_t)stream);
+    return c->dtype == SNP_F64 ? launch_large_checks<double>(c, o, view, radius, 1, M, (cudaStream_t)stream)
+                               : launch_large_checks<float>(c, o, view, radius, 1, M, (cudaStream_t)stream);
 }
 
 int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype) {
