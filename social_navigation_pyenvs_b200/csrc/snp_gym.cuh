@@ -1,5 +1,5 @@
 // snp_gym.cuh -- pieces of SocialNavGym.step shared by the small-crowd kernel (snp_step_small.inl) and the large-crowd path
-// (snp_step_large.cu): the reward / info code of a check, and the robot's unicycle step.
+// (snp_step_large.cu): the reward / info code of a check, and the robot's holonomic and unicycle steps.
 #pragma once
 #include "snp_kernels.cuh"
 
@@ -15,6 +15,12 @@ __device__ __forceinline__ int reward_and_info(bool collision, double dmin, bool
     if (goal) { reward = c[2]; truncated = false; terminated = true; return 3; }
     if (dmin < c[3]) { reward = __dmul_rn(__dmul_rn(__dsub_rn(dmin, c[3]), c[4]), c[5]); truncated = false; terminated = false; return 4; }
     reward = 0.0; truncated = false; terminated = false; return 0;
+}
+
+// RobotAgent.step with holonomic kinematics (robot_agent.py:126-131), one coordinate: p = p + a dt (the velocity becomes a).
+template <typename T> __device__ __forceinline__ T robot_holonomic_step(T p, T a, T dt) {
+    if (sizeof(T) == 8) return (T)__dadd_rn((double)p, __dmul_rn((double)a, (double)dt));
+    return p + a * dt;
 }
 
 // RobotAgent.step with unicycle kinematics (robot_agent.py:116-136), action = ActionRot(v, r): the position advances along

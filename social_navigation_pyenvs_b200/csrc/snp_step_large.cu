@@ -450,7 +450,7 @@ __global__ void __launch_bounds__(kTile) k_large_pairs_list(const LargeArgs<T> l
     }
 }
 
-// The robot after `steps` robot.step calls from the state in a.robot (robot_agent.py:116-136), with k_step's expressions: rb[] gets
+// The robot after `steps` robot.step calls from the state in a.robot (robot_agent.py:116-136), stepped as k_step does: rb[] gets
 // SNP_ROBOT_PX, PY, VX, VY and TH.  In a batch env e's robot is a.robot[field * E + e] and its action a.action[e], a.action[E + e].
 template <typename T, bool kBatch> __device__ __forceinline__ void large_robot_replay(const KArgs<T> &a, int steps, T *rb, int e) {
     const long long RE = kBatch ? a.E : 1;
@@ -458,13 +458,10 @@ template <typename T, bool kBatch> __device__ __forceinline__ void large_robot_r
     rb[SNP_ROBOT_VX] = a.robot[SNP_ROBOT_VX * RE + e]; rb[SNP_ROBOT_VY] = a.robot[SNP_ROBOT_VY * RE + e]; rb[SNP_ROBOT_TH] = a.robot[SNP_ROBOT_TH * RE + e];
     if (steps <= 0) return;
     const T dt = a.dt;
-    if (a.robot_mode == 1) {  // holonomic: p = p + a*dt ; v = a
+    if (a.robot_mode == 1) {  // holonomic: v = a
         const T ax = a.action[e], ay = a.action[RE + e];
         T px = rb[SNP_ROBOT_PX], py = rb[SNP_ROBOT_PY];
-        for (int s = 0; s < steps; ++s) {
-            if (sizeof(T) == 8) { px = (T)__dadd_rn((double)px, __dmul_rn((double)ax, (double)dt)); py = (T)__dadd_rn((double)py, __dmul_rn((double)ay, (double)dt)); }
-            else { px = px + ax * dt; py = py + ay * dt; }
-        }
+        for (int s = 0; s < steps; ++s) { px = robot_holonomic_step<T>(px, ax, dt); py = robot_holonomic_step<T>(py, ay, dt); }
         rb[SNP_ROBOT_PX] = px; rb[SNP_ROBOT_PY] = py; rb[SNP_ROBOT_VX] = ax; rb[SNP_ROBOT_VY] = ay;
     } else if (a.robot_mode == 3) {  // unicycle (v, r)
         for (int s = 0; s < steps; ++s) robot_unicycle_step<T>(rb, (double)a.action[e], (double)a.action[RE + e], (double)dt);
@@ -818,12 +815,18 @@ inline LargeBatchScratch large_batch_scratch(long long E, long long N, long long
 inline long long units_in(long long scratch_bytes, long long bytes_for_none, long long elem_bytes) {
     return scratch_bytes < bytes_for_none ? -1 : (scratch_bytes - bytes_for_none) / unit_bytes(elem_bytes);
 }
+// The longest decay length of a step's pair law (Helbing B, Guo max(B, D)) when the step is culled, else -1: SNP_OPT_NO_CULLING,
+// Moussaid (no culling distance) or a decay length that is not positive.
+inline double large_cull_length(const snp_crowd *c, const snp_step_opts *o) {
+    const int soc = o->type % 3;
+    const double B = c->params[3], D = c->params[7];
+    if ((o->reserved & SNP_OPT_NO_CULLING) || soc == 2 || !(B > 0) || (soc == 1 && !(D > 0))) return -1.0;
+    return soc == 1 && D > B ? D : B;
+}
+
 // Does a step take the work list (culled, one agent per thread) and hence the slot layout?  Otherwise the static grid.
 inline bool large_uses_list(const snp_crowd *c, const snp_step_opts *o, long long self_offset, long long blocks, long long J) {
-    const int soc = o->type % 3;
-    const bool culled = !(o->reserved & SNP_OPT_NO_CULLING) &&
-                        ((soc == 0 && c->params[3] > 0) || (soc == 1 && c->params[3] > 0 && c->params[7] > 0));
-    return culled && self_offset % kTile == 0 && blocks * J < (1LL << 31);
+    return large_cull_length(c, o) > 0.0 && self_offset % kTile == 0 && blocks * J < (1LL << 31);
 }
 
 template <typename T, bool kBatch> int dispatch_large(int type, const LargeArgs<T> &la, bool unit_slots, bool first, cudaStream_t st) {
@@ -882,13 +885,9 @@ template <typename T> int run_large(const snp_crowd *c, const snp_step_opts *o, 
     la.live_cnt = (int *)(base + sc.live_cnt);
     la.live_list = (int *)(base + sc.live_list);
     // culling distance beyond the r+s sums: where exp(rd/B) has fallen below e^-700 (fp64) / e^-88 (fp32), see the header
-    const int soc = o->type % 3;
     const double under = sizeof(T) == 8 ? 700.0 : 88.0;
-    double margin = -1.0;
-    if (!(o->reserved & 2)) {
-        if (soc == 0 && c->params[3] > 0) margin = under * c->params[3];
-        else if (soc == 1 && c->params[3] > 0 && c->params[7] > 0) margin = under * (c->params[3] > c->params[7] ? c->params[3] : c->params[7]);
-    }
+    const double cull_length = large_cull_length(c, o);
+    const double margin = cull_length > 0.0 ? under * cull_length : -1.0;
     la.cull_margin = (T)margin;
     // culled steps: one agent per thread (twice the units to hand out).  Round 2 kept two for fp32 on the static grid, where the
     // finer split only added CTAs to launch; on the work list one rank's slice of an 8-way split runs 0.0552 -> 0.0408 ms in fp32
