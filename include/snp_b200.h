@@ -32,6 +32,7 @@
  *   snp_pack_states / snp_unpack_states           <- src/agent.py:256-266 get_safe_state / set_state row layout
  *   snp_large_run_p2p                             <- same update for one very large crowd (tiled all-pairs), with its robot
  *   snp_large_checks                              <- the checks above for the robot of one very large crowd
+ *   snp_spatial_order / snp_gather_crowd          <- scenarios.spatial_order (+ deal_tiles) and new_rows = old_rows[perm], mid-run
  */
 #ifndef SNP_B200_H
 #define SNP_B200_H
@@ -307,6 +308,35 @@ int snp_large_batch_step(const snp_crowd *crowd, const snp_step_opts *opts, void
 /* Writes this crowd's [5][.] entity view (x,y,vx,vy,r+safety; v = R(yaw) bv for headed models) into `view` (field stride
  * `stride` elements, starting at element `offset`). */
 int snp_large_publish(const snp_crowd *crowd, int32_t type, void *view, int64_t stride, int64_t offset, void *cuda_stream);
+/* The [ceil(M/128)][5] tile-box table (xmin, xmax, ymin, ymax, max r+safety of every 128-entity tile) of a view buffer `view` =
+ * [5][M] entities followed by that table, as the first sub-step of a snp_large_run_p2p call computes it: a view republished between
+ * calls (e.g. after a re-numbering) then carries the boxes of its own entities. */
+int snp_large_tile_boxes(void *view, int64_t M, int32_t dtype, void *cuda_stream);
+
+/* ---- re-numbering the humans patch by patch (csrc/snp_order.cu) ----
+ * The far-tile culling of the tiled path compares bounding boxes of runs of 128 consecutive humans, so it skips more when
+ * consecutive humans stand close together.  A crowd that walks for long mixes; re-numbering it now and then keeps its tiles compact.
+ * snp_spatial_order: for each of E envs of N humans (positions px, py [E*N] in `dtype`), perm [E][N] int64 = the permutation
+ * scenarios.spatial_order(positions) returns with block = 256 -- max(1, round_half_even(sqrt(N / 256))) strips of equal head count
+ * (the first N % strips one human more, as np.array_split) cut from the humans in ascending x, each walked in ascending y, every
+ * sort stable (ties keep index order), -0.0 equal to +0.0, fp32 positions ordered as their float64 widening.  perm[e][k] is the
+ * env-local index the human going to place k has now: new rows = old rows[perm].  world > 1 (N a whole number of 128-human tiles)
+ * then deals the tiles round-robin to `world` ranks (scenarios.deal_tiles).  *nonfinite (device int32) is set to 1 when a position
+ * is NaN or infinite, to 0 otherwise; perm is then meaningless.  Stable CUB radix sorts on `cuda_stream`, no host synchronisation;
+ * `scratch` = 16-byte aligned device workspace of at least snp_spatial_order_scratch_bytes(E, N) bytes (which asks CUB for its
+ * temporary storage: it needs the CUDA device; -1 for bad arguments or a CUDA error).  E * N < 2^31. */
+int64_t snp_spatial_order_scratch_bytes(int32_t E, int32_t N);
+int snp_spatial_order(const void *px, const void *py, int32_t E, int32_t N, int32_t dtype, int32_t world, int64_t *perm,
+                      int32_t *nonfinite, void *scratch, int64_t scratch_bytes, void *cuda_stream);
+/* Applies a re-numbering to every per-agent array of `dst` (dyn, all SNP_DYN_FIELDS fields with the carried desired force; stat;
+ * goals; goal_idx; goal_cnt) from `src`, a crowd of the same E, G and dtype with src->N >= offset + dst->N humans per env: agent k
+ * of env e of dst = agent perm[e * src->N + offset + k] of env e of src.  So a rank of an agent-sharded crowd takes its slice
+ * [offset, offset + n_local) of the re-numbered whole crowd from a gathered copy of it, and one crowd (offset 0, same N) from a
+ * copy of itself; dst and src must not overlap.  The robot, walls and parameters are not per-agent arrays and are not touched;
+ * agent_params is SNP_ERR_UNSUPPORTED.  An entry of perm outside 0..src->N-1 sets *error_flag (optional device int32) and leaves
+ * that agent unwritten.  One launch, no host synchronisation. */
+int snp_gather_crowd(const snp_crowd *dst, const snp_crowd *src, const int64_t *perm, int64_t offset, int32_t *error_flag,
+                     void *cuda_stream);
 
 /* ---- host-pointer API (the reference operator, batched over a leading env axis) ----
  * update_humans_parallel(type, agents_state, goals, obstacles, agents_params, dt, safety_space,

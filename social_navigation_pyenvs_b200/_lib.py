@@ -91,6 +91,10 @@ _SIGNATURES = {
     "snp_large_batch_scratch_bytes": (c_int64, [c_int32, c_int32, c_int32]),
     "snp_large_batch_scratch_bytes_units": (c_int64, [c_int32, c_int32, c_int32, c_int64]),
     "snp_large_batch_step": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p, c_int64, c_void_p]),
+    "snp_large_tile_boxes": (ctypes.c_int, [c_void_p, c_int64, c_int32, c_void_p]),
+    "snp_spatial_order_scratch_bytes": (c_int64, [c_int32, c_int32]),
+    "snp_spatial_order": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "snp_gather_crowd": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpCrowd), c_void_p, c_int64, c_void_p, c_void_p]),
     "snp_update_humans_parallel_host":(ctypes.c_int, [c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                                        c_void_p, c_double, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,
                                                        c_void_p, c_void_p]),

@@ -1247,4 +1247,16 @@ int snp_large_publish(const snp_crowd *c, int32_t type, void *view, int64_t stri
     return SNP_OK;
 }
 
+int snp_large_tile_boxes(void *view, int64_t M, int32_t dtype, void *stream) {
+    if (!view) { set_error("snp_large_tile_boxes: null argument"); return SNP_ERR_INVALID; }
+    if (M < 1) { set_error("snp_large_tile_boxes: M must be >= 1 (got %lld)", (long long)M); return SNP_ERR_INVALID; }
+    if (dtype != SNP_F64 && dtype != SNP_F32) { set_error("snp_large_tile_boxes: bad dtype %d", dtype); return SNP_ERR_INVALID; }
+    const unsigned n_tiles = (unsigned)((M + kTile - 1) / kTile);
+    if (dtype == SNP_F64) k_tile_boxes<double, false><<<n_tiles, kTile, 0, (cudaStream_t)stream>>>((const double *)view, M, (double *)view + 5 * M, 0, 0);
+    else k_tile_boxes<float, false><<<n_tiles, kTile, 0, (cudaStream_t)stream>>>((const float *)view, M, (float *)view + 5 * M, 0, 0);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    return SNP_OK;
+}
+
 }  // extern "C"

@@ -22,7 +22,7 @@ import torch
 
 from . import _lib as L
 from .engine import CrowdEngine, SFMS
-from .parallel import all_gather_columns, agent_shard
+from .parallel import all_gather_columns, all_gather_columns_packed, agent_shard
 
 # unit_capacity="auto" starts with this many partial-sum slots per 128-agent block (DESIGN 4.3: what the bench crowd lists)
 AUTO_UNITS_PER_BLOCK = 32
@@ -87,6 +87,45 @@ class _UnitSlots:
         The counts are kept only with a capacity: None at the default size."""
         most, fallback = (int(v) for v in self._stats.tolist()) if self._stats_valid else (None, None)
         return {"capacity": self._last_capacity, "max_listed": most, "fallback_units": fallback}
+
+
+def device_spatial_order(px, py, world=1):
+    """scenarios.spatial_order of every env's positions on the device (snp_spatial_order): px, py device tensors [E, N] (or [N]) of
+    float32 / float64 -> int64 device tensor of the same shape, perm[e][k] = the index the human going to place k has now.  world > 1
+    also deals the 128-human tiles to `world` ranks (scenarios.deal_tiles; N a whole number of tiles).  Non-finite positions raise
+    ValueError (reading that flag synchronises the stream)."""
+    lib = L.lib()
+    x, y = px.contiguous(), py.contiguous()
+    E, N = (1, x.numel()) if x.dim() == 1 else tuple(x.shape)
+    perm = torch.empty(x.shape, dtype=torch.int64, device=x.device)
+    flag = torch.empty((1,), dtype=torch.int32, device=x.device)
+    scratch = torch.empty((L.check_size(lib.snp_spatial_order_scratch_bytes(E, N)),), dtype=torch.uint8, device=x.device)
+    dt = L.SNP_F64 if x.dtype == torch.float64 else L.SNP_F32
+    L.check(lib.snp_spatial_order(ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(y.data_ptr()), E, N, dt, int(world),
+                                  ctypes.c_void_p(perm.data_ptr()), ctypes.c_void_p(flag.data_ptr()), ctypes.c_void_p(scratch.data_ptr()),
+                                  scratch.numel(), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    if int(flag.item()):
+        raise ValueError("spatial order: a position is NaN or infinite")
+    return perm
+
+
+def _gather_crowd(eng, perm, offset, src):
+    """eng's per-agent arrays (its slice [offset, offset + eng.N) of every env) := those of `src` re-numbered by perm [E, M] (device
+    int64); src = (dyn [10, E, M], stat [4, E, M], goals [G, 2, E, M], goal_idx [E, M], goal_cnt [E, M]) not overlapping eng's."""
+    dyn, stat, goals, gi, gc = src
+    c = eng._crowd()  # the source crowd: eng's E, G, dtype and parameters, its own N and arrays
+    c.N = gi.shape[-1]
+    c.dyn, c.stat, c.goals, c.goal_idx, c.goal_cnt = dyn.data_ptr(), stat.data_ptr(), goals.data_ptr(), gi.data_ptr(), gc.data_ptr()
+    err = torch.zeros((1,), dtype=torch.int32, device=eng.device)
+    L.check(eng.lib.snp_gather_crowd(ctypes.byref(eng._crowd()), ctypes.byref(c), ctypes.c_void_p(perm.data_ptr()), int(offset),
+                                     ctypes.c_void_p(err.data_ptr()), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    if int(err.item()):
+        raise ValueError("renumber: a permutation entry is out of range")
+
+
+def _own_arrays(eng):
+    """Copies of eng's per-agent arrays: the source of a re-numbering of the crowd itself."""
+    return eng.dyn.clone(), eng.stat.clone(), eng.goals.clone(), eng.goal_idx.clone(), eng.goal_cnt.clone()
 
 
 class LargeCrowd(_UnitSlots):
@@ -166,6 +205,7 @@ class LargeCrowd(_UnitSlots):
         self._setup_units(unit_capacity, -(-self.n_local // 128), -(-self.n_total // 128), size_of, self.eng.device)
         self.culling = True
         self.cur = 0
+        self._sharded_slice = shard is not None
         if shard is not None:  # the frozen rest of the crowd: both view buffers start from the whole crowd's entries
             whole = CrowdEngine.from_reference_arrays(model, states[None], goals[None], consider_robot=False, all_params_equal=symmetric, dtype=dtype, device=device)
             for v in self.view:
@@ -190,6 +230,42 @@ class LargeCrowd(_UnitSlots):
         L.check(self.eng.lib.snp_large_publish(ctypes.byref(self.eng._crowd()), self.type, ctypes.c_void_p(v.data_ptr()), self.n_total,
                                                self.offset, self._stream()))
         self._gather(v)
+
+    def renumber(self):
+        """Re-numbers the whole crowd patch by patch (scenarios.spatial_order of the current positions, then deal_tiles over the ranks
+        when world > 1 and the crowd is a whole number of 128-human tiles) and returns perm (int64 [n_total], host): perm[k] is the
+        index the human now at k had before, new_rows = old_rows[perm]; np.argsort(perm) undoes it.  Every per-agent array moves with
+        its human -- state, carried desired force, safety, goal list and the index of the current goal -- and so do the radii the
+        checks and the laser read; the view and its tile boxes are republished.  Every index reported afterwards (rows, laser hits)
+        is in the new numbering.  The steps that follow compute what a crowd built from the re-numbered rows computes, bit for bit,
+        and their far-tile culling skips as much as on a freshly ordered crowd.  Every rank computes the same permutation from the
+        view it holds; with world > 1 the other ranks' agents arrive in one all-gather.  Slice sizes and offsets, the robot and the
+        unit capacity do not change."""
+        if self._sharded_slice:
+            raise ValueError("renumber: a crowd built with shard= steps a slice against a frozen rest and cannot be re-numbered")
+        e, M, v = self.eng, self.n_total, self.view[self.cur]
+        deal = self.world if self.world > 1 and M % 128 == 0 else 1
+        perm = device_spatial_order(v[0], v[1], world=deal)
+        if self.world == 1:
+            src = _own_arrays(e)
+        else:  # the whole crowd in the old numbering, from every rank's slice
+            d = e.dtype
+            dyn, stat = torch.empty((L.DYN_FIELDS, 1, M), dtype=d, device=e.device), torch.empty((L.STAT_FIELDS, 1, M), dtype=d, device=e.device)
+            goals = torch.empty((e.G, 2, 1, M), dtype=d, device=e.device)
+            ints = torch.empty((2, M), dtype=torch.int32, device=e.device)
+            sl = slice(self.offset, self.offset + self.n_local)
+            dyn[..., sl], stat[..., sl], goals[..., sl] = e.dyn, e.stat, e.goals
+            ints[0, sl], ints[1, sl] = e.goal_idx[0], e.goal_cnt[0]
+            all_gather_columns_packed([dyn.view(-1, M), stat.view(-1, M), goals.view(-1, M), ints], self.offset, self.n_local, self.world,
+                                      self.group)
+            src = (dyn, stat, goals, ints[0:1], ints[1:2])
+        _gather_crowd(e, perm.view(1, M), self.offset, src)
+        if self.has_robot:
+            self.radius = self.radius[perm]
+        self._publish()
+        L.check(e.lib.snp_large_tile_boxes(ctypes.c_void_p(self.view[self.cur].data_ptr()), M,
+                                           L.SNP_F64 if e.dtype == torch.float64 else L.SNP_F32, self._stream()))
+        return perm.cpu().numpy()
 
     def step(self, dt=0.0125, n_substeps=1, action=None, kinematics="holonomic", pre_checks=False, post_checks=False):
         """n_substeps updates of the crowd.  With a robot: SocialNavGym.step -- the swept check on the current state (pre_checks),
@@ -316,6 +392,17 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
             self.action.copy_(a.t() if a.shape == (self.E, 2) else a)
         self._run(self._opts(dt, n_substeps, robot_mode=1 if kinematics == "holonomic" else 3, pre_checks=pre_checks,
                              post_checks=post_checks, advance_time=True))
+
+    def renumber(self):
+        """Re-numbers the humans of every env among themselves patch by patch (scenarios.spatial_order of the env's current
+        positions) and returns perm (int64 [E, N], host): perm[e][k] is the index in env e the human now at k had before,
+        new_rows[e] = old_rows[e][perm[e]]; np.argsort(perm[e]) undoes it.  Every per-agent array moves with its human -- state,
+        carried desired force, safety, goal list and the index of the current goal; the robots and the walls stay.  Every index
+        reported afterwards (rows, laser hits, the swept check's first collision) is in the new numbering: compose perm with any
+        bookkeeping of your own.  Env e then steps bit for bit as a LargeCrowd of env e alone re-numbered the same way."""
+        perm = device_spatial_order(self.dyn[L.DYN_PX], self.dyn[L.DYN_PY])
+        _gather_crowd(self, perm, 0, _own_arrays(self))
+        return perm.cpu().numpy()
 
     def _unsupported(self, what):
         raise NotImplementedError(f"TiledCrowdEngine: {what} is not available on the tiled path (snp_large_batch_step)")

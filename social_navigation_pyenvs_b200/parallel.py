@@ -39,6 +39,27 @@ def all_gather_columns(buf, offset, n_local, world, group=None):
     return buf
 
 
+def all_gather_columns_packed(bufs, offset, n_local, world, group=None):
+    """all_gather_columns for several buffers [F_i, N_total] of any dtypes in ONE collective: this rank's columns of every buffer
+    travel as one byte string."""
+    if world == 1:
+        return bufs
+    import torch.distributed as dist
+    local = torch.cat([b[:, offset:offset + n_local].contiguous().view(torch.uint8).reshape(-1) for b in bufs])
+    parts = torch.empty((world, local.numel()), dtype=torch.uint8, device=local.device)
+    if local.is_cuda:
+        dist.all_gather_into_tensor(parts, local, group=group)
+    else:  # gloo has no all_gather_into_tensor
+        dist.all_gather(list(parts.unbind(0)), local, group=group)
+    for r in range(world):
+        at = 0
+        for b in bufs:
+            nb = b.shape[0] * n_local * b.element_size()
+            b[:, r * n_local:(r + 1) * n_local].copy_(parts[r, at:at + nb].view(b.dtype).view(b.shape[0], n_local))
+            at += nb
+    return bufs
+
+
 def max_over_ranks(value, device, world, group=None):
     """Device-timed durations are reported as the max over ranks."""
     if world == 1:
