@@ -178,7 +178,10 @@ typedef struct snp_lookahead_args {
     int32_t type;             /* the humans' model 0..8 (headed models take yaw / omega from `next`, the others from the crowd) */
     int32_t A;                /* number of actions */
     int32_t theta_and_omega_visible; /* 0: 13 values per (action, human); 1: 15 (cadrl.py:14-21) */
-    int32_t reserved;         /* bit 0: write the rows with per-thread vector stores instead of bulk asynchronous copies (A/B measurement) */
+    int32_t reserved;         /* bit 0: write the rows with per-thread vector stores instead of bulk asynchronous copies (A/B measurement);
+                                 bit 1: split every env's humans into chunks of 256 over several CTAs, which is what runs by itself
+                                 where one CTA's shared memory cannot hold an env (fp64 N > 673 / > 609 visible, fp32 > 1312 / > 1190);
+                                 the same bits either way (tests and measurement).  Any N; the outputs may exceed 2^31 words */
     const void *next;         /* [SNP_DYN_FIELDS][E*N] the humans one policy time step ahead: output of the peek (snp_step with dyn_out) */
     const double *actions;    /* [A][2] holonomic velocities (vx, vy), shared by all envs (cadrl.py build_action_space) */
     double dt;                /* the policy's time step (0.25) */

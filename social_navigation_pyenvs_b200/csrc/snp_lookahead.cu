@@ -12,6 +12,21 @@
 // 16-byte aligned; the (at most 15-byte) head and tail are written with scalar stores.
 // Rewards are computed in double with formula-exact operations (snp_math.cuh) so that they are bit-identical to the
 // reference for fp64 state; in fp32 mode from the widened fp32 state.
+//
+// Any N.  The CTA above stages all N humans of its env; once that layout needs more than 200 KB of shared memory even for one
+// action per CTA (fp64: N > 673 with 13 values, > 609 with 15; fp32: > 1312 / > 1190) the humans are split instead:
+// k_lookahead<T, true> covers (env, range of actions, chunk of H = kLookThreads humans), stages only its chunk, and writes the
+// rows [e][a][j0 : j0+H] of each action as one tile -- contiguous, so it leaves through the same bulk copy with the same 16-byte
+// head / tail handling and double buffering.  A thread owns one human of the chunk for all the CTA's actions, so a rotated row is
+// computed by the same code from the same operands whatever the decomposition.  Actions per CTA: split the action range until
+// E x chunks x ranges reaches 12 CTAs per SM, then further while shared memory exceeds 200 KB.
+// The reward needs collision = (some d < 0) and dmin = min over d >= 0 across all chunks, NaN taking part in neither: the
+// rewards are first filled with 0x7F bytes (as an int64 key 0x7F7F...7F, as a double a positive value above the reference's
+// initial dmin 9223372036854775807.0), every CTA folds its chunk into one signed 64-bit atomicMin per action (-1 for a
+// collision, else the bits of its smallest d >= 0 plus 0.0 -- positive doubles order like their bits), and k_lookahead_fold
+// decodes the key and applies the same reward expression (look_reward) as the whole-env kernel: bit-identical rewards, in
+// any order of the atomics.  snp_lookahead_args.reserved bit 1 forces the split where one CTA would hold the env (tests and
+// measurement), as bit 0 forces the vector stores.
 #include "snp_kernels.cuh"
 
 namespace snp {
@@ -30,7 +45,19 @@ struct LookArgs {
     void *rotated;
     double *rewards;
     int bulk;  // 1: tiles leave through cp.async.bulk; 0: cooperative vector stores (A/B comparison)
+    int H, nhc;  // split kernel: humans per chunk, chunks per env (blockIdx.x = action range * nhc + chunk)
 };
+
+// cadrl.py:56-72 from the folded swept test: the reward of action (axd, ayd) for the robot at (rpx, rpy) with goal (rgx, rgy)
+__device__ __forceinline__ double look_reward(bool collision, double dmin, double axd, double ayd, double dt, double rpx, double rpy,
+                                              double rgx, double rgy, double rr) {
+    const double npx = __dadd_rn(rpx, __dmul_rn(axd, dt)), npy = __dadd_rn(rpy, __dmul_rn(ayd, dt));
+    const bool reached = xnorm_plain(__dsub_rn(npx, rgx), __dsub_rn(npy, rgy)) < rr;
+    if (collision) return -0.25;
+    if (reached) return 1.0;
+    if (dmin < 0.2) return __dmul_rn(__dmul_rn(__dsub_rn(dmin, 0.2), 0.5), dt);
+    return 0.0;
+}
 
 // Per-action quantities shared by the humans of an env: next robot position, (cos, sin) of the rotation, distance to goal.
 template <typename T> struct PerAction { double axd, ayd; T npx, npy, c, s, dg, ax, ay, pad; };
@@ -49,15 +76,21 @@ template <typename T> struct LookSmem {
     }
 };
 
-template <typename T>
-__global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : 3) k_lookahead(const LookArgs a) {
+// kSplit = false: one CTA per (env, range of actions) with all N humans; true: per (env, range of actions, chunk of a.H humans),
+// the rewards folded by atomicMin (header comment).  N below is the number of humans the CTA stages.  An fp64 split CTA stages 256
+// humans and two tiles of 256 rows (> 75 KB of shared memory): 2 CTAs per SM, so it may use the registers of 2 without spilling.
+template <typename T, bool kSplit>
+__global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : (kSplit ? 2 : 3)) k_lookahead(const LookArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int N = a.N, OW = a.visible ? 15 : 13;
+    const int OW = a.visible ? 15 : 13;
     const int e = blockIdx.y;
-    const int abeg = blockIdx.x * a.aper;
+    const int hc = kSplit ? (int)(blockIdx.x % (unsigned)a.nhc) : 0;
+    const int j0 = kSplit ? hc * a.H : 0;
+    const int N = kSplit ? min(a.H, a.N - j0) : a.N;
+    const int abeg = (kSplit ? (int)(blockIdx.x / (unsigned)a.nhc) : (int)blockIdx.x) * a.aper;
     const int acnt = min(a.aper, a.A - abeg);
     const T *dyn = (const T *)a.dyn, *stat = (const T *)a.stat, *nxt = (const T *)a.next, *robot = (const T *)a.robot;
-    const long long EN = a.EN, base = (long long)e * N;
+    const long long EN = a.EN, base = (long long)e * a.N + j0;
 
     // shared memory: [cur: px py vx vy r | N each][next: x y vx vy th om | N each][per-action][dist x2][tile x2]
     const LookSmem<T> lay(N, OW, a.chunk, a.aper);
@@ -106,7 +139,7 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : 3) k_lookah
     }
     __syncthreads();
 
-    const size_t row_words = (size_t)N * OW;
+    const size_t row_words = (size_t)a.N * OW;  // one action's rows of the env; a split CTA's tile (chunk = 1) is its part of them
     const int nchunks = (acnt + a.chunk - 1) / a.chunk;
     // A thread keeps the same (action slot k, human j) in every tile (a tile holds at most blockDim pairs unless N > blockDim):
     // the human's state and everything of the swept test that does not depend on the action stay in registers across tiles.
@@ -144,7 +177,7 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : 3) k_lookah
         const int k0 = c * a.chunk;                    // first action of the tile, relative to abeg
         const int na = min(a.chunk, acnt - k0);
         const int pairs = na * N;
-        T *gdst = (T *)a.rotated + ((size_t)e * a.A + abeg + k0) * row_words;
+        T *gdst = (T *)a.rotated + ((size_t)e * a.A + abeg + k0) * row_words + (size_t)j0 * OW;
         const unsigned mis = (unsigned)(reinterpret_cast<uintptr_t>(gdst) & 15);
         // the tile sits in shared memory at the same offset modulo 16 as its destination: both sides of the copy 16-byte aligned
         T *tile = reinterpret_cast<T *>(smem_raw + lay.tile + (size_t)(c & 1) * lay.tile_stride + mis);
@@ -209,20 +242,67 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : 3) k_lookah
             collision |= d < 0;
             dmin = (d >= 0 && d < dmin) ? d : dmin;
         }
-        const PerAction<T> q = pa[k];
-        const double npx = __dadd_rn((double)rpx, __dmul_rn(q.axd, a.dt)), npy = __dadd_rn((double)rpy, __dmul_rn(q.ayd, a.dt));
-        const bool reached = xnorm_plain(__dsub_rn(npx, (double)rgx), __dsub_rn(npy, (double)rgy)) < (double)rr;
-        double rew;
-        if (collision) rew = -0.25;
-        else if (reached) rew = 1.0;
-        else if (dmin < 0.2) rew = __dmul_rn(__dmul_rn(__dsub_rn(dmin, 0.2), 0.5), a.dt);
-        else rew = 0.0;
-        a.rewards[(size_t)e * a.A + abeg + k] = rew;
+        if (kSplit) {  // this chunk's part of the swept test as an order-independent key (header comment)
+            const long long key = collision ? -1LL : __double_as_longlong(__dadd_rn(dmin, 0.0));  // -0.0 -> +0.0
+            atomicMin(reinterpret_cast<long long *>(a.rewards) + (size_t)e * a.A + abeg + k, key);
+        } else {
+            const PerAction<T> q = pa[k];
+            a.rewards[(size_t)e * a.A + abeg + k] =
+                look_reward(collision, dmin, q.axd, q.ayd, a.dt, (double)rpx, (double)rpy, (double)rgx, (double)rgy, (double)rr);
+        }
     }
     if (a.bulk && threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // tiles must outlive the copies' reads
 }
 
-template <typename T> int launch_lookahead(LookArgs a, cudaStream_t st) {
+// after the split kernel: rewards[e][a] holds the atomicMin key of the whole swept test; a thread per (env, action) decodes it
+template <typename T> __global__ void k_lookahead_fold(const LookArgs a) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)a.E * a.A) return;
+    const int e = (int)(i / a.A), k = (int)(i - (long long)e * a.A);
+    const long long key = reinterpret_cast<const long long *>(a.rewards)[i];
+    const double d = __longlong_as_double(key), cap = 9223372036854775807.0;  // np.iinfo(np.int64).max, the reference's initial dmin
+    const T *robot = (const T *)a.robot;
+    const long long E = a.E;
+    a.rewards[i] = look_reward(key < 0, d < cap ? d : cap, a.actions[2 * k], a.actions[2 * k + 1], a.dt, (double)robot[SNP_ROBOT_PX * E + e],
+                               (double)robot[SNP_ROBOT_PY * E + e], (double)robot[SNP_ROBOT_GX * E + e], (double)robot[SNP_ROBOT_GY * E + e],
+                               (double)robot[SNP_ROBOT_R * E + e]);
+}
+
+template <typename T> int launch_lookahead_split(LookArgs a, cudaStream_t st) {
+    const int N = a.N, OW = a.visible ? 15 : 13;
+    a.H = kLookThreads;  // a thread per human of the chunk, which it keeps across the CTA's actions
+    a.nhc = (N + a.H - 1) / a.H;
+    a.chunk = 1;         // a tile is one action's part of the rows: contiguous in the output
+    const int staged = min(N, a.H);
+    const int sms = device_sm_count();
+    int splits = 1;
+    // 12 CTAs per SM: of 6, 12, 24 and 48 the fastest for fp64 at 64 x 1024, 16 x 4096 and 1 x 65536 (DESIGN 4.5)
+    while (splits < a.A && (long long)a.E * a.nhc * splits < 12LL * sms) ++splits;
+    for (;; ++splits) {
+        a.aper = (a.A + splits - 1) / splits;
+        if (LookSmem<T>(staged, OW, 1, a.aper).total <= 200 * 1024 || a.aper == 1) break;
+    }
+    const LookSmem<T> lay(staged, OW, 1, a.aper);
+    const long long ctas = (long long)((a.A + a.aper - 1) / a.aper) * a.nhc;
+    if (lay.total > 200 * 1024 || ctas > 0x7fffffffLL) {
+        set_error("snp_lookahead: %d humans x %d values x %d actions exceed the split decomposition", N, OW, a.A);
+        return SNP_ERR_UNSUPPORTED;
+    }
+    SNP_CUDA_OK(cudaMemsetAsync(a.rewards, 0x7F, sizeof(double) * (size_t)a.E * a.A, st));
+    auto kern = k_lookahead<T, true>;
+    if (lay.total > 48 * 1024) SNP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
+    kern<<<dim3((unsigned)ctas, (unsigned)a.E), kLookThreads, lay.total, st>>>(a);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    const long long EA = (long long)a.E * a.A;
+    k_lookahead_fold<T><<<(unsigned)((EA + 255) / 256), 256, 0, st>>>(a);
+    count_launch();
+    SNP_CUDA_OK(cudaGetLastError());
+    return SNP_OK;
+}
+
+template <typename T> int launch_lookahead(LookArgs a, cudaStream_t st, bool split) {
+    if (split) return launch_lookahead_split<T>(a, st);
     const int N = a.N, OW = a.visible ? 15 : 13;
     // actions per tile: as many (action, human) pairs as threads, balanced over the tiles of a CTA; capped by shared memory
     int per = kLookThreads / N;
@@ -240,8 +320,8 @@ template <typename T> int launch_lookahead(LookArgs a, cudaStream_t st) {
         if (LookSmem<T>(N, OW, a.chunk, a.aper).total <= 200 * 1024 || a.aper == 1) break;
     }
     const LookSmem<T> lay(N, OW, a.chunk, a.aper);
-    if (lay.total > 200 * 1024) { set_error("snp_lookahead: %d humans x %d values do not fit a shared-memory tile", N, OW); return SNP_ERR_UNSUPPORTED; }
-    auto kern = k_lookahead<T>;
+    if (lay.total > 200 * 1024) return launch_lookahead_split<T>(a, st);  // the env's humans do not fit one CTA
+    auto kern = k_lookahead<T, false>;
     if (lay.total > 48 * 1024) SNP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
     kern<<<dim3((unsigned)((a.A + a.aper - 1) / a.aper), (unsigned)a.E), kLookThreads, lay.total, st>>>(a);
     count_launch();
@@ -306,8 +386,10 @@ extern "C" int snp_lookahead(const snp_crowd *c, const snp_lookahead_args *g, vo
     a.dyn = c->dyn; a.stat = c->stat; a.next = g->next; a.robot = c->robot;
     a.actions = g->actions; a.dt = g->dt; a.rotated = g->rotated; a.rewards = g->rewards;
     a.bulk = (g->reserved & 1) ? 0 : 1;
-    if (c->dtype == SNP_F64) return launch_lookahead<double>(a, (cudaStream_t)stream);
-    if (c->dtype == SNP_F32) return launch_lookahead<float>(a, (cudaStream_t)stream);
+    a.H = a.nhc = 0;
+    const bool split = (g->reserved & 2) != 0;
+    if (c->dtype == SNP_F64) return launch_lookahead<double>(a, (cudaStream_t)stream, split);
+    if (c->dtype == SNP_F32) return launch_lookahead<float>(a, (cudaStream_t)stream, split);
     set_error("dtype %d is neither SNP_F32 nor SNP_F64", c->dtype);
     return SNP_ERR_INVALID;
 }

@@ -507,11 +507,13 @@ class CrowdEngine:
         L.check(self.lib.snp_constant_velocity(ctypes.byref(self._crowd()), float(dt), ctypes.c_void_p(self._peek_buf.data_ptr()), _stream()))
         return self._peek_buf
 
-    def lookahead_from(self, nxt, time_step=0.25, theta_and_omega_visible=False, bulk_store=True, yaw_from_next=False):
+    def lookahead_from(self, nxt, time_step=0.25, theta_and_omega_visible=False, bulk_store=True, yaw_from_next=False, split_humans=False):
         """compute_rotated_states_and_reward on a given `nxt` [DYN_FIELDS,E,N].  With theta_and_omega_visible the next yaw / omega are
         read from `nxt` for headed models and from the current state otherwise (what get_next_human_observable_states returns,
         mmm:691-709); yaw_from_next=True reads them from `nxt` whatever the model (the constant-velocity propagation integrates
-        theta + omega dt for every model, cadrl.py:103)."""
+        theta + omega dt for every model, cadrl.py:103).  Any N: envs whose humans do not fit one CTA's shared memory are split
+        into chunks of humans (csrc/snp_lookahead.cu); split_humans=True splits them even where one CTA would hold them (the same
+        bits; for tests and measurement, like bulk_store=False)."""
         if getattr(self, "action_space", None) is None:
             raise ValueError("set_action_space(actions) first")
         if self.robot is None:
@@ -521,7 +523,7 @@ class CrowdEngine:
             self._rotated = torch.empty((self.E, A, self.N, ow), dtype=self.dtype, device=self.device)
             self._rewards = torch.empty((self.E, A), dtype=torch.float64, device=self.device)
         g = L.SnpLookaheadArgs()
-        g.type, g.A, g.theta_and_omega_visible, g.reserved = (max(self.type, 3) if yaw_from_next else self.type), A, int(theta_and_omega_visible), 0 if bulk_store else 1
+        g.type, g.A, g.theta_and_omega_visible, g.reserved = (max(self.type, 3) if yaw_from_next else self.type), A, int(theta_and_omega_visible), (0 if bulk_store else 1) | (2 if split_humans else 0)
         g.next, g.actions, g.dt = nxt.data_ptr(), self.action_space.data_ptr(), float(time_step)
         g.rotated, g.rewards = self._rotated.data_ptr(), self._rewards.data_ptr()
         L.check(self.lib.snp_lookahead(ctypes.byref(self._crowd()), ctypes.byref(g), _stream()))

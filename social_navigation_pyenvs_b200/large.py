@@ -355,9 +355,11 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
     """CrowdEngine for E environments of any number of humans each, N > 512 included: `update_humans` and `step` run
     snp_large_batch_step (the tiled kernels of LargeCrowd with an environment axis) in one call per step.  Environment e steps
     bit for bit as a LargeCrowd built from environment e alone.  Loading and reading are CrowdEngine's (from_reference_arrays,
-    rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env).  Per-agent parameter rows, respawn
-    and the snp_step features the tiled path does not have (peek and the lookahead through it, imitation_learning_step, sim_update,
-    step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
+    rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env), and so is the policies' lookahead
+    without a query of the env: lookahead(query_env=False) (the constant-velocity propagation, snp_constant_velocity) and
+    lookahead_from(next) work at any N (snp_lookahead splits an env's humans over several CTAs when one cannot hold them).
+    Per-agent parameter rows, respawn and the snp_step features the tiled path does not have (peek and the lookahead through it,
+    lookahead(query_env=True), imitation_learning_step, sim_update, step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
     carried from one step to the next.  culling=False evaluates every pair (the same result).  unit_capacity (a constructor and
     from_reference_arrays keyword): None, an int or "auto", as for LargeCrowd (_UnitSlots; unit_stats())."""
 
