@@ -198,12 +198,13 @@ typedef struct snp_lookahead_args {
 enum { SNP_RESET_CIRCULAR_CROSSING = 0, SNP_RESET_PARALLEL_TRAFFIC = 1, SNP_RESET_CCSO = 2,
        SNP_RESET_CCSO_SYNTHETIC = 3, /* 3 static humans + the circular-crossing sampler: the 25-human crowd of SURVEY.md 8(d) config 3 */
        SNP_RESET_HYBRID = 4          /* np.random.choice between the first two, then re-seed (social_nav_gym.py:155-157) */ };
+enum { SNP_RESET_FORCE_CTA = 1 };
 typedef struct snp_reset_args {
     int32_t scenario;
     int32_t randomize_attributes; /* desired speed ~ U(0.5,1.5), radius ~ U(0.3,0.5) per human, drawn first (social_nav_sim.py:217-220) */
     const uint32_t *seeds;        /* optional [E] device: np.random.seed argument of each env; NULL -> seed0 + env index */
     uint32_t seed0;
-    uint32_t reserved;
+    uint32_t reserved;            /* bit 0 (SNP_RESET_FORCE_CTA): use the CTA-per-env kernel even where the warp kernel fits */
     const uint8_t *mask;          /* optional [E] device: only envs with a non-zero entry are reset (restart of finished episodes) */
     double circle_radius, robot_radius, traffic_length, traffic_height;
     double human_mass, robot_mass, robot_desired_speed; /* 75 (social_nav_sim.py:141), 80 (robot_agent.py:16), 1 */
@@ -225,7 +226,11 @@ int snp_laser(const snp_laser_args *args, void *cuda_stream);
 /* RobotAgent.check_collisions (src/robot_agent.py:35-48): crowd->robot's position is pushed out of the humans it overlaps (in index
  * order), then out of the wall polygons it overlaps; sequential per env, bit-identical to the reference for fp64 state. */
 int snp_robot_push_out(const snp_crowd *crowd, void *cuda_stream);
-/* Rewrites crowd->dyn, stat (radius, mass, desired speed; the safety space is kept), goals, goal_idx, goal_cnt and crowd->robot. */
+/* Rewrites crowd->dyn, stat (radius, mass, desired speed; the safety space is kept), goals, goal_idx, goal_cnt and crowd->robot.
+ * One warp per env while four envs' scratch (624 generator words + 32 bytes per human) fits 200 KB of shared memory, N <= 1522;
+ * above that one CTA of 16 warps per env, which splits the test of a candidate against the placed humans between its warps, up to
+ * N = 6322; larger N is SNP_ERR_UNSUPPORTED before any launch (the host generators cover any N).  args->reserved bit 0
+ * (SNP_RESET_FORCE_CTA) takes the CTA kernel at any N up to that limit.  Both kernels give the same bits in every output. */
 int snp_reset(const snp_crowd *crowd, const snp_reset_args *args, void *cuda_stream);
 /* Uses crowd->dyn (current px,py,vx,vy,theta,omega), crowd->stat (radius) and crowd->robot (px,py,r,gx,gy,vd). */
 int snp_lookahead(const snp_crowd *crowd, const snp_lookahead_args *args, void *cuda_stream);
@@ -304,7 +309,9 @@ int snp_large_checks(const snp_crowd *crowd, const snp_step_opts *opts, const vo
  * bad E / N / G / dtype / type, missing arrays, a missing robot / action / flags and too small a scratch are SNP_ERR_INVALID.
  * snp_large_batch_scratch_bytes returns -1 for bad arguments.  SNP_OPT_UNIT_SCRATCH and the unit counts in words 1 and 2 of the
  * scratch are as for snp_large_run_p2p, with a scratch of snp_large_batch_scratch_bytes_units(E, N, dtype, units) bytes (units of
- * E * ceil(N/128) * ceil(N/128); Moussaid types and SNP_OPT_NO_CULLING refused); the same bits whatever the slot count. */
+ * E * ceil(N/128) * ceil(N/128); Moussaid types and SNP_OPT_NO_CULLING refused); the same bits whatever the slot count.
+ * With n_substeps = 0 a call is the checks alone, at any N (what snp_checks does for N <= 512): publish, then the pre- and / or
+ * post-checks on the current state; crowd->dyn, the robot and the clock are left as they are. */
 int64_t snp_large_batch_scratch_bytes(int32_t E, int32_t N, int32_t dtype);
 int64_t snp_large_batch_scratch_bytes_units(int32_t E, int32_t N, int32_t dtype, int64_t units);
 int snp_large_batch_step(const snp_crowd *crowd, const snp_step_opts *opts, void *scratch, int64_t scratch_bytes, void *cuda_stream);

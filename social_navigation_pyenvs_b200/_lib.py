@@ -12,6 +12,7 @@ SNP_F32, SNP_F64 = 0, 1
 # bits of snp_step_opts.reserved (include/snp_b200.h)
 SNP_OPT_FULL_PAIR_LOOP, SNP_OPT_NO_CULLING, SNP_OPT_MAP_WARP, SNP_OPT_MAP_BLOCK, SNP_OPT_STAGED_COPIES = 1, 2, 4, 8, 16
 SNP_OPT_UNIT_SCRATCH = 32
+SNP_RESET_FORCE_CTA = 1  # snp_reset_args.reserved bit 0
 # field order of the SoA buffers (include/snp_b200.h)
 DYN_PX, DYN_PY, DYN_VX, DYN_VY, DYN_TH, DYN_BVX, DYN_BVY, DYN_OM, DYN_DFX, DYN_DFY, DYN_FIELDS = range(11)
 STAT_R, STAT_M, STAT_VD, STAT_SAFETY, STAT_FIELDS = range(5)

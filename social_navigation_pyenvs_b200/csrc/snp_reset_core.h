@@ -15,7 +15,11 @@
 // the words the sequential algorithm would read if the l previous attempts were rejected), the first accepted attempt wins and
 // the stream advances past exactly the words a sequential run would have consumed.  Same draws, same result, but the serial latency
 // of an unlucky environment (hundreds of rejected attempts) shrinks by up to the group size.  On the host the group is one lane
-// (SoloGroup) and the code is the plain sequential algorithm; on the device it is a warp per environment.
+// (SoloGroup) and the code is the plain sequential algorithm; on the device it is a warp per environment, or, for crowds whose
+// scratch does not fit one warp's share of shared memory, a CTA per environment (CtaGroup, snp_reset.cu): every warp of the CTA
+// speculates on the same 32 attempts, tests them against its own STRIPE of the humans placed so far (j = j0(), j0() + jstep(), ...),
+// and first() / all() combine the warps' verdicts.  The collision test is a pure OR over j, so a striped test rejects exactly what a
+// full one rejects.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -33,9 +37,14 @@ enum { SNP_SCEN_CIRCULAR_CROSSING = 0, SNP_SCEN_PARALLEL_TRAFFIC = 1, SNP_SCEN_C
 // numpy/random/src/mt19937/mt19937.c: mt19937_seed (np.random.seed(int)), mt19937_gen, and random_double of the legacy
 // distributions: (a >> 5, b >> 6) -> (a * 2^26 + b) / 2^53.
 struct SoloGroup {  // one lane: the sequential algorithm
+    static constexpr bool kStriped = false;  // true: several warps share the candidates, see CtaGroup (snp_reset.cu)
     SNP_HD int lane() const { return 0; }
     SNP_HD int size() const { return 1; }
-    SNP_HD int first(bool v) const { return v ? 0 : -1; }  // lowest lane whose flag is set, or -1
+    SNP_HD bool leader() const { return true; }            // the one member that does the group's sequential writes
+    SNP_HD int j0() const { return 0; }                    // the stripe of placed humans this member tests: j0, j0 + jstep, ...
+    SNP_HD int jstep() const { return 1; }
+    SNP_HD int first(bool v) const { return v ? 0 : -1; }  // lowest lane whose flag is set (in every stripe), or -1
+    SNP_HD bool all(bool v) const { return v; }            // v holds in every stripe (every lane tests the same candidate)
     SNP_HD double bcast(double v, int) const { return v; }
     SNP_HD void sync() const {}
 };
@@ -48,28 +57,38 @@ template <class Group> struct Mt19937 {
     SNP_HD uint32_t &at(int i) { return mt[i]; }
     SNP_HD void seed(uint32_t s) {  // sequential recurrence: one lane writes, everybody waits
         g.sync();                   // nobody is still reading the previous state
-        if (g.lane() == 0)
+        if (g.leader())
             for (int i = 0; i < 624; ++i) { at(i) = s; s = 1812433253u * (s ^ (s >> 30)) + (uint32_t)(i + 1); }
         g.sync();
         pos = 624;
     }
     // mt19937_gen's regeneration of all 624 words.  Word kk needs the OLD words kk, kk+1 and, for kk < 227, the OLD word kk+397,
     // else the NEW word kk-227 (and the new word 0 for kk = 623): a batch of `size` consecutive words reads everything it needs
-    // before any of them is written, and what it reads as new was written by an earlier batch.
+    // before any of them is written, and what it reads as new was written by an earlier batch (a batch must not exceed 227 words).
+    // A striped group twists in its first warp, between barriers of the whole group.
     SNP_HD void twist() {
+        if constexpr (Group::kStriped) {
+            g.sync();
+            if (g.twister()) twist_by(g.warp());
+            g.sync();
+        } else {
+            twist_by(g);
+        }
+        pos = 0;
+    }
+    template <class W> SNP_HD void twist_by(const W &t) {
         const uint32_t UP = 0x80000000u, LO = 0x7fffffffu, A = 0x9908b0dfu;
-        for (int base = 0; base < 624; base += g.size()) {
-            const int kk = base + g.lane();
+        for (int base = 0; base < 624; base += t.size()) {
+            const int kk = base + t.lane();
             uint32_t v = 0;
             if (kk < 624) {
                 const uint32_t y = (at(kk) & UP) | (at(kk + 1 == 624 ? 0 : kk + 1) & LO);
                 v = at(kk < 624 - 397 ? kk + 397 : kk - (624 - 397)) ^ (y >> 1) ^ ((y & 1u) ? A : 0u);
             }
-            g.sync();
+            t.sync();
             if (kk < 624) at(kk) = v;
-            g.sync();
+            t.sync();
         }
-        pos = 0;
     }
     SNP_HD uint32_t peek32(int i) {  // tempered output of state word i (the output next32() returns when pos == i)
         uint32_t y = at(i);
@@ -97,7 +116,7 @@ struct ResetParams {
     double circle_radius, robot_radius, traffic_length, traffic_height;
 };
 
-// Scratch of one environment: positions, radii and desired speeds of the humans placed so far.  Every lane of the group writes the
+// Scratch of one environment: positions, radii and desired speeds of the humans placed so far.  Every member of the group writes the
 // same value to the same slot (benign), reads happen after a group sync.
 struct ResetScratch {
     double *px, *py, *rad, *vd;
@@ -134,7 +153,7 @@ SNP_HD void reset_place(Mt19937<Group> &rng, Cand &cand, Coll &collides, double 
             double u[DRAWS];
             for (int d = 0; d < DRAWS; ++d) u[d] = rng.random();
             cand(u, x, y, angle);
-            if (!collides(x, y)) return;
+            if (g.all(!collides(x, y))) return;
             continue;
         }
         const int width = avail < g.size() ? avail : g.size();
@@ -195,9 +214,9 @@ SNP_HD int reset_generate(const ResetParams &p, uint32_t seed, Mt19937<Group> &r
                 angle = 0.0;
             };
             auto collides = [&](double x, double y) {  // any hit rejects (the reference's `break` only ends its loop)
-                for (int j = 0; j < i; ++j)
+                for (int j = g.j0(); j < i; j += g.jstep())
                     if (reset_norm(x - w.X(j), y - w.Y(j)) - ri - w.R(j) - 0.1 < 0) return true;
-                return reset_norm(x - rx, y - ry) - ri - p.robot_radius - 0.1 < 0;
+                return g.j0() == 0 && reset_norm(x - rx, y - ry) - ri - p.robot_radius - 0.1 < 0;  // the robot: once, in stripe 0
             };
             double x, y, angle;
             reset_place<2>(rng, cand, collides, x, y, angle);
@@ -234,7 +253,7 @@ SNP_HD int reset_generate(const ResetParams &p, uint32_t seed, Mt19937<Group> &r
             }
         };
         auto collides = [&](double x, double y) {
-            for (int j = 0; j < i; ++j) {
+            for (int j = g.j0(); j < i; j += g.jstep()) {
                 const double md = ri + w.R(j) + 0.2;
                 const double ox = w.X(j), oy = w.Y(j);
                 if (reset_norm(x - ox, y - oy) < md) return true;
@@ -244,7 +263,7 @@ SNP_HD int reset_generate(const ResetParams &p, uint32_t seed, Mt19937<Group> &r
                     if (reset_norm(x - gx, y - gy) < md) return true;
                 }
             }
-            if (!positions_only) {
+            if (!positions_only && g.j0() == 0) {  // the robot: once, in stripe 0
                 const double rm = ri + p.robot_radius + 0.2;
                 if (reset_norm(x - 0.0, y - (-R)) < rm || reset_norm(x - 0.0, y - R) < rm) return true;
             }

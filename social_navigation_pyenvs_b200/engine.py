@@ -432,11 +432,14 @@ class CrowdEngine:
 
     # ------------------------------------------------------------------ on-device reset (SURVEY 8f-4)
     def reset_scenario(self, scenario, seeds=None, seed0=0, mask=None, randomize_attributes=False, circle_radius=7.0, robot_radius=0.3,
-                       traffic_length=14.0, traffic_height=3.0, human_mass=75.0, robot_mass=80.0, robot_desired_speed=1.0):
+                       traffic_length=14.0, traffic_height=3.0, human_mass=75.0, robot_mass=80.0, robot_desired_speed=1.0,
+                       force_cta=False):
         """SocialNavGym.reset (social_nav_gym.py:120-225) for every env -- or those selected by `mask` [E] bool -- without leaving the
         device: env e replays the reference's generator for `scenario` on NumPy's MT19937 stream seeded with seeds[e] (default
         seed0 + e), as np.random.seed(offset[phase] + case) does (:135-137).  Returns (scenario_of_env int32 [E], draws int32 [E])
-        device tensors; parallel-traffic envs get their respawn switched on (mmm:407-422)."""
+        device tensors; parallel-traffic envs get their respawn switched on (mmm:407-422).  A warp generates an env up to 1,522
+        humans, a CTA above that (up to 6,322); force_cta=True takes the CTA kernel at any N (the same bits; for tests and
+        measurement)."""
         if self.robot is None:
             raise ValueError("the scenarios place a robot: build the engine with has_robot=True")
         g = L.SnpResetArgs()
@@ -453,6 +456,7 @@ class CrowdEngine:
                 raise ValueError("seeds must have one entry per env")
             g.seeds = seeds_t.data_ptr()
         g.seed0 = int(seed0) & 0xFFFFFFFF
+        g.reserved = L.SNP_RESET_FORCE_CTA if force_cta else 0
         mask_t = None
         if mask is not None:
             mask_t = torch.as_tensor(mask, device=dev).to(torch.uint8).contiguous()

@@ -357,7 +357,8 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
     bit for bit as a LargeCrowd built from environment e alone.  Loading and reading are CrowdEngine's (from_reference_arrays,
     rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env), and so is the policies' lookahead
     without a query of the env: lookahead(query_env=False) (the constant-velocity propagation, snp_constant_velocity) and
-    lookahead_from(next) work at any N (snp_lookahead splits an env's humans over several CTAs when one cannot hold them).
+    lookahead_from(next) work at any N (snp_lookahead splits an env's humans over several CTAs when one cannot hold them).  The
+    checks without a step (run_checks, check_actual_collisions_and_goal, collision_detection_and_reaching_goal) work at any N.
     Per-agent parameter rows, respawn and the snp_step features the tiled path does not have (peek and the lookahead through it,
     lookahead(query_env=True), imitation_learning_step, sim_update, step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
     carried from one step to the next.  culling=False evaluates every pair (the same result).  unit_capacity (a constructor and
@@ -395,6 +396,21 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
         self._run(self._opts(dt, n_substeps, robot_mode=1 if kinematics == "holonomic" else 3, pre_checks=pre_checks,
                              post_checks=post_checks, advance_time=True))
 
+    def run_checks(self, action=None, pre=True, post=True, kinematics="holonomic"):
+        """CrowdEngine.run_checks at any N, and through it check_actual_collisions_and_goal and
+        collision_detection_and_reaching_goal.  N <= 512 with a holonomic action keeps CrowdEngine's snp_checks; otherwise one
+        snp_large_batch_step call with n_substeps = 0, whose env e gives the flags and checks of a LargeCrowd of env e alone, bit for
+        bit.  kinematics="unicycle" sweeps the robot with action (v, r), as step does."""
+        if kinematics not in ("holonomic", "unicycle"):
+            raise ValueError("kinematics must be 'holonomic' or 'unicycle'")
+        if self.N <= 512 and kinematics == "holonomic":
+            return super().run_checks(action, pre, post)
+        if action is not None:
+            a = torch.as_tensor(action, dtype=self.dtype, device=self.device)
+            self.action.copy_(a.t() if a.shape == (self.E, 2) else a)
+        self._run(self._opts(0.0, 0, robot_mode=1 if kinematics == "holonomic" else 3, pre_checks=pre, post_checks=post))
+        return self.decode_flags()
+
     def renumber(self):
         """Re-numbers the humans of every env among themselves patch by patch (scenarios.spatial_order of the env's current
         positions) and returns perm (int64 [E, N], host): perm[e][k] is the index in env e the human now at k had before,
@@ -402,9 +418,13 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
         carried desired force, safety, goal list and the index of the current goal; the robots and the walls stay.  Every index
         reported afterwards (rows, laser hits, the swept check's first collision) is in the new numbering: compose perm with any
         bookkeeping of your own.  Env e then steps bit for bit as a LargeCrowd of env e alone re-numbered the same way."""
+        return self._renumber().cpu().numpy()
+
+    def _renumber(self):
+        """renumber() with perm left on the device."""
         perm = device_spatial_order(self.dyn[L.DYN_PX], self.dyn[L.DYN_PY])
         _gather_crowd(self, perm, 0, _own_arrays(self))
-        return perm.cpu().numpy()
+        return perm
 
     def _unsupported(self, what):
         raise NotImplementedError(f"TiledCrowdEngine: {what} is not available on the tiled path (snp_large_batch_step)")

@@ -8,14 +8,27 @@ Env e of a reset is seeded `offset[phase] + case + e`, the rule of social_nav_gy
 
 One `step` is ONE kernel launch: swept collision / goal test + reward on the current state, then
 `robot_time_step / time_step` fused (robot.step + update_humans) sub-steps (social_nav_gym.py:232-245).
+
+Above 512 humans per env (human_num > MAX_FUSED_HUMANS) the gym runs on a TiledCrowdEngine: `step` is one snp_large_batch_step
+call, the checks run on the tiled path and the on-device reset takes a CTA per env above about 1,520 humans (up to about 6,300; the
+host reset covers any N).  The scenario generators place humans in random angular order, so every 128-human tile of an env would
+span the whole circle and the tiled step's far-tile culling would skip nothing: with `spatial_order` (a configure key, default
+True) the gym re-numbers the humans patch by patch after every reset (TiledCrowdEngine.renumber).  That changes only the order of
+summation (the last bits) and which colliding human the swept check stops at; rewards, terminated, truncated and info are the
+same.  observation() always lists the humans in the generator's order.  spatial_order=False keeps the generator's numbering: the
+gym then computes bit for bit what a TiledCrowdEngine built from the same rows computes.  Above 512 humans imitation_learning_step
+raises NotImplementedError, and so does `step` in parallel traffic and the hybrid scenario (their respawn is not on the tiled
+path).
 """
 import numpy as np
 import torch
 
 from .engine import CrowdEngine, SFMS, INFO_NAMES  # noqa: F401
+from .large import TiledCrowdEngine
 from . import scenarios, _lib as L
 
 HUMAN_MODELS = SFMS  # social_nav_gym.py:11-12 minus "orca"
+MAX_FUSED_HUMANS = 512  # snp_step's limit: larger envs run on the tiled path
 
 
 class BatchedSocialNavGym:
@@ -38,6 +51,8 @@ class BatchedSocialNavGym:
         self.robot_kinematics = "holonomic"   # or "unicycle" (robot_agent.py:95: the robot policy's kinematics)
         self._robot_goals = None
         self.walls = None
+        self.spatial_order = True  # above MAX_FUSED_HUMANS: re-number the humans patch by patch after every reset
+        self._order = None         # [E, N] int64 device: the generator's index of the human at each row (None: the identity)
 
     def configure(self, config):
         """config: a configparser object with the reference's sections (social_nav_gym.py:59-84) or a flat dict."""
@@ -70,7 +85,8 @@ class BatchedSocialNavGym:
     def reset(self, phase="test", test_case=None, on_device=True):
         """SocialNavGym.reset (social_nav_gym.py:120-225) for the whole batch: env e gets case `case_counter + e`, i.e. the seed
         offset[phase] + case + e (:135-137).  on_device=True generates the scenarios with the reset kernel (snp_reset: the reference's
-        generators on NumPy's MT19937 stream, one thread per env); False builds them on the host (scenarios.py) and uploads."""
+        generators on NumPy's MT19937 stream, a warp per env, or a CTA per env above about 1,520 humans, up to about 6,300); False
+        builds them on the host (scenarios.py, any N) and uploads."""
         assert phase in ["train", "val", "test"]
         if test_case is not None:
             self.case_counter[phase] = test_case
@@ -103,7 +119,7 @@ class BatchedSocialNavGym:
         self._robot_goals = np.stack([robot[:, 10:12], robot[:, 0:2]], 1)
         robot[:, 3:5] = 0.0                                                      # robot.set(..., vx=0, vy=0) (social_nav_gym.py:213)
         states = np.concatenate([sc["states"], robot[:, None]], 1) if self.robot_visible else sc["states"]
-        self.engine = CrowdEngine.from_reference_arrays(self.human_policy, states, sc["goals"], walls=self.walls, consider_robot=self.robot_visible,
+        self.engine = self._engine_class().from_reference_arrays(self.human_policy, states, sc["goals"], walls=self.walls, consider_robot=self.robot_visible,
                                                         all_params_equal=True, dtype=self.dtype, device=self.device,
                                                         robot=None if self.robot_visible else robot)
         self.engine.respawn_bounds = sc.get("respawn_bounds")   # parallel traffic: respawn at the right end (mmm:407-422)
@@ -111,13 +127,32 @@ class BatchedSocialNavGym:
                               self.discomfort_penalty_factor, self.robot_time_step]
         if self.safety_space > 0:
             self.engine.set_safety_space(self.safety_space)
+        self._spatial_order()
         return self.observation(), np.zeros(self.E, int)
+
+    def _engine_class(self):
+        return TiledCrowdEngine if self.human_num > MAX_FUSED_HUMANS else CrowdEngine
+
+    def _spatial_order(self, mask=None):
+        """After a reset of all envs (mask None) or of those of `mask`: rows of reset envs are in the generator's order again; on
+        the tiled path with spatial_order, every env is then re-numbered patch by patch and the permutation composed into _order."""
+        if mask is None or self._order is None:
+            self._order = None
+        else:
+            ident = torch.arange(self.human_num, device=self._order.device).expand_as(self._order)
+            self._order = torch.where(mask.bool()[:, None], ident, self._order)
+        if not (isinstance(self.engine, TiledCrowdEngine) and self.spatial_order):
+            return
+        perm = self.engine._renumber()  # new_rows[e] = old_rows[e][perm[e]]
+        self._order = perm if self._order is None else torch.gather(self._order, 1, perm)
 
     def _reset_on_device(self, sim, seed0, phase, mask=None, seeds=None):
         e = self.engine
-        fresh = e is None or e.N != self.human_num or e.motion_model_title != self.human_policy or e.consider_robot != self.robot_visible
+        cls = self._engine_class()
+        fresh = (e is None or type(e) is not cls or e.N != self.human_num or e.motion_model_title != self.human_policy or
+                 e.consider_robot != self.robot_visible)
         if fresh:
-            e = self.engine = CrowdEngine(self.human_policy, self.E, self.human_num, G=2, dtype=self.dtype, device=self.device,
+            e = self.engine = cls(self.human_policy, self.E, self.human_num, G=2, dtype=self.dtype, device=self.device,
                                           consider_robot=self.robot_visible, symmetric=True, walls=self.walls, has_robot=True)
         e.consts = [float(self.time_limit), self.collision_penalty, self.success_reward, self.discomfort_dist,
                     self.discomfort_penalty_factor, self.robot_time_step]
@@ -136,6 +171,7 @@ class BatchedSocialNavGym:
         self._robot_goals = torch.stack([torch.stack([r[L.ROBOT_GX], r[L.ROBOT_GY]], -1), torch.stack([r[L.ROBOT_GX2], r[L.ROBOT_GY2]], -1)], 1).double().cpu().numpy()
         if self.robot_motion_model_title is not None:
             e.set_robot_motion_model(self.robot_motion_model_title)
+        self._spatial_order(None if fresh else mask)
         return self.observation(), np.zeros(self.E, int)
 
     def reset_finished(self, finished, phase="train"):
@@ -152,16 +188,21 @@ class BatchedSocialNavGym:
         return self.observation()
 
     def observation(self, theta_and_omega_visible=False):
+        """[E,N,5] (or [E,N,7]) with the humans in the generator's order, whatever the engine's numbering."""
         e = self.engine
         cols = [e.dyn[L.DYN_PX], e.dyn[L.DYN_PY], e.dyn[L.DYN_VX], e.dyn[L.DYN_VY], e.stat[L.STAT_R]]
         if theta_and_omega_visible:
             cols += [e.dyn[L.DYN_TH], e.dyn[L.DYN_OM]]
-        return torch.stack(cols, -1).double().cpu().numpy()
+        obs = torch.stack(cols, -1)
+        if self._order is not None:
+            obs = torch.empty_like(obs).scatter_(1, self._order[..., None].expand_as(obs), obs)
+        return obs.double().cpu().numpy()
 
     def step(self, action):
         """SocialNavGym.step (social_nav_gym.py:227-250) for every env.  `action` [E,2]: (vx, vy) for a holonomic robot (ActionXY) or
         (v, r) for a unicycle one (ActionRot; set `robot_kinematics = "unicycle"`, what RobotAgent takes from its policy,
-        robot_agent.py:95)."""
+        robot_agent.py:95).  Above 512 humans per env, parallel traffic and the hybrid scenario raise NotImplementedError here
+        (their respawn is not on the tiled path)."""
         self.engine.step(action, self.time_step, n_substeps=self.time_step_factor, pre_checks=True, kinematics=self.robot_kinematics)
         r = self.engine.decode_flags()
         return self.observation(), r["reward"], r["terminated"], r["truncated"], r["info"]
@@ -174,7 +215,8 @@ class BatchedSocialNavGym:
 
     def imitation_learning_step(self):
         """social_nav_gym.py:252-274 for every env: time_step_factor x (update_robot; update_humans), then the ACTUAL collision /
-        goal checks and the reward at the end time -- one launch."""
+        goal checks and the reward at the end time -- one launch.  Above 512 humans per env it raises NotImplementedError (the
+        tiled path has no robot moved by its own motion model)."""
         if self.engine.robot_type is None:
             self.engine.set_robot_motion_model(self.robot_motion_model_title, goals=self._robot_goals)
         self.engine.imitation_learning_step(self.time_step, n_substeps=self.time_step_factor)
