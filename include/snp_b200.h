@@ -27,6 +27,7 @@
  *                                                   social_nav_gym.py:252-274 imitation_learning_step
  *   snp_lookahead (+ dyn_out peek of snp_step)    <- crowd_nav/policy/cadrl.py:42-83 compute_rotated_states_and_reward, :13-40;
  *                                                   motion_model_manager.py:691-709 get_next_human_observable_states
+ *   snp_value_lookahead                           <- crowd_nav/policy/cadrl.py:235-276 CADRL.predict (value network, min, argmax)
  *   snp_robot_push_out                            <- src/robot_agent.py:35-48 RobotAgent.check_collisions (social_nav_sim.py:509)
  *   snp_reset                                     <- social_nav_gym.py:120-225 reset, social_nav_sim.py:200-431 scenario generators
  *   snp_pack_states / snp_unpack_states           <- src/agent.py:256-266 get_safe_state / set_state row layout
@@ -190,6 +191,27 @@ typedef struct snp_lookahead_args {
     double *rewards;          /* out [E][A]: -0.25 collision, 1 goal, (dmin - 0.2) * 0.5 * dt discomfort, 0 (cadrl.py:68-72), bit-exact */
 } snp_lookahead_args;
 
+/* CADRL's action choice (crowd_nav/policy/cadrl.py:235-276 CADRL.predict) for every env of a crowd, with the value network evaluated
+ * on the device where the lookahead's rows are made (csrc/snp_value.cu): rotated rows (as snp_lookahead, rounded to fp32) -> MLP ->
+ * minimum over the humans -> value = reward + gamma ^ (dt * v_pref) * (double) minimum in double -> first action of largest value.
+ * The rows and the network's activations never reach device memory. */
+typedef struct snp_value_args {
+    int32_t type;             /* the humans' model 0..8, as snp_lookahead_args.type */
+    int32_t A;                /* number of actions, 1..65535 */
+    int32_t theta_and_omega_visible; /* 0: 13 values per row; 1: 15 -- must equal widths[0] */
+    int32_t reserved;         /* bit 1: split every env's humans into chunks of 32 over several CTAs (the same bits; tests and measurement) */
+    const void *next;         /* [SNP_DYN_FIELDS][E*N] the humans one policy time step ahead (as snp_lookahead_args.next) */
+    const double *actions;    /* [A][2] holonomic velocities (vx, vy) */
+    double dt;                /* the policy's time step (0.25) */
+    double gamma;             /* the policy's discount factor */
+    int32_t layers;           /* Linear layers, 1..6, with ReLU between them and none after the last */
+    int32_t widths[7];        /* widths[0] = 13 | 15 inputs, widths[1..layers-1] hidden widths in 1..256, widths[layers] = 1 */
+    const float *weights;     /* device fp32, layer by layer: W transposed ([in][out] row-major, i.e. torch's weight.t()) then b [out] */
+    double *values;           /* out [E][A] */
+    int32_t *best;            /* out [E]: first index of the largest value (-1 if no value exceeds -inf) */
+    uint8_t *reached;         /* out [E]: 1 where the robot is within its radius of its goal now (predict returns the zero action there) */
+} snp_value_args;
+
 /* SocialNavGym.reset for every (selected) environment of a crowd, on the device (social_gym/social_nav_gym.py:120-225): env e replays
  * the reference's scenario generator (social_gym/social_nav_sim.py:200-299 circular crossing, :301-362 parallel traffic, :364-431
  * circular crossing with static obstacles; insert_robot = True, randomize_human_positions = True) on NumPy's own MT19937 stream seeded
@@ -234,6 +256,10 @@ int snp_robot_push_out(const snp_crowd *crowd, void *cuda_stream);
 int snp_reset(const snp_crowd *crowd, const snp_reset_args *args, void *cuda_stream);
 /* Uses crowd->dyn (current px,py,vx,vy,theta,omega), crowd->stat (radius) and crowd->robot (px,py,r,gx,gy,vd). */
 int snp_lookahead(const snp_crowd *crowd, const snp_lookahead_args *args, void *cuda_stream);
+/* Uses what snp_lookahead uses; values / best / reached only.  SNP_ERR_INVALID before any launch for null pointers, E or N < 1,
+ * E > 65535, A outside 1..65535, a bad type or dtype, layers outside 1..6, widths[0] != 13 | 15 (theta_and_omega_visible), a hidden
+ * width outside 1..256 or widths[layers] != 1. */
+int snp_value_lookahead(const snp_crowd *crowd, const snp_value_args *args, void *cuda_stream);
 /* The policies' query_env = False branch (crowd_nav/policy/cadrl.py:92-105 propagate_humans_state_with_constant_velocity_model):
  * `next` [SNP_DYN_FIELDS][E*N] (crowd dtype) = the humans one step of length dt ahead under constant velocity (x + vx dt, y + vy dt,
  * theta + omega dt, velocities carried over) -- the `next` input of snp_lookahead when the env is not queried. */

@@ -55,6 +55,12 @@ class SnpLookaheadArgs(ctypes.Structure):
                 ("next", c_void_p), ("actions", c_void_p), ("dt", c_double), ("rotated", c_void_p), ("rewards", c_void_p)]
 
 
+class SnpValueArgs(ctypes.Structure):
+    _fields_ = [("type", c_int32), ("A", c_int32), ("theta_and_omega_visible", c_int32), ("reserved", c_int32),
+                ("next", c_void_p), ("actions", c_void_p), ("dt", c_double), ("gamma", c_double), ("layers", c_int32),
+                ("widths", c_int32 * 7), ("weights", c_void_p), ("values", c_void_p), ("best", c_void_p), ("reached", c_void_p)]
+
+
 class SnpResetArgs(ctypes.Structure):
     _fields_ = [("scenario", c_int32), ("randomize_attributes", c_int32), ("seeds", c_void_p), ("seed0", ctypes.c_uint32),
                 ("reserved", ctypes.c_uint32), ("mask", c_void_p), ("circle_radius", c_double), ("robot_radius", c_double),
@@ -76,6 +82,7 @@ _SIGNATURES = {
     "snp_checks": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpStepOpts), c_void_p]),
     "snp_laser": (ctypes.c_int, [ctypes.POINTER(SnpLaserArgs), c_void_p]),
     "snp_lookahead": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpLookaheadArgs), c_void_p]),
+    "snp_value_lookahead": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpValueArgs), c_void_p]),
     "snp_constant_velocity": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_double, c_void_p, c_void_p]),
     "snp_reset": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), ctypes.POINTER(SnpResetArgs), c_void_p]),
     "snp_robot_push_out": (ctypes.c_int, [ctypes.POINTER(SnpCrowd), c_void_p]),

@@ -27,7 +27,7 @@
 // decodes the key and applies the same reward expression (look_reward) as the whole-env kernel: bit-identical rewards, in
 // any order of the atomics.  snp_lookahead_args.reserved bit 1 forces the split where one CTA would hold the env (tests and
 // measurement), as bit 0 forces the vector stores.
-#include "snp_kernels.cuh"
+#include "snp_lookahead.cuh"
 
 namespace snp {
 namespace {
@@ -47,20 +47,6 @@ struct LookArgs {
     int bulk;  // 1: tiles leave through cp.async.bulk; 0: cooperative vector stores (A/B comparison)
     int H, nhc;  // split kernel: humans per chunk, chunks per env (blockIdx.x = action range * nhc + chunk)
 };
-
-// cadrl.py:56-72 from the folded swept test: the reward of action (axd, ayd) for the robot at (rpx, rpy) with goal (rgx, rgy)
-__device__ __forceinline__ double look_reward(bool collision, double dmin, double axd, double ayd, double dt, double rpx, double rpy,
-                                              double rgx, double rgy, double rr) {
-    const double npx = __dadd_rn(rpx, __dmul_rn(axd, dt)), npy = __dadd_rn(rpy, __dmul_rn(ayd, dt));
-    const bool reached = xnorm_plain(__dsub_rn(npx, rgx), __dsub_rn(npy, rgy)) < rr;
-    if (collision) return -0.25;
-    if (reached) return 1.0;
-    if (dmin < 0.2) return __dmul_rn(__dmul_rn(__dsub_rn(dmin, 0.2), 0.5), dt);
-    return 0.0;
-}
-
-// Per-action quantities shared by the humans of an env: next robot position, (cos, sin) of the rotation, distance to goal.
-template <typename T> struct PerAction { double axd, ayd; T npx, npy, c, s, dg, ax, ay, pad; };
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 
@@ -113,30 +99,9 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : (kSplit ? 2
     const long long E = a.E;
     const T rpx = robot[SNP_ROBOT_PX * E + e], rpy = robot[SNP_ROBOT_PY * E + e], rr = robot[SNP_ROBOT_R * E + e];
     const T rgx = robot[SNP_ROBOT_GX * E + e], rgy = robot[SNP_ROBOT_GY * E + e], rvd = robot[SNP_ROBOT_VD * E + e];
-    // ---- per action, once per CTA: next robot position (cadrl.py:54), rotation (:22), distance to goal ----
-    // (cos rot, sin rot) with rot = atan2(gy, gx) is the unit vector towards the goal: g / |g| (and (1, 0) for g = 0, atan2(0,0) = 0)
-    // -- one division instead of an atan2 + sincos chain; agrees with the reference's libm round trip to ~1e-16.
-    for (int k = threadIdx.x; k < acnt; k += blockDim.x) {
-        PerAction<T> p;
-        p.axd = a.actions[2 * (abeg + k)]; p.ayd = a.actions[2 * (abeg + k) + 1];
-        p.ax = (T)p.axd; p.ay = (T)p.ayd; p.pad = T(0);
-        if (sizeof(T) == 8) {  // no contraction: p + a * dt
-            p.npx = (T)__dadd_rn((double)rpx, __dmul_rn(p.axd, a.dt)); p.npy = (T)__dadd_rn((double)rpy, __dmul_rn(p.ayd, a.dt));
-            const double gx = __dsub_rn((double)rgx, (double)p.npx), gy = __dsub_rn((double)rgy, (double)p.npy);
-            const double dg = xnorm_plain(gx, gy);
-            p.dg = (T)dg;
-            const double inv = dg > 0.0 ? 1.0 / dg : 0.0;
-            p.c = (T)(dg > 0.0 ? gx * inv : 1.0); p.s = (T)(gy * inv);
-        } else {
-            const T dtT = (T)a.dt;
-            p.npx = rpx + p.ax * dtT; p.npy = rpy + p.ay * dtT;
-            const T gx = rgx - p.npx, gy = rgy - p.npy;
-            p.dg = Real<T>::sqrt_exact(gx * gx + gy * gy);
-            const T inv = p.dg > T(0) ? T(1) / p.dg : T(0);
-            p.c = p.dg > T(0) ? gx * inv : T(1); p.s = gy * inv;
-        }
-        pa[k] = p;
-    }
+    // ---- per action, once per CTA: next robot position (cadrl.py:54), rotation (:22), distance to goal (look_action) ----
+    for (int k = threadIdx.x; k < acnt; k += blockDim.x)
+        pa[k] = look_action<T>(a.actions[2 * (abeg + k)], a.actions[2 * (abeg + k) + 1], a.dt, rpx, rpy, rgx, rgy);
     __syncthreads();
 
     const size_t row_words = (size_t)a.N * OW;  // one action's rows of the env; a split CTA's tile (chunk = 1) is its part of them
@@ -145,30 +110,15 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : (kSplit ? 2
     // the human's state and everything of the swept test that does not depend on the action stay in registers across tiles.
     const int k_own = threadIdx.x / N, j_own = threadIdx.x - k_own * N;
     const bool own = k_own < a.chunk;
-    struct Human { T hr, nxx, nxy, nvx, nvy, th, om; double dx, dy, hvx, hvy, rsum; };
+    using Human = LookHuman<T>;
     auto load_human = [&](int j) {
-        Human h;
-        h.hr = cur[4 * N + j];
-        h.nxx = nx[j]; h.nxy = nx[N + j]; h.nvx = nx[2 * N + j]; h.nvy = nx[3 * N + j]; h.th = nx[4 * N + j]; h.om = nx[5 * N + j];
-        h.dx = __dsub_rn((double)cur[j], (double)rpx); h.dy = __dsub_rn((double)cur[N + j], (double)rpy);  // sim:962 difference
-        h.hvx = (double)cur[2 * N + j]; h.hvy = (double)cur[3 * N + j];
-        h.rsum = (double)h.hr;
-        return h;
+        return look_human<T>(cur[j], cur[N + j], cur[2 * N + j], cur[3 * N + j], cur[4 * N + j], nx[j], nx[N + j], nx[2 * N + j], nx[3 * N + j],
+                             nx[4 * N + j], nx[5 * N + j], rpx, rpy);
     };
-    // one (action, human) pair: swept distance (social_nav_sim.py:962-976 via utils.py:22-36, formula-exact) and the rotated row
+    // one (action, human) pair: swept distance and the rotated row (snp_lookahead.cuh)
     auto do_pair = [&](const Human &h, const PerAction<T> &q, double *dist_out, T *o) {
-        const double vx = __dsub_rn(h.hvx, q.axd), vy = __dsub_rn(h.hvy, q.ayd);
-        const double ex = __dadd_rn(h.dx, __dmul_rn(vx, a.dt)), ey = __dadd_rn(h.dy, __dmul_rn(vy, a.dt));
-        *dist_out = __dsub_rn(__dsub_rn(origin_to_segment(h.dx, h.dy, ex, ey), h.rsum), (double)rr);
-        const T ddx = h.nxx - q.npx, ddy = h.nxy - q.npy;
-        o[0] = q.dg; o[1] = rvd; o[2] = T(0); o[3] = rr;
-        o[4] = q.ax * q.c + q.ay * q.s; o[5] = q.ay * q.c - q.ax * q.s;
-        o[6] = ddx * q.c + ddy * q.s; o[7] = ddy * q.c - ddx * q.s;
-        o[8] = h.nvx * q.c + h.nvy * q.s; o[9] = h.nvy * q.c - h.nvx * q.s;
-        o[10] = h.hr;
-        o[11] = Real<T>::sqrt_(ddx * ddx + ddy * ddy);  // < 1.5 ulp (snp_math.cuh); the rotated states carry the 1e-9 / 1e-4 tolerance
-        o[12] = rr + h.hr;
-        if (a.visible) { o[13] = h.th - T(0); o[14] = h.om; }
+        *dist_out = look_swept<T>(h, q, a.dt, rr);
+        look_row<T>(h, q, rvd, rr, a.visible, o);
     };
     Human mine{};
     if (own) mine = load_human(j_own);
@@ -243,8 +193,7 @@ __global__ void __launch_bounds__(kLookThreads, sizeof(T) == 4 ? 4 : (kSplit ? 2
             dmin = (d >= 0 && d < dmin) ? d : dmin;
         }
         if (kSplit) {  // this chunk's part of the swept test as an order-independent key (header comment)
-            const long long key = collision ? -1LL : __double_as_longlong(__dadd_rn(dmin, 0.0));  // -0.0 -> +0.0
-            atomicMin(reinterpret_cast<long long *>(a.rewards) + (size_t)e * a.A + abeg + k, key);
+            atomicMin(reinterpret_cast<long long *>(a.rewards) + (size_t)e * a.A + abeg + k, look_key(collision, dmin));
         } else {
             const PerAction<T> q = pa[k];
             a.rewards[(size_t)e * a.A + abeg + k] =
@@ -260,12 +209,11 @@ template <typename T> __global__ void k_lookahead_fold(const LookArgs a) {
     if (i >= (long long)a.E * a.A) return;
     const int e = (int)(i / a.A), k = (int)(i - (long long)e * a.A);
     const long long key = reinterpret_cast<const long long *>(a.rewards)[i];
-    const double d = __longlong_as_double(key), cap = 9223372036854775807.0;  // np.iinfo(np.int64).max, the reference's initial dmin
     const T *robot = (const T *)a.robot;
     const long long E = a.E;
-    a.rewards[i] = look_reward(key < 0, d < cap ? d : cap, a.actions[2 * k], a.actions[2 * k + 1], a.dt, (double)robot[SNP_ROBOT_PX * E + e],
-                               (double)robot[SNP_ROBOT_PY * E + e], (double)robot[SNP_ROBOT_GX * E + e], (double)robot[SNP_ROBOT_GY * E + e],
-                               (double)robot[SNP_ROBOT_R * E + e]);
+    a.rewards[i] = look_key_reward(key, a.actions[2 * k], a.actions[2 * k + 1], a.dt, (double)robot[SNP_ROBOT_PX * E + e],
+                                   (double)robot[SNP_ROBOT_PY * E + e], (double)robot[SNP_ROBOT_GX * E + e], (double)robot[SNP_ROBOT_GY * E + e],
+                                   (double)robot[SNP_ROBOT_R * E + e]);
 }
 
 template <typename T> int launch_lookahead_split(LookArgs a, cudaStream_t st) {

@@ -43,6 +43,35 @@ def model_parameters(title: str) -> np.ndarray:
     return p
 
 
+def value_network_layout(model):
+    """The packed form snp_value_lookahead takes of a value network: `model`'s leaf modules must be Linear and ReLU alternating and
+    end in Linear(., 1) -- CADRL's ValueNetwork (crowd_nav/policy/cadrl.py mlp(input_dim, mlp_dims), last_relu=False), or its
+    `value_network` Sequential -- with 13 or 15 inputs, hidden widths in 1..256 and at most 6 Linear layers.  Returns (widths,
+    packed): widths [in, h1, ..., 1] and a CPU float32 tensor holding, layer by layer, W transposed ([in][out] row-major,
+    weight.t()) then the bias [out] (zeros for a Linear without one).  Anything else raises ValueError."""
+    leaves = [m for m in model.modules() if next(m.children(), None) is None]
+    kinds = [type(m) for m in leaves]
+    if not leaves or len(leaves) % 2 == 0 or any(k is not (torch.nn.Linear if i % 2 == 0 else torch.nn.ReLU) for i, k in enumerate(kinds)):
+        raise ValueError("the value network must be Linear / ReLU alternating and end in a Linear layer, got "
+                         + ", ".join(k.__name__ for k in kinds))
+    linears = leaves[0::2]
+    if len(linears) > 6:
+        raise ValueError(f"at most 6 Linear layers (got {len(linears)})")
+    widths = [linears[0].in_features] + [m.out_features for m in linears]
+    if widths[0] not in (13, 15):
+        raise ValueError(f"the value network takes the 13 or 15 values of a rotated state, not {widths[0]}")
+    if widths[-1] != 1:
+        raise ValueError(f"the value network has one output, not {widths[-1]}")
+    if any(not 1 <= w <= 256 for w in widths[1:-1]):
+        raise ValueError(f"hidden widths must be in 1..256 (got {widths[1:-1]})")
+    parts = []
+    with torch.no_grad():
+        for m in linears:
+            parts.append(m.weight.detach().float().cpu().t().reshape(-1))
+            parts.append(torch.zeros(m.out_features) if m.bias is None else m.bias.detach().float().cpu().reshape(-1))
+    return widths, torch.cat(parts).contiguous()
+
+
 def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
@@ -91,6 +120,7 @@ class CrowdEngine:
         self.consts = [50.0, -0.25, 1.0, 0.2, 0.5, 0.25]
         self._peek_buf, self._peek_idx, self.action_space, self._rotated, self._rewards = None, None, None, None, None
         self._reset_scen, self._reset_draws = None, None
+        self._value_net, self._value_out = None, None
         self.walls, self.W, self.S, self.walls_per_env = None, 0, 0, 0
         if walls is not None:
             self.set_walls(walls)
@@ -532,6 +562,51 @@ class CrowdEngine:
         g.rotated, g.rewards = self._rotated.data_ptr(), self._rewards.data_ptr()
         L.check(self.lib.snp_lookahead(ctypes.byref(self._crowd()), ctypes.byref(g), _stream()))
         return self._rotated, self._rewards
+
+    # ------------------------------------------------------------------ the policy's action choice on the device
+    def set_value_network(self, model, gamma):
+        """CADRL's value network for predict(): `model` is packed once (value_network_layout) into a device fp32 buffer; `gamma` is
+        the policy's discount factor.  Raises ValueError for a network that is not Linear / ReLU alternating ending in Linear(., 1)."""
+        widths, packed = value_network_layout(model)
+        self._value_net = (widths, packed.to(self.device), float(gamma))
+
+    def predict(self, time_step=0.25, theta_and_omega_visible=False, query_env=True):
+        """CADRL.predict (crowd_nav/policy/cadrl.py:235-276) for every env, without the exploration: the humans `time_step` ahead
+        (query_env as in lookahead()), the value network on every rotated state, its minimum over the humans, value = reward +
+        gamma ^ (time_step * v_pref) * minimum and the first action of largest value.  Returns device tensors (best [E] int64,
+        values [E,A] float64, reached [E] bool); where `reached` is set the policy takes the zero action instead of best.  best is -1
+        in an env where no value exceeds -inf (a network that outputs NaN): predict's max_action stays None there, and
+        action_space[best] must not be taken for it."""
+        if query_env:
+            return self.predict_from(self.peek(time_step), time_step, theta_and_omega_visible)
+        return self.predict_from(self.constant_velocity_next(time_step), time_step, theta_and_omega_visible, yaw_from_next=True)
+
+    def predict_from(self, nxt, time_step=0.25, theta_and_omega_visible=False, yaw_from_next=False, split_humans=False):
+        """predict() on a given `nxt` [DYN_FIELDS,E,N] (as lookahead_from).  One fused kernel evaluates the network where each rotated
+        row is made and a small one folds rewards, values and the choice (csrc/snp_value.cu); the rows never reach device memory.
+        split_humans=True spreads every env's humans over several CTAs in chunks of 32 (the same bits; for tests and measurement)."""
+        if getattr(self, "action_space", None) is None:
+            raise ValueError("set_action_space(actions) first")
+        if self.robot is None:
+            raise ValueError("the lookahead needs the robot's state")
+        if getattr(self, "_value_net", None) is None:
+            raise ValueError("set_value_network(model, gamma) first")
+        widths, weights, gamma = self._value_net
+        A = self.action_space.shape[0]
+        if self._value_out is None or self._value_out[0].shape != (self.E, A):
+            dev = self.device
+            self._value_out = (torch.empty((self.E, A), dtype=torch.float64, device=dev), torch.empty((self.E,), dtype=torch.int32, device=dev),
+                               torch.empty((self.E,), dtype=torch.bool, device=dev))
+        values, best, reached = self._value_out
+        g = L.SnpValueArgs()
+        g.type, g.A, g.theta_and_omega_visible = (max(self.type, 3) if yaw_from_next else self.type), A, int(theta_and_omega_visible)
+        g.reserved = 2 if split_humans else 0
+        g.next, g.actions, g.dt, g.gamma = nxt.data_ptr(), self.action_space.data_ptr(), float(time_step), gamma
+        g.layers = len(widths) - 1
+        g.widths = (ctypes.c_int32 * 7)(*(widths + [0] * (7 - len(widths))))
+        g.weights, g.values, g.best, g.reached = weights.data_ptr(), values.data_ptr(), best.data_ptr(), reached.data_ptr()
+        L.check(self.lib.snp_value_lookahead(ctypes.byref(self._crowd()), ctypes.byref(g), _stream()))
+        return best.long(), values, reached
 
     def set_safety_space(self, safety_space):
         """motion_model_manager.py:147-164: every human gets 0.01 + safety_space; the robot gets it only when it is driven by an

@@ -357,7 +357,8 @@ class TiledCrowdEngine(_UnitSlots, CrowdEngine):
     bit for bit as a LargeCrowd built from environment e alone.  Loading and reading are CrowdEngine's (from_reference_arrays,
     rows, robot_rows, set_robot_rows, decode_flags, set_safety_space, walls shared or per env), and so is the policies' lookahead
     without a query of the env: lookahead(query_env=False) (the constant-velocity propagation, snp_constant_velocity) and
-    lookahead_from(next) work at any N (snp_lookahead splits an env's humans over several CTAs when one cannot hold them).  The
+    lookahead_from(next) work at any N (snp_lookahead splits an env's humans over several CTAs when one cannot hold them), and so do
+    predict(query_env=False) and predict_from(next), CADRL's action choice with its value network on the device (snp_value_lookahead).  The
     checks without a step (run_checks, check_actual_collisions_and_goal, collision_detection_and_reaching_goal) work at any N.
     Per-agent parameter rows, respawn and the snp_step features the tiled path does not have (peek and the lookahead through it,
     lookahead(query_env=True), imitation_learning_step, sim_update, step_host) raise.  `scratch` is the call's workspace (view buffers, tile boxes, partial sums, work lists); nothing in it is
